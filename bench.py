@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — geodesic rays/s and ms/frame of the 4K Schwarzschild lensed render.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json metric "geodesic rays/sec and ms/frame at 4K"; SURVEY.md §8d):
@@ -34,6 +34,10 @@ figure; the nominal peak and the fraction of it are given too); cpu_baseline = t
 port of the reference's CPU path) timed on this box's host cores.
 
 --impl reference times that CPU port alone (all host threads), one bounded sample per step.
+
+--dump-outputs DIR (GPU arm, rank 0): after the timed steps, the frame the last timed step
+returned, as a fixed seeded sample of its pixels (dump_frame), so that two builds run with the
+same arguments can be compared pixel for pixel.
 """
 import argparse
 import json
@@ -250,6 +254,23 @@ def stat(ms):
     return {"mean": float(a.mean()), "best": float(a.min()), "median": float(np.median(a))}
 
 
+DUMP_PIXELS = 1 << 21       # 2 M pixels: 24 MiB of float32 RGB + 16 MiB of float64 indices
+
+
+def dump_frame(frame, out_dir):
+    """Write a (H, W, C) frame tensor as out_dir/frame.npy: float32 (n, C), the pixels at the flat
+    indices out_dir/frame_pixel_index.npy (float64, ascending), n = min(H W, DUMP_PIXELS) drawn
+    without replacement from a generator with a fixed seed — the same pixels for every frame of
+    that shape (a whole 4K frame in float32 would be 95 MiB)."""
+    import torch
+    n_px = frame.shape[0] * frame.shape[1]
+    idx = np.sort(np.random.default_rng(0).choice(n_px, size=min(n_px, DUMP_PIXELS), replace=False))
+    pix = frame.reshape(n_px, -1)[torch.from_numpy(idx).to(frame.device)].float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frame.npy"), pix)
+    np.save(os.path.join(out_dir, "frame_pixel_index.npy"), idx.astype(np.float64))
+
+
 # ---------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------
@@ -407,10 +428,17 @@ def run_gpu(args):
     # ---- value: device-resident steps ---------------------------------------------------------
     for _ in range(args.warmup):
         step_resident()
+    last = [None]          # the frame the latest step returned (rank 0; None elsewhere)
+
+    def step_kept():
+        last[0] = step_resident()
     with ClockSampler(local) as clk:
-        ms = timed(step_resident, args.steps)
+        ms = timed(step_kept, args.steps)
     total_ms = max_over_ranks(float(np.sum(ms)))
     ms_stat = stat(ms)
+    if args.dump_outputs and rank == 0:
+        # before any later step can reuse the frame buffer (peer gather: two buffers, one more step)
+        dump_frame(last[0], args.dump_outputs)
 
     # ---- N > 1: rank 0 re-renders the gathered frame alone, in row chunks, and compares -----------
     gather_identical = None
@@ -962,7 +990,13 @@ def main():
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="N > 1: peer = rows stored straight into rank 0's frame over NVLink peer memory; "
                          "nccl = NCCL gather of row bands overlapped with the render")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="GPU arm: write a seeded sample of the frame the last timed step returned to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)
