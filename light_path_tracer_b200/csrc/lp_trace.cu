@@ -20,7 +20,10 @@
                                        half of the round 64 and 128 were equal; 512-thread CTAs are no faster than 256:
                                        profiles/r2ak_block512.log) */
 /* frames of fewer rays than this run two RK4 steps per trip instead of four (less speculation past the exit and a
-   smaller loop: 7 % faster at 1024 x 1024, 1 % at 4K r_obs = 15; four steps are 2.5-3.5 % faster at 4K / 8K r_obs = 100) */
+   smaller loop: 7 % faster at 1024 x 1024, 1 % at 4K r_obs = 15; four steps are 2.5-3.5 % faster at 4K / 8K r_obs = 100;
+   measured on the one-ray-per-pixel kernel).  The mirror-image kernel applies it to the rays it traces: 2 steps for a
+   mirrored 4K frame (2.08M traces; within 2 % either way) and 1080p (12 % faster), 4 for 8K (3 % faster):
+   profiles/r3a_trip_sweep.log */
 #define LP_RENDER_TRIP4_MIN_RAYS 4000000LL
 
 // LP_TRACE_HYBRID rule.  The FMA loop (scaled second-order form, lp_internal.cuh) differs from the strict one
@@ -387,6 +390,117 @@ lp_render_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts c, con
     }
 }
 
+// ---------------------------------------------------------------------------
+// Mirror-image frame kernel: one ray per SET of mirror-image pixels.
+// final_alpha, the winding and the step count of a pixel depend on its float32 viewing angle a32 alone, and
+// a32 is mirror-symmetric bit for bit when the view direction d has d0 == 0 (x) or d1 == 0 (y) and d2 != 0:
+// cam_x(W - col) == -cam_x(col) exactly (an exact integer / half-integer subtraction, then RN(x / f) or the
+// Markstein sequence, both odd under round-to-nearest), pixel_alpha64 sees xc only as xc * xc and as
+// xc * d0 = +-0, and a signed zero added to the nonzero d2 (or to yc * d1) disappears.  Pairs are col <-> W - col
+// and row <-> H - row; column 0 / row 0 have no partner and W / 2, H / 2 (even sizes) are their own.
+// So a lane traces a pixel of the traced quarter (or half) once and then remaps and stores each of its
+// images with that image's own camera coordinates: the frame, the lookups and the statistics are the ones
+// of the one-ray-per-pixel kernel.  8x4 warp tiles over the traced domain (see TraceArgs::mx_main).
+// Staged stores (RGB, float32 / 8-bit): each run of an image (a tile row: up to 8 pixels, contiguous in the
+// output, in reverse order for an x mirror) is staged at the same address modulo 16 as its destination; the
+// run's lanes then store the 16-byte (float32) / 8-byte (8-bit) windows that lie inside it as vectors and the
+// run's ends element by element.  A mirror image starts one pixel off the vector grid (column 0 is unpaired).
+// ---------------------------------------------------------------------------
+#define LP_MIRROR_RUN_SLOT 112      /* bytes of one staged run: 96 + up to 15 of alignment offset, rounded */
+
+template <bool FUSED, bool FAST, typename T, int MINB, int TRIP>
+__global__ void __launch_bounds__(LP_TRACE_BLOCK, MINB)
+lp_render_mirror_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts c, const CamConsts cam)
+{
+    const LoopRegs L = load_loop_regs<FUSED>(c);
+    __shared__ __align__(16) unsigned char stage[LP_TRACE_BLOCK / 32][4][LP_MIRROR_RUN_SLOT];
+    const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5, j = lane & 7, q = lane >> 3;
+    const unsigned wt = blockIdx.x * (blockDim.x >> 5) + wrp;
+    const unsigned ty = wt / a.mtiles_x, tx = wt - ty * a.mtiles_x;
+    int col, r;                  // frame column, tile-local row of the traced pixel
+    bool live;
+    if ((int)tx < a.mtx_main) { col = (int)(tx * 8u) + j; live = col < a.mx_main; col += a.mx_base; }
+    else { col = 0; live = j == 0; }
+    if ((int)ty < a.mty_main) { r = (int)(ty * 4u) + q; live = live && r < a.my_main; r += a.my_base; }
+    else { r = 0; live = live && q == 0; }
+    live = live && wt < a.m_warps;
+    RayResult res;
+    res.status = 0; res.steps = 0; res.nh = 0; res.fa = 0.0;
+    if (live) {
+        const float a32 = (float)pixel_alpha64(cam, cam_x(cam, col), cam_y(cam, a.row0 + r));
+        binet_trace<FUSED, FAST, TRIP>(c, L, (double)a32, res);
+        if (FUSED && hybrid_needs_retrace(res, a.retrace_steps, a.retrace_steps_small, a.retrace_h, a.retrace_off))
+            binet_trace<false, FAST>(c, load_loop_regs<false>(c), (double)a32, res);   // cold
+    }
+    // (formed again rather than kept across the loop: fewer registers live in it)
+    const double xc = cam_x(cam, col), yc = cam_y(cam, a.row0 + r);
+    const float fa32 = (float)((res.status == 1) ? res.fa : __longlong_as_double(0x7ff8000000000000LL));
+    const unsigned nh = (unsigned)(res.nh < 0 ? 0 : (res.nh > 65535 ? 65535 : res.nh));
+    const int W = cam.width, H = cam.height;
+    const bool xm = live && !(a.mir_skip & 1) && col != 0 && 2 * col != W;     // has an x mirror image
+    const bool ym = live && !(a.mir_skip & 2) && r != 0 && 2 * r != H;         // (y mirror: row0 == 0, rows == H)
+    const bool vec = (sizeof(T) == 4 || sizeof(T) == 1) && ra.vec_ok;
+    const int px = 3 * (int)sizeof(T);               // bytes of a staged (RGB) pixel
+#pragma unroll 1
+    for (int k = 0; k < 4; ++k) {
+        if (k & a.mir_skip) continue;                                   // warp-uniform
+        const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
+        const bool has = live && (!fx || xm) && (!fy || ym);
+        const int ic = fx ? W - col : col, ir = fy ? H - r : r;
+        const long long pi = (long long)ir * W + ic;                    // compact tile index of this image
+        if (has) {
+            if (a.out_fa) ((float *)a.out_fa)[pi] = fa32;
+            if (a.out_w) ((unsigned short *)a.out_w)[pi] = (unsigned short)nh;
+        }
+        // cam_x(W - col) == -cam_x(col), cam_y(H - r) == -cam_y(r) bit for bit (see above)
+        const double xi = fx ? -xc : xc, yi = fy ? -yc : yc;
+        if (vec) {
+            // the run of tile row q in this image: columns [cmin, cmax] of tile-local row rr
+            int cmin = has ? ic : 0x7fffffff, cmax = has ? ic : -1, rr = has ? ir : -1;
+#pragma unroll
+            for (int off = 1; off < 8; off <<= 1) {
+                cmin = min(cmin, __shfl_xor_sync(0xffffffffu, cmin, off));
+                cmax = max(cmax, __shfl_xor_sync(0xffffffffu, cmax, off));
+                rr = max(rr, __shfl_xor_sync(0xffffffffu, rr, off));
+            }
+            uintptr_t lo = 0, hi = 0;
+            unsigned char *sb = stage[wrp][q];
+            if (cmax >= 0) {
+                lo = (uintptr_t)ra.out + (uintptr_t)(((long long)rr * W + cmin) * px);
+                hi = lo + (uintptr_t)((cmax - cmin + 1) * px);
+                sb += lo & 15u;                                         // same address modulo 16 as the run
+            }
+            if (has) remap_pixel_xy<T, true>(ra, cam, (T *)(sb + (ic - cmin) * px), xi, yi, fa32, nh, res.fa, res.cf, res.sf);
+            __syncwarp();
+            if (cmax >= 0) {
+                const unsigned vb = (sizeof(T) == 4) ? 16u : 8u;
+                const uintptr_t g = (lo & ~(uintptr_t)(vb - 1u)) + j * vb;      // lane j: the run's window j
+                const unsigned char *s = sb - (lo & (vb - 1u)) + j * vb;
+                if (g < hi) {
+                    if (g >= lo && g + vb <= hi) {
+                        if (vb == 16u) *reinterpret_cast<uint4 *>(g) = *reinterpret_cast<const uint4 *>(s);
+                        else *reinterpret_cast<uint2 *>(g) = *reinterpret_cast<const uint2 *>(s);
+                    } else {
+#pragma unroll
+                        for (unsigned e = 0; e < vb; e += (unsigned)sizeof(T))
+                            if (g + e >= lo && g + e < hi) *reinterpret_cast<T *>(g + e) = *reinterpret_cast<const T *>(s + e);
+                    }
+                }
+            }
+            __syncwarp();      // the staging slots are reused by the next image
+        } else if (has) {
+            remap_pixel_xy<T, true>(ra, cam, (T *)ra.out + pi * ra.channels, xi, yi, fa32, nh, res.fa, res.cf, res.sf);
+        }
+    }
+    if (a.stats) {
+        const unsigned m = (xm ? 2u : 1u) * (ym ? 2u : 1u);
+        StatAcc acc;
+        acc.init();
+        acc.add_mult(res, live, m);
+        lp_stats_flush(acc, live ? m : 0ull, a.stats);
+    }
+}
+
 // RK4 steps per loop trip of the fast path: LP_RENDER_TRIP=2|4 (tuning knob).
 static int render_trip(long long n_rays)
 {
@@ -476,6 +590,40 @@ static int launch_render(const TraceArgs &a, const RemapArgs &ra, const BinetCon
                          const CamConsts &cam, uint32_t flags, cudaStream_t stream)
 {
     return launch_render_mb<T, 4>(a, ra, c, cam, flags, stream);
+}
+
+// The mirror-image kernel for a contiguous row tile: x mirror when mir_x, y mirror when mir_y (whole frame).
+template <typename T>
+static int launch_render_mirror(const TraceArgs &a_in, const RemapArgs &ra, const BinetConsts &c,
+                                const CamConsts &cam, int32_t rows, bool mir_x, bool mir_y, uint32_t flags,
+                                cudaStream_t stream)
+{
+    const bool fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
+    const bool icmp = (fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) != 0;
+    TraceArgs a = a_in;
+    const int W = cam.width;
+    a.mir_skip = (mir_x ? 0 : 1) | (mir_y ? 0 : 2);
+    a.mx_main = mir_x ? W / 2 : W;           a.mx_base = mir_x ? W - W / 2 : 0;
+    a.my_main = mir_y ? rows / 2 : rows;     a.my_base = mir_y ? rows - rows / 2 : 0;
+    a.mtx_main = (a.mx_main + 7) / 8;        a.mty_main = (a.my_main + 3) / 4;
+    const long long tiles_x = a.mtx_main + (mir_x ? 1 : 0), tiles_y = a.mty_main + (mir_y ? 1 : 0);
+    const long long warps = tiles_x * tiles_y;
+    const int block = trace_block_size();
+    if (warps * 32 > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
+    a.mtiles_x = (uint32_t)tiles_x; a.m_warps = (uint32_t)warps;
+    const unsigned grid = (unsigned)((warps * 32 + block - 1) / block);
+    const long long traced = (long long)(a.mx_main + (mir_x ? 1 : 0)) * (a.my_main + (mir_y ? 1 : 0));
+    const int trip = render_trip(traced);
+    if (fused) {
+        if (icmp && trip == 4) lp_render_mirror_kernel<true, true, T, 4, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
+        else if (icmp) lp_render_mirror_kernel<true, true, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+        else      lp_render_mirror_kernel<true, false, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+    } else {
+        if (icmp && trip == 4) lp_render_mirror_kernel<false, true, T, 4, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
+        else if (icmp) lp_render_mirror_kernel<false, true, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+        else      lp_render_mirror_kernel<false, false, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+    }
+    return lp_check_launch();
 }
 
 // Frame rows of a (possibly interleaved) tile: last frame row + 1, or -1 for a bad request.
@@ -569,6 +717,23 @@ extern "C" int lp_render_frame_bands(const void *src, int32_t src_dtype, int32_t
     if ((flags & LP_TRACE_REPACK) && (rp_fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) && c.valid && n <= 0x7fffffffLL) {
         ra.vec_ok = (contiguous32 && ((uintptr_t)out % 16) == 0) ? 1 : 0;   // chunks are staged by construction
         return lp_launch_render_repack(a, ra, c, cam, src_dtype, flags, st);
+    }
+    // mirror images (lp_render_mirror_kernel): contiguous rows stored compactly, default schedule; x needs
+    // d0 == 0 (either sign), y needs d1 == 0 and the whole frame, both need d2 != 0
+    const bool mir_ok = band_rows == 0 && !(flags & (LP_RENDER_OUT_FRAME_ROWS | LP_RENDER_ROW_RUNS)) &&
+                        !render_dyn() && cam.d2 != 0.0;
+    const bool mir_x = mir_ok && cam.d0 == 0.0;
+    const bool mir_y = mir_ok && cam.d1 == 0.0 && row0 == 0 && rows == cam.height;
+    if (mir_x || mir_y) {
+        const int esz = (src_dtype == LP_DTYPE_F32) ? 4 : 1;
+        ra.vec_ok = ((flags & LP_RENDER_STAGED_STORES) && channels == 3 &&
+                     (src_dtype == LP_DTYPE_F32 || src_dtype == LP_DTYPE_U8) && ((uintptr_t)out % esz) == 0) ? 1 : 0;
+        switch (src_dtype) {
+        case LP_DTYPE_U8: return launch_render_mirror<unsigned char>(a, ra, c, cam, rows, mir_x, mir_y, flags, st);
+        case LP_DTYPE_F32: return launch_render_mirror<float>(a, ra, c, cam, rows, mir_x, mir_y, flags, st);
+        case LP_DTYPE_F64: return launch_render_mirror<double>(a, ra, c, cam, rows, mir_x, mir_y, flags, st);
+        default: return LP_ERR_INVALID_ARG;
+        }
     }
     switch (src_dtype) {
     case LP_DTYPE_U8: return launch_render<unsigned char>(a, ra, c, cam, flags, st);

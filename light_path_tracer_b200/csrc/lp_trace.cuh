@@ -43,6 +43,13 @@ struct TraceArgs {
     // lanes that store (tile_h * per_run), and ceil(2^16 / per_run) for lane / per_run by multiply-shift
     int32_t st_run_bytes, st_vb, st_per_run, st_lanes;
     uint32_t st_magic;
+    // mirror-image frame kernel (lp_render_mirror_kernel): the traced columns are mx_base .. mx_base + mx_main - 1
+    // in mtx_main warp-tile columns of 8, then (x mirror) one more tile column whose first lane traces column 0;
+    // the same for tile-local rows in tiles of 4 (my_*).  Image k = 0..3 of a ray is mirrored in x when k & 1 and
+    // in y when k & 2; the images with k & mir_skip do not exist in this launch.
+    int32_t mir_skip;
+    int32_t mx_main, mx_base, mtx_main, my_main, my_base, mty_main;
+    uint32_t mtiles_x, m_warps;     // warp tiles per tile row, warp tiles in the launch
 };
 
 // frame row of tile-local row r (interleaved bands, see above)
