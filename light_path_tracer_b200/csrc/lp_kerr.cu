@@ -24,8 +24,9 @@
 // divisions share 7 denominators: each quotient is formed as the compiler's own division
 // sequence with the reciprocal part hoisted (div_rcp / div_by, lp_internal.cuh) — bit-identical
 // quotients, 204 instead of 235 FP64-pipe slots and 325 instead of 604 instructions per
-// evaluation.  A second form over three approximate reciprocals (within a few ulp; opt-in,
-// outside the parity bar for axis_refine rays: see kerr_fast_rhs) is kept for comparison.
+// evaluation.  Three shared approximate reciprocals (a few ulp per term) would be cheaper, but with
+// the axis_refine tolerances (rtol 1e-8) they move step sizes by ~1e-8, and the reference's linear
+// interpolation at the exit radius turns that into up to 6e-9 in final_alpha, outside the 1e-9 bar.
 #include "lp_internal.cuh"
 #include <stdlib.h>
 
@@ -59,13 +60,11 @@ static __constant__ double kA21 = 1.0 / 5.0, kA31 = 3.0 / 40.0, kA32 = 9.0 / 40.
     kE1 = 71.0 / 57600.0, kE3 = -71.0 / 16695.0, kE4 = 71.0 / 1920.0, kE5 = -17253.0 / 339200.0,
     kE6 = 22.0 / 525.0, kE7 = -1.0 / 40.0;
 
-// metrics.py:227-306.  EXACT: the reference's expression tree with one IEEE division per `/`;
-// otherwise the same expressions over three shared reciprocals (see below).
+// metrics.py:227-306
 struct K5 { double v0, v1, v2, v3, v4; };
 
 // All arguments and the five derivatives travel in registers (scalars by value, a plain struct
 // back): array references to a __noinline__ function would go through local memory.
-template <bool EXACT>
 __device__ __noinline__ K5 kerr_rhs_regs(double r, double th, double p_r, double p_th, double p_t, double p_phi,
                                          double M, double a, double r_floor)
 {
@@ -82,7 +81,6 @@ __device__ __noinline__ K5 kerr_rhs_regs(double r, double th, double p_r, double
     else sincos(th, &sin_th, &cos_th);
     double sin_th_sq = sin_th * sin_th;
     if (sin_th_sq < 1e-15) sin_th_sq = 1e-15;
-    if (EXACT) {
     // The reference's expression tree, one IEEE quotient per `/` (bit for bit: div_by), over the
     // 7 distinct denominators its 14 divisions share.
     const double Sigma = r * r + a * a * cos_th * cos_th;
@@ -138,68 +136,18 @@ __device__ __noinline__ K5 kerr_rhs_regs(double r, double th, double p_r, double
                                  + dg_thth_inv_dth * p_th * p_th
                                  + dg_phiphi_inv_dth * p_phi * p_phi);
     out.v0 = dr; out.v1 = dth; out.v2 = dphi; out.v3 = dp_r; out.v4 = dp_th;
-    } else {
-    const double Sigma = r * r + a * a * cos_th * cos_th;
-    const double Delta = r * r - 2.0 * M * r + a * a;
-    const double A = (r * r + a * a) * (r * r + a * a) - a * a * Delta * sin_th_sq;
-    // Same expressions as the reference with its 14 divisions replaced by products of three
-    // reciprocals (1/Sigma, 1/Delta, 1/sin^2 theta): every term within a few ulp.  The tests hold
-    // the result to the same bar as the exact-division build (identical accept/reject sequences,
-    // final_alpha <= 1e-9).
-    const double iS = fast_rcp(Sigma), iD = fast_rcp(Delta), is2 = fast_rcp(sin_th_sq);
-    const double iSD = iS * iD, iS2 = iS * iS;
-    const double iSD2 = iSD * iSD, iden2 = iSD2 * (is2 * is2);
-    const double twoMa = 2.0 * M * a;
-    const double num = Delta - a * a * sin_th_sq;
-    const double g_tphi_inv = -twoMa * r * iSD;
-    const double g_rr_inv = Delta * iS;
-    const double g_thth_inv = iS;
-    const double g_phiphi_inv = num * iSD * is2;
-    const double dr = g_rr_inv * p_r;
-    const double dth = g_thth_inv * p_th;
-    const double dphi = g_tphi_inv * p_t + g_phiphi_inv * p_phi;
-    const double dSigma_dr = 2.0 * r;
-    const double dDelta_dr = 2.0 * r - 2.0 * M;
-    const double dA_dr = 4.0 * r * (r * r + a * a) - a * a * dDelta_dr * sin_th_sq;
-    const double sigma_delta = Sigma * Delta;
-    const double X = dSigma_dr * Delta + Sigma * dDelta_dr;
-    const double dg_tt_inv_dr = -(dA_dr * sigma_delta - A * X) * iSD2;
-    const double dg_tphi_inv_dr = -(twoMa * (sigma_delta - r * X)) * iSD2;
-    const double dg_rr_inv_dr = (dDelta_dr * Sigma - Delta * dSigma_dr) * iS2;
-    const double dg_thth_inv_dr = -dSigma_dr * iS2;
-    const double den = sigma_delta * sin_th_sq;
-    const double dg_phiphi_inv_dr = (dDelta_dr * den - num * X * sin_th_sq) * iden2;
-    const double pt2 = p_t * p_t, ptpp = p_t * p_phi, pr2 = p_r * p_r, pth2 = p_th * p_th, pp2 = p_phi * p_phi;
-    const double dp_r = -0.5 * (dg_tt_inv_dr * pt2 + 2.0 * dg_tphi_inv_dr * ptpp + dg_rr_inv_dr * pr2
-                                + dg_thth_inv_dr * pth2 + dg_phiphi_inv_dr * pp2);
-    const double sc2 = 2.0 * sin_th * cos_th;
-    const double dSigma_dth = -a * a * sc2;
-    const double dA_dth = -a * a * Delta * sc2;
-    const double dg_tt_inv_dth = -(dA_dth * sigma_delta - A * dSigma_dth * Delta) * iSD2;
-    const double dg_tphi_inv_dth = twoMa * r * dSigma_dth * iS2 * iD;
-    const double dg_rr_inv_dth = -Delta * dSigma_dth * iS2;
-    const double dg_thth_inv_dth = -dSigma_dth * iS2;
-    const double dnum_dth = -a * a * sc2;
-    const double dden_dth = dSigma_dth * Delta * sin_th_sq + sigma_delta * sc2;
-    const double dg_phiphi_inv_dth = (dnum_dth * den - num * dden_dth) * iden2;
-    const double dp_th = -0.5 * (dg_tt_inv_dth * pt2 + 2.0 * dg_tphi_inv_dth * ptpp + dg_rr_inv_dth * pr2
-                                 + dg_thth_inv_dth * pth2 + dg_phiphi_inv_dth * pp2);
-    out.v0 = dr; out.v1 = dth; out.v2 = dphi; out.v3 = dp_r; out.v4 = dp_th;
-    }
     return out;
 }
 
-template <bool EXACT>
 __device__ __forceinline__ void kerr_rhs(const double (&s)[5], double p_t, double p_phi, double M, double a,
                                          double r_floor, double (&out)[5])
 {
-    const K5 k = kerr_rhs_regs<EXACT>(s[0], s[1], s[3], s[4], p_t, p_phi, M, a, r_floor);
+    const K5 k = kerr_rhs_regs(s[0], s[1], s[3], s[4], p_t, p_phi, M, a, r_floor);
     out[0] = k.v0; out[1] = k.v1; out[2] = k.v2; out[3] = k.v3; out[4] = k.v4;
 }
 
 // One Dormand-Prince attempt from (state, k1 = f(state)) with step h: stages 2-7 and the 5th-order
 // solution (metrics.py:461-496).
-template <bool EXACT>
 __device__ __forceinline__ void kerr_dp_stages(const double (&state)[5], const double (&k1)[5], double h,
                                                double p_t, double p_phi, double M, double sp, double r_floor,
                                                double (&k3)[5], double (&k4)[5], double (&k5)[5], double (&k6)[5],
@@ -208,25 +156,25 @@ __device__ __forceinline__ void kerr_dp_stages(const double (&state)[5], const d
     double k2[5], tmp[5];
 #pragma unroll
     for (int i = 0; i < 5; ++i) tmp[i] = state[i] + h * kA21 * k1[i];
-    kerr_rhs<EXACT>(tmp, p_t, p_phi, M, sp, r_floor, k2);
+    kerr_rhs(tmp, p_t, p_phi, M, sp, r_floor, k2);
 #pragma unroll
     for (int i = 0; i < 5; ++i) tmp[i] = state[i] + h * (kA31 * k1[i] + kA32 * k2[i]);
-    kerr_rhs<EXACT>(tmp, p_t, p_phi, M, sp, r_floor, k3);
+    kerr_rhs(tmp, p_t, p_phi, M, sp, r_floor, k3);
 #pragma unroll
     for (int i = 0; i < 5; ++i) tmp[i] = state[i] + h * (kA41 * k1[i] + kA42 * k2[i] + kA43 * k3[i]);
-    kerr_rhs<EXACT>(tmp, p_t, p_phi, M, sp, r_floor, k4);
+    kerr_rhs(tmp, p_t, p_phi, M, sp, r_floor, k4);
 #pragma unroll
     for (int i = 0; i < 5; ++i)
         tmp[i] = state[i] + h * (kA51 * k1[i] + kA52 * k2[i] + kA53 * k3[i] + kA54 * k4[i]);
-    kerr_rhs<EXACT>(tmp, p_t, p_phi, M, sp, r_floor, k5);
+    kerr_rhs(tmp, p_t, p_phi, M, sp, r_floor, k5);
 #pragma unroll
     for (int i = 0; i < 5; ++i)
         tmp[i] = state[i] + h * (kA61 * k1[i] + kA62 * k2[i] + kA63 * k3[i] + kA64 * k4[i] + kA65 * k5[i]);
-    kerr_rhs<EXACT>(tmp, p_t, p_phi, M, sp, r_floor, k6);
+    kerr_rhs(tmp, p_t, p_phi, M, sp, r_floor, k6);
 #pragma unroll
     for (int i = 0; i < 5; ++i)
         nxt[i] = state[i] + h * (kB1 * k1[i] + kB3 * k3[i] + kB4 * k4[i] + kB5 * k5[i] + kB6 * k6[i]);
-    kerr_rhs<EXACT>(nxt, p_t, p_phi, M, sp, r_floor, k7);
+    kerr_rhs(nxt, p_t, p_phi, M, sp, r_floor, k7);
 }
 
 // Sum of squared scaled errors (metrics.py:505-513).  The five quotients e_i / scale_i go over a
@@ -392,7 +340,6 @@ __device__ __forceinline__ void kerr_store_result(const KerrArgs &a, long long i
 // One trip of the reference's `for _step in range(max_steps)` (metrics.py:451-566) for one lane: the
 // loop guards, one Dormand-Prince attempt, the controller, the exit events.  done: 0 running,
 // 1 finished -> extract the final direction, 2 invalid (status 0).
-template <bool EXACT>
 __device__ __forceinline__ void kerr_trip(double (&state)[5], double (&k1)[5], double p_t, double p_phi,
                                           double M, double sp, double r_floor, double r_capture, double r_escape,
                                           double lambda_max, double h_min, double atol, double rtol,
@@ -412,7 +359,7 @@ __device__ __forceinline__ void kerr_trip(double (&state)[5], double (&k1)[5], d
         } else {
             attempts++;
             double k3[5], k4[5], k5[5], k6[5], k7[5], nxt[5];
-            kerr_dp_stages<EXACT>(state, k1, h, p_t, p_phi, M, sp, r_floor, k3, k4, k5, k6, k7, nxt);
+            kerr_dp_stages(state, k1, h, p_t, p_phi, M, sp, r_floor, k3, k4, k5, k6, k7, nxt);
 
             if (!finite5(nxt) || nxt[0] <= 0.0) {                        // metrics.py:498-503
                 h *= 0.25;
@@ -464,7 +411,7 @@ __device__ __forceinline__ void kerr_trip(double (&state)[5], double (&k1)[5], d
     }
 }
 
-template <bool EXACT, int MINB>
+template <int MINB>
 __global__ void __launch_bounds__(KERR_BLOCK, MINB)
 lp_kerr_kernel(const KerrArgs a, const CamConsts cam)
 {
@@ -516,7 +463,7 @@ lp_kerr_kernel(const KerrArgs a, const CamConsts cam)
                 atol = refine ? 1e-10 : 1e-8;                               // metrics.py:432-433
                 rtol = refine ? 1e-8 : 1e-6;
                 if (kerr_init(M, sp, a.r_obs, alpha, theta, a.theta_obs, a.sin_th_obs, a.cos_th_obs, state, p_t, p_phi)) {
-                    kerr_rhs<EXACT>(state, p_t, p_phi, M, sp, r_floor, k1);   // FSAL seed, metrics.py:447
+                    kerr_rhs(state, p_t, p_phi, M, sp, r_floor, k1);   // FSAL seed, metrics.py:447
                     lam = 0.0;
                     h = fmax(1.0, 0.01 * a.r_obs);
                     accepted = 0; attempts = 0; iters = 0;
@@ -534,8 +481,8 @@ lp_kerr_kernel(const KerrArgs a, const CamConsts cam)
 
         // ---------------- one trip of the reference's `for _step in range(max_steps)` ----------------
         int done, event_status;
-        kerr_trip<EXACT>(state, k1, p_t, p_phi, M, sp, r_floor, r_capture, r_escape, lambda_max, h_min, atol, rtol,
-                         lam, h, accepted, attempts, iters, done, event_status);
+        kerr_trip(state, k1, p_t, p_phi, M, sp, r_floor, r_capture, r_escape, lambda_max, h_min, atol, rtol,
+                  lam, h, accepted, attempts, iters, done, event_status);
         if (done) {          // park the lane: its result is produced in the next flush phase
             pending = done;
             pend_event = event_status;
@@ -565,7 +512,7 @@ struct KerrWarpQueues {
     int in_flag[32];                                        // bit 0 valid, bit 1 axis_refine
 };
 
-template <bool EXACT, int MINB>
+template <int MINB>
 __global__ void __launch_bounds__(KERR_BLOCK, MINB)
 lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
 {
@@ -658,7 +605,7 @@ lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
                     const bool ok = kerr_init(M, sp, a.r_obs, alpha, theta, a.theta_obs, a.sin_th_obs, a.cos_th_obs,
                                               s0, i_p_t, i_p_phi);
                     if (ok) {
-                        kerr_rhs<EXACT>(s0, p_t, i_p_phi, M, sp, r_floor, kk);   // FSAL seed, metrics.py:447
+                        kerr_rhs(s0, p_t, i_p_phi, M, sp, r_floor, kk);   // FSAL seed, metrics.py:447
                         Q.in[0][lane] = s0[0]; Q.in[1][lane] = s0[1]; Q.in[2][lane] = s0[3]; Q.in[3][lane] = s0[4];
                         Q.in[4][lane] = i_p_phi;
 #pragma unroll
@@ -703,8 +650,8 @@ lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
 
         // ---------------- one trip of the reference's `for _step in range(max_steps)` ----------------
         int done, event_status;
-        kerr_trip<EXACT>(state, k1, p_t, p_phi, M, sp, r_floor, r_capture, r_escape, lambda_max, h_min, atol, rtol,
-                         lam, h, accepted, attempts, iters, done, event_status);
+        kerr_trip(state, k1, p_t, p_phi, M, sp, r_floor, r_capture, r_escape, lambda_max, h_min, atol, rtol,
+                  lam, h, accepted, attempts, iters, done, event_status);
         if (done) {
             pending = done;
             pend_event = event_status;
@@ -713,29 +660,11 @@ lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
     }
 }
 
-// LP_KERR_FAST=1 selects the approximate-reciprocal right-hand side (it was 2.7x faster than the
-// first exact build; against the exact build over shared reciprocals: 47 vs 51 ms).  NOT the default: with
-// the tight axis_refine tolerances (rtol 1e-8) the error norm is a 9-digit cancellation, a few ulp
-// in the stages move the step sizes by ~1e-8, and the reference's LINEAR interpolation at the exit
-// radius (metrics.py:533-548, an O(h^2) error that depends on where the last step falls) turns
-// that into up to 6e-9 in final_alpha — measured, and reproduced on the CPU — which is outside the
-// 1e-9 parity bar.  Rays traced with rtol 1e-6 stay within 1e-9 either way.
-static bool kerr_fast_rhs()
-{
-    static int cached = -1;
-    if (cached < 0) {
-        const char *e = getenv("LP_KERR_FAST");
-        cached = (e && atoi(e) == 1) ? 1 : 0;
-    }
-    return cached == 1;
-}
-
 static int kerr_launch(KerrArgs &a, const CamConsts &cam, cudaStream_t stream)
 {
     if (a.n == 0) return LP_OK;
     a.sin_th_obs = sin(a.theta_obs);
     a.cos_th_obs = cos(a.theta_obs);
-    const bool fast = kerr_fast_rhs();
     static int refill = 0;
     if (!refill) {
         const char *e = getenv("LP_KERR_REFILL");
@@ -751,39 +680,38 @@ static int kerr_launch(KerrArgs &a, const CamConsts &cam, cudaStream_t stream)
         const int v = e ? atoi(e) : 0;
         minb = (v >= 2 && v <= 6) ? v : KERR_DEFAULT_MINB;
     }
-#define KERR_DISPATCH(EX, MB) \
+#define KERR_DISPATCH(MB) \
     do { \
         int grid = 0; \
-        int rc = lp_grid_for((const void *)lp_kerr_kernel<EX, MB>, KERR_BLOCK, &grid); \
+        int rc = lp_grid_for((const void *)lp_kerr_kernel<MB>, KERR_BLOCK, &grid); \
         if (rc != LP_OK) return rc; \
         const long long chunks = (a.n + KERR_BLOCK - 1) / KERR_BLOCK; \
         if (chunks < grid) grid = (int)chunks; \
-        lp_kerr_kernel<EX, MB><<<grid, KERR_BLOCK, 0, stream>>>(a, cam); \
+        lp_kerr_kernel<MB><<<grid, KERR_BLOCK, 0, stream>>>(a, cam); \
     } while (0)
     const char *qe = getenv("LP_KERR_QUEUE");
     const bool queued = !(qe && atoi(qe) == 0);
-#define KERR_DISPATCH_Q(EX, MB) \
+#define KERR_DISPATCH_Q(MB) \
     do { \
         int grid = 0; \
-        int rc = lp_grid_for((const void *)lp_kerr_queued_kernel<EX, MB>, KERR_BLOCK, &grid); \
+        int rc = lp_grid_for((const void *)lp_kerr_queued_kernel<MB>, KERR_BLOCK, &grid); \
         if (rc != LP_OK) return rc; \
         const long long chunks = (a.n + KERR_BLOCK - 1) / KERR_BLOCK; \
         if (chunks < grid) grid = (int)chunks; \
-        lp_kerr_queued_kernel<EX, MB><<<grid, KERR_BLOCK, 0, stream>>>(a, cam); \
+        lp_kerr_queued_kernel<MB><<<grid, KERR_BLOCK, 0, stream>>>(a, cam); \
     } while (0)
-    if (queued && !fast) {
-        if (minb == 3) { KERR_DISPATCH_Q(true, 3); }
-        else if (minb == 5) { KERR_DISPATCH_Q(true, 5); }
-        else { KERR_DISPATCH_Q(true, 4); }
+    if (queued) {
+        if (minb == 3) { KERR_DISPATCH_Q(3); }
+        else if (minb == 5) { KERR_DISPATCH_Q(5); }
+        else { KERR_DISPATCH_Q(4); }
         return lp_check_launch();
     }
 #undef KERR_DISPATCH_Q
-    if (fast) { KERR_DISPATCH(false, 2); }
-    else if (minb == 2) { KERR_DISPATCH(true, 2); }
-    else if (minb == 3) { KERR_DISPATCH(true, 3); }
-    else if (minb == 4) { KERR_DISPATCH(true, 4); }
-    else if (minb == 5) { KERR_DISPATCH(true, 5); }
-    else { KERR_DISPATCH(true, 6); }
+    if (minb == 2) { KERR_DISPATCH(2); }
+    else if (minb == 3) { KERR_DISPATCH(3); }
+    else if (minb == 4) { KERR_DISPATCH(4); }
+    else if (minb == 5) { KERR_DISPATCH(5); }
+    else { KERR_DISPATCH(6); }
 #undef KERR_DISPATCH
     return lp_check_launch();
 }

@@ -36,7 +36,6 @@
 #define RK_BLOCK 128
 #define RK_REFILL_MIN 8
 #define RK_DEFAULT_MINB 3
-#define RK_DEFAULT_VARIANT 0
 #define RK_DEFAULT_EQ 1
 #define RK_DEFAULT_EQ_MINB 4
 #define RK_NC 6            /* moving components: t, r, theta, phi, p_r, p_theta */
@@ -99,19 +98,7 @@ __device__ __forceinline__ void rk_rhs(double R_S, double r_floor, double p_t, d
     double s2 = tc.s * tc.s;
     if (s2 < 1e-15) s2 = 1e-15;
     const double pp2 = p_phi * p_phi;
-#ifdef LP_RK45_EXACT_DIV
-    // the reference's expression tree, one IEEE division per `/` (9 per evaluation)
-    const double f = 1.0 - R_S / r;
-    const double r2 = r * r, r3 = r * r * r;
-    const double a = R_S / (2.0 * r2);
-    d[0] = -p_t / f;
-    d[1] = f * p_r;
-    d[2] = p_th / r2;
-    d[3] = p_phi / (r2 * s2);
-    d[4] = (-a * ((p_t * p_t) / (f * f)) - a * (p_r * p_r)) + ((p_th * p_th) + pp2 / s2) / r3;
-    d[5] = tc.c * pp2 / (r2 * s2 * tc.s);
-#else
-    // Same expressions with the nine divisions replaced by products of three reciprocals
+    // The reference's expressions with its nine divisions replaced by products of three reciprocals
     // (1/r, 1/f and, off the equator only, 1/sin theta): every term within a few ulp of the
     // reference's.  That is the level at which scipy's own BLAS stage sums already differ from
     // any restatement, and it removes most of the FP64-pipe work of an evaluation (an IEEE
@@ -133,7 +120,6 @@ __device__ __forceinline__ void rk_rhs(double R_S, double r_floor, double p_t, d
     d[3] = p_phi * ir2 * is2;
     d[4] = fma(-a, fma(ptf, ptf, p_r * p_r), fma(pp2, is2, p_th * p_th) * ir3);
     d[5] = tc.c * pp2 * ir2 * is2 * is1;
-#endif
 }
 
 // Kerr.geodesic_equations (metrics.py:946-1029) for the moving components (same six: p_t and
@@ -270,19 +256,10 @@ __device__ __forceinline__ void rk_f<1>(const Rk45Args &a, double r_floor, doubl
     rk_rhs_kerr(a.kerr_M, a.kerr_a, r_floor, p_t, p_phi, y, tc, d);
 }
 
-// NSM: the stage derivatives K[1] .. K[NSM] live in shared memory ([row][thread], conflict-free
-// 8-byte accesses) instead of registers.  With all seven stage vectors in registers the kernel
-// needs 168+ registers (12 warps per SM) and is bound by the latency of its dependent FP64 chains
-// (ncu round 1: FP64 pipe 52 %, issue 50 %, top stall `wait`); parking the stages that are only
-// read by later stage sums frees ~8 registers per row, and more resident warps hide that latency.
-// Same arithmetic in the same order: results are bit-identical for every NSM.
-template <int MINB, int METRIC, bool DENSE = false, int NSM = 0, int BLOCK = RK_BLOCK>
-__global__ void __launch_bounds__(BLOCK, MINB)
+template <int MINB, int METRIC, bool DENSE = false>
+__global__ void __launch_bounds__(RK_BLOCK, MINB)
 lp_rk45_kernel(const Rk45Args a)
 {
-    extern __shared__ double rk_ksm_all[];
-    double *const ksm = rk_ksm_all + threadIdx.x;
-#define KGET(j, i) ((((j) >= 1) && ((j) <= NSM)) ? ksm[(((j) - 1) * RK_NC + (i)) * BLOCK] : K[j][i])
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
     const long long warp_id = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -429,26 +406,19 @@ lp_rk45_kernel(const Rk45Args a)
                 for (int i = 0; i < RK_NC; ++i) {
                     double dy = K[0][i] * c_A[s][0];
 #pragma unroll
-                    for (int j = 1; j < s; ++j) dy = fma(KGET(j, i), c_A[s][j], dy);
+                    for (int j = 1; j < s; ++j) dy = fma(K[j][i], c_A[s][j], dy);
                     ys[i] = fma(dy, h, y[i]);
                 }
-                if (s <= NSM) {
-                    double kd[RK_NC];
-                    rk_f<METRIC>(a, r_floor, p_t, p_phi, ys, tc, kd);
-#pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) ksm[((s - 1) * RK_NC + i) * BLOCK] = kd[i];
-                } else {
-                    rk_f<METRIC>(a, r_floor, p_t, p_phi, ys, tc, K[s]);
-                }
+                rk_f<METRIC>(a, r_floor, p_t, p_phi, ys, tc, K[s]);
             }
             double y_new[RK_NC];
 #pragma unroll
             for (int i = 0; i < RK_NC; ++i) {
                 double acc = K[0][i] * c_B[0];
-                acc = fma(KGET(2, i), c_B[2], acc);
-                acc = fma(KGET(3, i), c_B[3], acc);
-                acc = fma(KGET(4, i), c_B[4], acc);
-                acc = fma(KGET(5, i), c_B[5], acc);
+                acc = fma(K[2][i], c_B[2], acc);
+                acc = fma(K[3][i], c_B[3], acc);
+                acc = fma(K[4][i], c_B[4], acc);
+                acc = fma(K[5][i], c_B[5], acc);
                 y_new[i] = fma(h, acc, y[i]);
             }
             rk_f<METRIC>(a, r_floor, p_t, p_phi, y_new, tc, K[6]);
@@ -461,10 +431,10 @@ lp_rk45_kernel(const Rk45Args a)
             for (int i = 0; i < RK_NC; ++i) {
                 es[i] = atol + max_sel(fabs(y[i]), fabs(y_new[i])) * rtol;
                 double acc = K[0][i] * c_E[0];
-                acc = fma(KGET(2, i), c_E[2], acc);
-                acc = fma(KGET(3, i), c_E[3], acc);
-                acc = fma(KGET(4, i), c_E[4], acc);
-                acc = fma(KGET(5, i), c_E[5], acc);
+                acc = fma(K[2][i], c_E[2], acc);
+                acc = fma(K[3][i], c_E[3], acc);
+                acc = fma(K[4][i], c_E[4], acc);
+                acc = fma(K[5][i], c_E[5], acc);
                 acc = fma(K[6][i], c_E[6], acc);
                 en[i] = acc * h;
             }
@@ -509,7 +479,7 @@ lp_rk45_kernel(const Rk45Args a)
                     for (int m = 0; m < 4; ++m) {
                         double acc = K[0][1] * c_P[0][m];
 #pragma unroll
-                        for (int j = 2; j < 7; ++j) acc = fma(KGET(j, 1), c_P[j][m], acc);
+                        for (int j = 2; j < 7; ++j) acc = fma(K[j][1], c_P[j][m], acc);
                         q[m] = acc;
                     }
                     double root = 0.0;
@@ -528,7 +498,7 @@ lp_rk45_kernel(const Rk45Args a)
                         for (int m = 0; m < 4; ++m) {
                             double acc = K[0][i] * c_P[0][m];
 #pragma unroll
-                            for (int j = 2; j < 7; ++j) acc = fma(KGET(j, i), c_P[j][m], acc);
+                            for (int j = 2; j < 7; ++j) acc = fma(K[j][i], c_P[j][m], acc);
                             qi[m] = acc;
                         }
                         yf[i] = dense_comp(qi, h, y[i], x);
@@ -545,7 +515,7 @@ lp_rk45_kernel(const Rk45Args a)
                         for (int m = 0; m < 4; ++m) {
                             double acc = K[0][i] * c_P[0][m];
 #pragma unroll
-                            for (int j = 2; j < 7; ++j) acc = fma(KGET(j, i), c_P[j][m], acc);
+                            for (int j = 2; j < 7; ++j) acc = fma(K[j][i], c_P[j][m], acc);
                             row[1 + 4 * i + m] = acc;
                         }
                     }
@@ -576,7 +546,6 @@ lp_rk45_kernel(const Rk45Args a)
             active = false;
         }
     }
-#undef KGET
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -900,30 +869,6 @@ static int rk45_launch_eq(const Rk45Args &a, cudaStream_t stream)
     return lp_check_launch();
 }
 
-template <int MINB, int NSM, int BLOCK>
-static int rk45_launch_variant(const Rk45Args &a, cudaStream_t stream)
-{
-    auto k = lp_rk45_kernel<MINB, 0, false, NSM, BLOCK>;
-    const size_t smem = (size_t)NSM * RK_NC * BLOCK * sizeof(double);
-    if (smem > 48 * 1024 &&
-        cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-        cudaGetLastError();
-        return LP_ERR_UNSUPPORTED;
-    }
-    if (cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, 100) != cudaSuccess) cudaGetLastError();
-    int dev = 0, sms = 0, per_sm = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, BLOCK, smem) != cudaSuccess) {
-        cudaGetLastError();
-        return LP_ERR_CUDA;
-    }
-    long long grid = (long long)sms * (per_sm < 1 ? 1 : per_sm);
-    const long long chunks = (a.n + BLOCK - 1) / BLOCK;
-    if (chunks < grid) grid = chunks;
-    k<<<(unsigned)grid, BLOCK, smem, stream>>>(a);
-    return lp_check_launch();
-}
-
 static int rk45_launch(bool metric_is_kerr, double kerr_a, const double *alphas, const double *state0, int64_t n,
                        double M, double R_S, double r_obs,
                        double lambda_max, double rtol, double atol, double max_step,
@@ -980,13 +925,6 @@ static int rk45_launch(bool metric_is_kerr, double kerr_a, const double *alphas,
     }
     a.fast_pow = fast_pow < 0 ? 0 : fast_pow;
     const bool kerr = metric_is_kerr;
-    // LP_RK45_VARIANT (tuning knob, Schwarzschild batch path): how many stage vectors are parked in shared
-    // memory / threads per CTA / resident CTAs per SM (the register cap follows from the last two)
-    static int variant = -1;
-    if (variant < 0) {
-        const char *e = getenv("LP_RK45_VARIANT");
-        variant = e ? atoi(e) : RK_DEFAULT_VARIANT;
-    }
     // LP_RK45_EQ = 0 | 1: the equatorial four-component kernel for the `alphas` batch entry (no trajectory)
     static int eq = -1, eq_minb = 0;
     if (eq < 0) {
@@ -1003,17 +941,6 @@ static int rk45_launch(bool metric_is_kerr, double kerr_a, const double *alphas,
         case 4: return rk45_launch_eq<4>(a, stream);
         case 5: return rk45_launch_eq<5>(a, stream);
         default: return rk45_launch_eq<6>(a, stream);
-        }
-    }
-    if (!kerr && !dense && variant > 0) {
-        switch (variant) {
-        case 1: return rk45_launch_variant<8, 4, 64>(a, stream);     // 128 registers, 16 warps / SM
-        case 2: return rk45_launch_variant<7, 3, 64>(a, stream);     // 144 registers, 14 warps / SM
-        case 3: return rk45_launch_variant<4, 4, 128>(a, stream);    // 128 registers, 16 warps / SM
-        case 4: return rk45_launch_variant<9, 5, 64>(a, stream);     // 112 registers, 18 warps / SM
-        case 5: return rk45_launch_variant<6, 0, 64>(a, stream);     // 168 registers, 12 warps / SM, small CTAs
-        case 6: return rk45_launch_variant<10, 5, 64>(a, stream);    // 96 registers, 20 warps / SM
-        default: break;
         }
     }
     if (dense) {            // single-ray API (OdeResult.sol): the variant that also stores every step's interpolant

@@ -12,8 +12,6 @@
 
 #define LP_RENDER_DEFAULT_TRIP 4
 #define LP_RENDER_DEFAULT_TILE_H 4
-#define LP_RENDER_DEFAULT_DYN 0
-#define LP_RENDER_DEFAULT_SPAN 2
 #define LP_TRACE_DEFAULT_BLOCK 256  /* rays per CTA; LP_TRACE_BLOCK=32|64|128|256 overrides (tuning).  Measured on the
                                        14-instruction kernel (profiles/r2af_knob_sweep*.log): 256 is 4 % faster than 64 at 4K
                                        and 8K, 8-9 % on 1080p / divergent frames (with the 18-instruction step of the first
@@ -254,54 +252,9 @@ extern "C" int lp_schw_trace_frame(const lp_camera *h_cam, int32_t row0, int32_t
 // Same per-ray code as the kernels above followed by remap_pixel() on the float32-rounded
 // result, so the output is bit-identical to trace_frame + remap run back to back.
 // ---------------------------------------------------------------------------
-// Work distribution of the frame kernel (a.dyn_tickets):
-//   0  one warp tile (32 pixels) per warp, one CTA per blockDim.x pixels, CTAs back-filled by the
-//      hardware work distributor;
-//   >0 a resident grid whose warps DRAW their warp tiles from a ticket counter (atomicAdd, one ticket
-//      = a.dyn_span consecutive warp tiles, the next ticket is requested before the current tiles are
-//      traced so its latency is hidden).  The SMSP scheduler issues greedily from the warp it issued
-//      from last and otherwise prefers older warps (ncu source view, round 2: the FP64 instructions
-//      of the low-ILP per-ray head of a freshly launched CTA wait ~20x longer for an issue slot than
-//      those of the RK4 loop); with a static split that unfairness leaves the slow warps to finish
-//      alone (LP_RENDER_SEQ > 1 measures it), with tickets a slow warp simply draws fewer tiles.
-//      The counter resets itself: every warp draws exactly one ticket beyond the last tile, and the
-//      warp that draws the very last of those (a.dyn_tickets + warps - 1) stores zero.
-#define LP_TICKET_SLOTS 256
-#define LP_TICKET_STRIDE 32          /* one counter per 128-byte line */
-__device__ unsigned int g_lp_tickets[LP_TICKET_SLOTS * LP_TICKET_STRIDE];
-
-// warp-level statistics flush (the ticket schedule has no CTA-wide rendezvous)
-static __device__ __forceinline__ void lp_stats_flush_warp(const StatAcc &a, unsigned long long n_rays_thread,
-                                                           lp_frame_stats *g)
-{
-    const unsigned full = 0xffffffffu;
-    unsigned long long v[7] = { n_rays_thread, a.escaped, a.captured, a.invalid, a.winding, a.sum_steps, a.warp_steps };
-    unsigned int mx0 = a.max_steps, mx1 = a.max_winding;
-    unsigned long long mn = dbl_to_ordered(a.min_fa), mxf = dbl_to_ordered(a.max_fa);
-    for (int off = 16; off > 0; off >>= 1) {
-#pragma unroll
-        for (int i = 0; i < 7; ++i) v[i] += __shfl_xor_sync(full, v[i], off);
-        mx0 = max(mx0, __shfl_xor_sync(full, mx0, off));
-        mx1 = max(mx1, __shfl_xor_sync(full, mx1, off));
-        mn = min(mn, __shfl_xor_sync(full, mn, off));
-        mxf = max(mxf, __shfl_xor_sync(full, mxf, off));
-    }
-    if ((threadIdx.x & 31) == 0) {
-        atomicAdd((unsigned long long *)&g->n_rays, v[0]);
-        atomicAdd((unsigned long long *)&g->n_escaped, v[1]);
-        atomicAdd((unsigned long long *)&g->n_captured, v[2]);
-        atomicAdd((unsigned long long *)&g->n_invalid, v[3]);
-        atomicAdd((unsigned long long *)&g->n_winding, v[4]);
-        atomicAdd((unsigned long long *)&g->sum_steps, v[5]);
-        atomicAdd((unsigned long long *)&g->sum_warp_steps, v[6]);
-        atomicMax(&g->max_steps, mx0);
-        atomicMax(&g->max_winding, mx1);
-        atomicMin((unsigned long long *)&g->min_final_alpha, mn);
-        atomicMax((unsigned long long *)&g->max_final_alpha, mxf);
-    }
-}
-
-template <bool FUSED, bool FAST, typename T, int MINB, int TRIP, bool DYN = false>
+// One warp tile (32 pixels) per warp, one CTA per blockDim.x pixels, CTAs back-filled by the hardware
+// work distributor.
+template <bool FUSED, bool FAST, typename T, int MINB, int TRIP>
 __global__ void __launch_bounds__(LP_TRACE_BLOCK, MINB)
 lp_render_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts c, const CamConsts cam)
 {
@@ -312,81 +265,54 @@ lp_render_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts c, con
     // destinations need (dist.PeerFrame).
     __shared__ __align__(16) float stage[LP_TRACE_BLOCK / 32][96];
     const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
-    const bool dyn = DYN;
-    unsigned int *const tickets = g_lp_tickets + a.dyn_slot * LP_TICKET_STRIDE;
-    const unsigned int n_warps = gridDim.x * (blockDim.x >> 5);
-    unsigned int cur = 0, nxt = 0;       // current ticket (warp-uniform); the next one (lane 0, requested early)
-    if (dyn) {
-        if (lane == 0) cur = atomicAdd(tickets, 1u);
-        cur = __shfl_sync(0xffffffffu, cur, 0);
+    const long long wt = (long long)blockIdx.x * (blockDim.x >> 5) + wrp;
+    const long long i = wt * 32 + lane;
+    const bool live = i < a.n;
+    const bool vec = (sizeof(T) == 4 || sizeof(T) == 1) && ra.vec_ok && (wt * 32 + 31 < a.n);      // warp-uniform
+    RayResult r;
+    r.status = 0; r.steps = 0; r.nh = 0; r.fa = 0.0;
+    int tr = 0, col = 0;
+    if (live) {
+        warp_tile_rc(a, cam.width, i, tr, col);
+        const int row = tile_row(a, tr);
+        const long long pi = (long long)tr * cam.width + col;                    // compact tile index
+        const double xc = cam_x(cam, col), yc = cam_y(cam, row);     // also the remap's (kept across the loop)
+        const float a32 = (float)pixel_alpha64(cam, xc, yc);
+        binet_trace<FUSED, FAST, TRIP>(c, L, (double)a32, r);
+        if (FUSED && hybrid_needs_retrace(r, a.retrace_steps, a.retrace_steps_small, a.retrace_h, a.retrace_off))
+            binet_trace<false, FAST>(c, load_loop_regs<false>(c), (double)a32, r);   // cold
+        const float fa32 = (float)((r.status == 1) ? r.fa : __longlong_as_double(0x7ff8000000000000LL));
+        const long long nh = r.nh < 0 ? 0 : (r.nh > 65535 ? 65535 : r.nh);
+        if (a.out_fa) ((float *)a.out_fa)[pi] = fa32;
+        if (a.out_w) ((unsigned short *)a.out_w)[pi] = (unsigned short)nh;
+        const long long oi = a.out_frame_rows ? (long long)(row - a.row0) * cam.width + col : pi;
+        // two call sites so that each store has a known address space (shared / global) instead of
+        // a generic pointer
+        if (vec) remap_pixel_xy<T, true>(ra, cam, (T *)&stage[wrp][0] + lane * 3, xc, yc, fa32, (unsigned)nh, r.fa, r.cf, r.sf);
+        else remap_pixel_xy<T, true>(ra, cam, (T *)ra.out + oi * ra.channels, xc, yc, fa32, (unsigned)nh, r.fa, r.cf, r.sf);
     }
-    // warp tiles [wt, wt_end) of this pass
-    long long wt = dyn ? (long long)cur * a.dyn_span : (long long)blockIdx.x * (blockDim.x >> 5) + wrp;
-    long long wt_end = dyn ? wt + a.dyn_span : wt + 1;
-#pragma unroll 1
-    for (;;) {
-        if (dyn) {
-            if (cur >= (unsigned)a.dyn_tickets) {
-                if (lane == 0 && cur == (unsigned)a.dyn_tickets + n_warps - 1u) *tickets = 0u;   // last draw of the launch
-                break;
-            }
-            if (lane == 0 && wt == (long long)cur * a.dyn_span) nxt = atomicAdd(tickets, 1u);   // hidden behind the tiles
+    if (vec) {
+        // vec_ok (host): every run of the warp tile is contiguous in the output and starts on a
+        // vector boundary.  Vector v of the staged 96 floats / bytes belongs to run v / per_run.
+        __syncwarp();
+        const int r0 = __shfl_sync(0xffffffffu, tr, 0), c0 = __shfl_sync(0xffffffffu, col, 0);
+        if (lane < a.st_lanes) {
+            const int run = (int)(((unsigned)lane * a.st_magic) >> 16), part = lane - run * a.st_per_run;
+            const int rr = r0 + run;
+            const long long o0 = a.out_frame_rows ? (long long)(tile_row(a, rr) - a.row0) * cam.width + c0
+                                                  : (long long)rr * cam.width + c0;
+            unsigned char *g = (unsigned char *)((T *)ra.out + o0 * 3) + part * a.st_vb;
+            const unsigned char *sm = (const unsigned char *)stage[wrp] + run * a.st_run_bytes + part * a.st_vb;
+            if (a.st_vb == 16) *reinterpret_cast<uint4 *>(g) = *reinterpret_cast<const uint4 *>(sm);
+            else *reinterpret_cast<uint2 *>(g) = *reinterpret_cast<const uint2 *>(sm);
         }
-        const long long i = wt * 32 + lane;
-        const bool live = i < a.n;
-        const bool vec = (sizeof(T) == 4 || sizeof(T) == 1) && ra.vec_ok && (wt * 32 + 31 < a.n);      // warp-uniform
-        RayResult r;
-        r.status = 0; r.steps = 0; r.nh = 0; r.fa = 0.0;
-        int tr = 0, col = 0;
-        if (live) {
-            warp_tile_rc(a, cam.width, i, tr, col);
-            const int row = tile_row(a, tr);
-            const long long pi = (long long)tr * cam.width + col;                    // compact tile index
-            const double xc = cam_x(cam, col), yc = cam_y(cam, row);     // also the remap's (kept across the loop)
-            const float a32 = (float)pixel_alpha64(cam, xc, yc);
-            binet_trace<FUSED, FAST, TRIP>(c, L, (double)a32, r);
-            if (FUSED && hybrid_needs_retrace(r, a.retrace_steps, a.retrace_steps_small, a.retrace_h, a.retrace_off))
-                binet_trace<false, FAST>(c, load_loop_regs<false>(c), (double)a32, r);   // cold
-            const float fa32 = (float)((r.status == 1) ? r.fa : __longlong_as_double(0x7ff8000000000000LL));
-            const long long nh = r.nh < 0 ? 0 : (r.nh > 65535 ? 65535 : r.nh);
-            if (a.out_fa) ((float *)a.out_fa)[pi] = fa32;
-            if (a.out_w) ((unsigned short *)a.out_w)[pi] = (unsigned short)nh;
-            const long long oi = a.out_frame_rows ? (long long)(row - a.row0) * cam.width + col : pi;
-            // two call sites so that each store has a known address space (shared / global) instead of
-            // a generic pointer
-            if (vec) remap_pixel_xy<T, true>(ra, cam, (T *)&stage[wrp][0] + lane * 3, xc, yc, fa32, (unsigned)nh, r.fa, r.cf, r.sf);
-            else remap_pixel_xy<T, true>(ra, cam, (T *)ra.out + oi * ra.channels, xc, yc, fa32, (unsigned)nh, r.fa, r.cf, r.sf);
-        }
-        if (vec) {
-            // vec_ok (host): every run of the warp tile is contiguous in the output and starts on a
-            // vector boundary.  Vector v of the staged 96 floats / bytes belongs to run v / per_run.
-            __syncwarp();
-            const int r0 = __shfl_sync(0xffffffffu, tr, 0), c0 = __shfl_sync(0xffffffffu, col, 0);
-            if (lane < a.st_lanes) {
-                const int run = (int)(((unsigned)lane * a.st_magic) >> 16), part = lane - run * a.st_per_run;
-                const int rr = r0 + run;
-                const long long o0 = a.out_frame_rows ? (long long)(tile_row(a, rr) - a.row0) * cam.width + c0
-                                                      : (long long)rr * cam.width + c0;
-                unsigned char *g = (unsigned char *)((T *)ra.out + o0 * 3) + part * a.st_vb;
-                const unsigned char *sm = (const unsigned char *)stage[wrp] + run * a.st_run_bytes + part * a.st_vb;
-                if (a.st_vb == 16) *reinterpret_cast<uint4 *>(g) = *reinterpret_cast<const uint4 *>(sm);
-                else *reinterpret_cast<uint2 *>(g) = *reinterpret_cast<const uint2 *>(sm);
-            }
-            __syncwarp();      // the staging slots are reused by the warp's next tile
-        }
-        if (a.stats) {
-            StatAcc acc;
-            acc.init();
-            acc.add(r, live);
-            if (dyn) lp_stats_flush_warp(acc, live ? 1ull : 0ull, a.stats);
-            else lp_stats_flush(acc, live ? 1ull : 0ull, a.stats);         // CTA-uniform: one pass per CTA
-        }
-        if (!dyn) break;
-        if (++wt == wt_end) {                                   // ticket exhausted: move to the one requested above
-            cur = __shfl_sync(0xffffffffu, nxt, 0);
-            wt = (long long)cur * a.dyn_span;
-            wt_end = wt + a.dyn_span;
-        }
+        __syncwarp();      // reconverge the warp after the lane-divergent stores
+    }
+    if (a.stats) {
+        StatAcc acc;
+        acc.init();
+        acc.add(r, live);
+        lp_stats_flush(acc, live ? 1ull : 0ull, a.stats);         // CTA-uniform: one pass per CTA
     }
 }
 
@@ -513,83 +439,28 @@ static int render_trip(long long n_rays)
     return n_rays >= LP_RENDER_TRIP4_MIN_RAYS ? 4 : 2;
 }
 
-// LP_RENDER_DYN=0|1 (tuning knob): ticket-drawing resident grid (see lp_render_kernel) or one CTA per
-// blockDim.x pixels; LP_RENDER_SPAN = warp tiles per ticket.
-static int render_dyn()
-{
-    static int cached = -1;
-    if (cached < 0) {
-        const char *e = getenv("LP_RENDER_DYN");
-        cached = e ? (atoi(e) != 0) : LP_RENDER_DEFAULT_DYN;
-    }
-    return cached;
-}
-static int render_span()
-{
-    static int cached = 0;
-    if (!cached) {
-        const char *e = getenv("LP_RENDER_SPAN");
-        const int v = e ? atoi(e) : 0;
-        cached = (v >= 1 && v <= 64) ? v : LP_RENDER_DEFAULT_SPAN;
-    }
-    return cached;
-}
-
-template <typename T, int MINB>
-static int launch_render_mb(const TraceArgs &a_in, const RemapArgs &ra, const BinetConsts &c,
-                            const CamConsts &cam, uint32_t flags, cudaStream_t stream)
-{
-    const bool fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
-    const bool icmp = (fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) != 0;
-    const int block = trace_block_size();
-    const long long chunks = (a_in.n + block - 1) / block;
-    if (chunks > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
-    TraceArgs a = a_in;
-    unsigned grid = (unsigned)chunks;
-    a.dyn_tickets = 0; a.dyn_span = 1; a.dyn_slot = 0;
-    const long long warp_tiles = (a.n + 31) / 32;
-    if (render_dyn()) {
-        // resident grid: as many CTAs as fit (occupancy of the default instantiation; every variant is
-        // bounded by the same 64 registers); frames smaller than one wave keep the plain schedule
-        static int resident = 0;
-        if (!resident) {
-            int g = 0;
-            if (lp_grid_for((const void *)lp_render_kernel<true, true, T, MINB, 4, true>, block, &g) != LP_OK) return LP_ERR_CUDA;
-            resident = g;
-        }
-        const int span = render_span();
-        const long long tickets = (warp_tiles + span - 1) / span;
-        // (the ticket schedule is instantiated for the default arithmetic only: FMA loop, fast path, 4-step trips)
-        if (chunks > resident && tickets < 0x7fffffffLL - 0x100000 && fused && icmp && render_trip(a.n) == 4) {
-            static unsigned next_slot = 0;
-            a.dyn_tickets = (int32_t)tickets; a.dyn_span = span;
-            a.dyn_slot = (int32_t)(__atomic_fetch_add(&next_slot, 1u, __ATOMIC_RELAXED) % LP_TICKET_SLOTS);
-            grid = (unsigned)resident;
-        }
-    }
-    if (a.dyn_tickets > 0) {
-        lp_render_kernel<true, true, T, MINB, 4, true><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        return lp_check_launch();
-    }
-    if (fused) {
-        if (icmp && render_trip(a.n) == 4) lp_render_kernel<true, true, T, MINB, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else if (icmp) lp_render_kernel<true, true, T, MINB, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else      lp_render_kernel<true, false, T, MINB, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-    } else {
-        if (icmp && render_trip(a.n) == 4) lp_render_kernel<false, true, T, MINB, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else if (icmp) lp_render_kernel<false, true, T, MINB, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else      lp_render_kernel<false, false, T, MINB, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-    }
-    return lp_check_launch();
-}
-
 // MINB = 4 CTAs of LP_TRACE_BLOCK threads per SM -> ptxas keeps the kernel at 64 registers
 // (32 warps/SM); a 48-register build (40 warps/SM, spills outside the loop) measured 1 % slower.
 template <typename T>
 static int launch_render(const TraceArgs &a, const RemapArgs &ra, const BinetConsts &c,
                          const CamConsts &cam, uint32_t flags, cudaStream_t stream)
 {
-    return launch_render_mb<T, 4>(a, ra, c, cam, flags, stream);
+    const bool fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
+    const bool icmp = (fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) != 0;
+    const int block = trace_block_size();
+    const long long chunks = (a.n + block - 1) / block;
+    if (chunks > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
+    const unsigned grid = (unsigned)chunks;
+    if (fused) {
+        if (icmp && render_trip(a.n) == 4) lp_render_kernel<true, true, T, 4, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
+        else if (icmp) lp_render_kernel<true, true, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+        else      lp_render_kernel<true, false, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+    } else {
+        if (icmp && render_trip(a.n) == 4) lp_render_kernel<false, true, T, 4, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
+        else if (icmp) lp_render_kernel<false, true, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+        else      lp_render_kernel<false, false, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+    }
+    return lp_check_launch();
 }
 
 // The mirror-image kernel for a contiguous row tile: x mirror when mir_x, y mirror when mir_y (whole frame).
@@ -720,8 +591,7 @@ extern "C" int lp_render_frame_bands(const void *src, int32_t src_dtype, int32_t
     }
     // mirror images (lp_render_mirror_kernel): contiguous rows stored compactly, default schedule; x needs
     // d0 == 0 (either sign), y needs d1 == 0 and the whole frame, both need d2 != 0
-    const bool mir_ok = band_rows == 0 && !(flags & (LP_RENDER_OUT_FRAME_ROWS | LP_RENDER_ROW_RUNS)) &&
-                        !render_dyn() && cam.d2 != 0.0;
+    const bool mir_ok = band_rows == 0 && !(flags & (LP_RENDER_OUT_FRAME_ROWS | LP_RENDER_ROW_RUNS)) && cam.d2 != 0.0;
     const bool mir_x = mir_ok && cam.d0 == 0.0;
     const bool mir_y = mir_ok && cam.d1 == 0.0 && row0 == 0 && rows == cam.height;
     if (mir_x || mir_y) {

@@ -35,9 +35,8 @@ struct TraceArgs {
     // tile_shift = log2(tile_h); tiles_x_magic = ceil(2^32 / tiles_x) when the host has verified that
     // __umulhi(w, magic) == w / tiles_x for every warp tile index w of this launch, else 0 (plain division)
     uint32_t tile_shift, tiles_x_magic;
-    // frame kernel, ticket schedule (lp_trace.cu): tickets in this launch (0 = static one tile per warp),
-    // warp tiles per ticket, counter slot
-    int32_t dyn_tickets, dyn_span, dyn_slot;
+    uint32_t m_warps;       // mirror-image frame kernel: warp tiles in the launch (placed here so that the
+                            // 4-byte fields below share 8-byte words in pairs as the kernels load them)
     // staged stores of the frame kernel (host-side arithmetic of the warp's write-out, so that the kernel
     // has no integer division): bytes of one run of the warp tile, vector width (16 / 8), vectors per run,
     // lanes that store (tile_h * per_run), and ceil(2^16 / per_run) for lane / per_run by multiply-shift
@@ -49,7 +48,7 @@ struct TraceArgs {
     // in y when k & 2; the images with k & mir_skip do not exist in this launch.
     int32_t mir_skip;
     int32_t mx_main, mx_base, mtx_main, my_main, my_base, mty_main;
-    uint32_t mtiles_x, m_warps;     // warp tiles per tile row, warp tiles in the launch
+    uint32_t mtiles_x;      // warp tiles per tile row
 };
 
 // frame row of tile-local row r (interleaved bands, see above)

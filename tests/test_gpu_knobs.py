@@ -1,10 +1,9 @@
 """GPU parity of the opt-in KERNEL VARIANTS that are selected by environment knobs (the library reads a
-knob once per process, so every variant renders in its own subprocess): the ticket-drawing resident
-grid of the frame kernel (LP_RENDER_DYN, lp_trace.cu), 2-step loop trips (LP_RENDER_TRIP), warp-tile
-shapes (LP_RENDER_TILE_H), CTA sizes (LP_TRACE_BLOCK) and the TMA-staged remap (LP_REMAP_TMA,
-lp_remap_tma.cu).  None of them may change a single output byte: they only move work between warps or
-stage the same source texels differently (reference: metrics.py:49-145, image_lens.py:133-178,
-:296-397)."""
+knob once per process, so every variant renders in its own subprocess): 2-step loop trips of the frame
+kernel (LP_RENDER_TRIP, lp_trace.cu), warp-tile shapes (LP_RENDER_TILE_H), CTA sizes (LP_TRACE_BLOCK)
+and the TMA-staged remap (LP_REMAP_TMA, lp_remap_tma.cu).  None of them may change a single output
+byte: they only move work between warps or stage the same source texels differently (reference:
+metrics.py:49-145, image_lens.py:133-178, :296-397)."""
 import hashlib
 import json
 import os
@@ -31,8 +30,8 @@ def digest(*ts):
         h.update(t.detach().cpu().contiguous().numpy().tobytes())
     return h.hexdigest()
 g = torch.Generator(device="cuda").manual_seed(7)
-# frames larger than one resident wave (the ticket schedule only engages there), a ragged one, a
-# close observer (divergent warps), a rotated camera, uint8 and float32, strict and hybrid
+# frames larger than one wave of CTAs, a ragged one, a close observer (divergent warps), a rotated
+# camera, uint8 and float32, strict and hybrid
 for (H, W, r_obs, vf, psi) in [(1080, 1920, 100.0, 40.0, (0.0, 0.0)), (1000, 1500, 15.0, 40.0, (0.04, -0.03)),
                                (1031, 1217, 30.0, 25.0, (0.0, 0.1)), (96, 128, 100.0, 12.0, (0.0, 0.0))]:
     vfov = np.radians(vf); fov = (2 * np.arctan(np.tan(vfov / 2) * W / H), vfov)
@@ -60,7 +59,7 @@ print("RESULT " + json.dumps(out, sort_keys=True))
 
 def _run(env_extra):
     env = dict(os.environ)
-    for k in ("LP_RENDER_DYN", "LP_RENDER_SPAN", "LP_RENDER_TRIP", "LP_RENDER_TILE_H", "LP_TRACE_BLOCK", "LP_REMAP_TMA"):
+    for k in ("LP_RENDER_TRIP", "LP_RENDER_TILE_H", "LP_TRACE_BLOCK", "LP_REMAP_TMA"):
         env.pop(k, None)
     env.update(env_extra)
     r = subprocess.run([sys.executable, "-c", CHILD % {"root": ROOT}], env=env, capture_output=True, text=True,
@@ -76,12 +75,10 @@ def default_outputs(native):
 
 
 @pytest.mark.parametrize("knobs", [
-    {"LP_RENDER_DYN": "1"},
-    {"LP_RENDER_DYN": "1", "LP_RENDER_SPAN": "5"},
     {"LP_RENDER_TRIP": "2"},
     {"LP_RENDER_TILE_H": "1"},
     {"LP_RENDER_TILE_H": "2", "LP_TRACE_BLOCK": "128"},
-    {"LP_TRACE_BLOCK": "32", "LP_RENDER_DYN": "1"},
+    {"LP_TRACE_BLOCK": "32"},
     {"LP_REMAP_TMA": "1"},
 ], ids=lambda k: ",".join("%s=%s" % kv for kv in sorted(k.items())))
 def test_knob_variants_are_bit_identical(native, default_outputs, knobs):
@@ -89,36 +86,3 @@ def test_knob_variants_are_bit_identical(native, default_outputs, knobs):
     assert set(got) == set(default_outputs)
     differing = [k for k in got if got[k] != default_outputs[k]]
     assert not differing, "outputs differ under %s: %s" % (knobs, differing)
-
-
-def test_ticket_counters_reset_themselves(native):
-    """The ticket schedule's counters are module-scope device words that every launch must leave at
-    zero: 600 launches (more than the 256 slots, so every slot is reused) of frames of different
-    sizes in one process give the frames of the default schedule."""
-    code = r'''
-import sys, hashlib
-import numpy as np, torch
-sys.path.insert(0, %(root)r)
-from light_path_tracer_b200 import image_lens as il
-from light_path_tracer_b200.metrics import Schwarzschild
-m = Schwarzschild(1.0)
-h = hashlib.sha256()
-srcs = {}
-for i in range(600):
-    H, W = [(1080, 1920), (720, 1280), (1000, 1504)][i %% 3]
-    vfov = np.radians(40.0); fov = (2 * np.arctan(np.tan(vfov / 2) * W / H), vfov)
-    if (H, W) not in srcs:
-        srcs[(H, W)] = (torch.rand(H, W, 3, device="cuda", generator=torch.Generator(device="cuda").manual_seed(H)) * 255).to(torch.uint8)
-    out = il.render_frame(srcs[(H, W)], fov, 100.0 + (i %% 7), m, flags=4 | 8, unit_u8=True)
-    if i %% 50 == 0 or i > 590:
-        h.update(out.cpu().numpy().tobytes())
-print("RESULT " + h.hexdigest())
-'''
-    outs = []
-    for dyn in ("0", "1"):
-        env = dict(os.environ, LP_RENDER_DYN=dyn)
-        r = subprocess.run([sys.executable, "-c", code % {"root": ROOT}], env=env, capture_output=True, text=True,
-                           timeout=600)
-        assert r.returncode == 0, r.stderr[-2000:]
-        outs.append([l for l in r.stdout.splitlines() if l.startswith("RESULT ")][-1])
-    assert outs[0] == outs[1]

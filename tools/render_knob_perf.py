@@ -1,7 +1,7 @@
 """Frame-kernel timing under one tuning knob (the library reads knobs once per process, so every value
 runs in its own subprocess).
 
-    python tools/render_knob_perf.py LP_RENDER_SEQ 1 2 4 8
+    python tools/render_knob_perf.py LP_RENDER_TRIP 2 4
 """
 import os
 import subprocess
