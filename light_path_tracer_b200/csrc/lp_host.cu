@@ -43,8 +43,9 @@ int lp_check_launch(void)
     return cudaGetLastError() == cudaSuccess ? LP_OK : LP_ERR_CUDA;
 }
 
-// Persistent grid: (resident CTAs per SM) x (SM count) for this kernel / block size.
-int lp_grid_for(const void *kernel, int block, int *grid_out)
+// Persistent grid: (resident CTAs per SM) x (SM count) for this kernel / block size, but no more CTAs
+// than the n items fill (ceil(n / block)).
+int lp_grid_for(const void *kernel, int block, long long n, int *grid_out)
 {
     int dev = 0, sms = 0, per_sm = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) { cudaGetLastError(); return LP_ERR_CUDA; }
@@ -52,6 +53,8 @@ int lp_grid_for(const void *kernel, int block, int *grid_out)
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, block, 0) != cudaSuccess) { cudaGetLastError(); return LP_ERR_CUDA; }
     if (per_sm < 1) per_sm = 1;
     *grid_out = sms * per_sm;
+    const long long chunks = (n + block - 1) / block;
+    if (chunks < *grid_out) *grid_out = (int)chunks;
     return LP_OK;
 }
 

@@ -417,8 +417,6 @@ lp_kerr_kernel(const KerrArgs a, const CamConsts cam)
 {
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
-    const long long warp_id = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
     const double M = a.M, sp = a.a, r_floor = a.r_plus * 1.001;
     const double r_capture = a.r_plus * 1.01, r_escape = a.r_obs * 2.0, lambda_max = a.lambda_max;
     const double h_min = 1e-12;
@@ -433,8 +431,7 @@ lp_kerr_kernel(const KerrArgs a, const CamConsts cam)
     double p_t = -1.0, p_phi = 0.0, lam = 0.0, h = 1.0, atol = 1e-8, rtol = 1e-6;
     int accepted = 0, attempts = 0, iters = 0;
 
-    long long cursor = 0;
-    bool queue_empty = (warp_id * 32 >= a.n);
+    LpWarpQueue queue(a.n);
 
     while (true) {
         // ---------------- lane refill ----------------
@@ -449,12 +446,8 @@ lp_kerr_kernel(const KerrArgs a, const CamConsts cam)
             kerr_store_result(a, idx, status, fa, nh, accepted, attempts);
             pending = 0;
         }
-        if (flush && !queue_empty) {
-            const int rank = __popc(idle & ((1u << lane) - 1u));
-            const long long v = cursor + rank;
-            const long long ray = ((v >> 5) * n_warps + warp_id) * 32 + (v & 31);
-            cursor += __popc(idle);
-            if (((cursor >> 5) * n_warps + warp_id) * 32 + (cursor & 31) >= a.n) queue_empty = true;
+        if (flush && !queue.empty) {
+            const long long ray = queue.take(idle, lane);
             if (!active && ray < a.n) {
                 idx = ray;
                 double alpha, theta;
@@ -474,7 +467,7 @@ lp_kerr_kernel(const KerrArgs a, const CamConsts cam)
             }
         }
         if (!__any_sync(full, active)) {
-            if (queue_empty) break;
+            if (queue.empty) break;
             continue;
         }
         if (!active) continue;
@@ -521,8 +514,6 @@ lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
     const unsigned lt_mask = (1u << lane) - 1u;
-    const long long warp_id = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
     const double M = a.M, sp = a.a, r_floor = a.r_plus * 1.001;
     const double r_capture = a.r_plus * 1.01, r_escape = a.r_obs * 2.0, lambda_max = a.lambda_max;
     const double h_min = 1e-12;
@@ -538,15 +529,15 @@ lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
     double p_phi = 0.0, lam = 0.0, h = 1.0, atol = 1e-8, rtol = 1e-6;
     int accepted = 0, attempts = 0, iters = 0;
 
-    // warp-uniform queue state.  Chunk c of this warp = rays (c * n_warps + warp_id) * 32 + 0..31
+    // warp-uniform queue state: the warp's chunks of 32 rays (LpWarpQueue::chunk_ray), one chunk at a time
+    LpWarpQueue queue(a.n);
     long long chunk = 0, in_ray0 = 0;
     int in_base = 0, in_avail = 0, out_count = 0;
-    bool queue_empty = (warp_id * 32 >= a.n);
 
     while (true) {
         // ---------------- finished lanes -> out-queue ----------------
         const unsigned fin = __ballot_sync(full, pending != 0);
-        const bool last_round = !fin && queue_empty && in_avail == 0 && !__any_sync(full, active);
+        const bool last_round = !fin && queue.empty && in_avail == 0 && !__any_sync(full, active);
         if (out_count && (out_count + __popc(fin) > 32 || last_round)) {
             // all lanes together: final direction + stores for the gathered results
             __syncwarp();
@@ -591,9 +582,9 @@ lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
             const unsigned empty = __ballot_sync(full, !active);
             if (!empty) break;
             if (in_avail == 0) {
-                if (queue_empty) break;
+                if (queue.empty) break;
                 // all lanes together: initial conditions + FSAL seed of the next 32 rays
-                in_ray0 = (chunk * n_warps + warp_id) * 32;
+                in_ray0 = queue.chunk_ray(chunk);
                 const long long ray = in_ray0 + lane;
                 int flag = 0;
                 __syncwarp();
@@ -619,7 +610,7 @@ lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
                 in_avail = left < 32 ? (int)left : 32;
                 in_base = 0;
                 chunk++;
-                queue_empty = ((chunk * n_warps + warp_id) * 32 >= a.n);
+                queue.empty = (queue.chunk_ray(chunk) >= a.n);
             }
             const int rank = __popc(empty & lt_mask);
             if (!active && rank < in_avail) {
@@ -673,46 +664,31 @@ static int kerr_launch(KerrArgs &a, const CamConsts &cam, cudaStream_t stream)
     }
     a.refill_min = refill;
     // resident CTAs per SM ptxas must fit (register cap): the kernel is latency-bound, so more
-    // resident warps win until the spills cost more (LP_KERR_MINB = 2..6, tuning knob)
+    // resident warps win until the spills cost more (LP_KERR_MINB = 2..6, tuning knob; the queued
+    // kernel is built for 3..5 and runs 4 for the others)
     static int minb = 0;
     if (!minb) {
         const char *e = getenv("LP_KERR_MINB");
         const int v = e ? atoi(e) : 0;
         minb = (v >= 2 && v <= 6) ? v : KERR_DEFAULT_MINB;
     }
-#define KERR_DISPATCH(MB) \
-    do { \
-        int grid = 0; \
-        int rc = lp_grid_for((const void *)lp_kerr_kernel<MB>, KERR_BLOCK, &grid); \
-        if (rc != LP_OK) return rc; \
-        const long long chunks = (a.n + KERR_BLOCK - 1) / KERR_BLOCK; \
-        if (chunks < grid) grid = (int)chunks; \
-        lp_kerr_kernel<MB><<<grid, KERR_BLOCK, 0, stream>>>(a, cam); \
-    } while (0)
     const char *qe = getenv("LP_KERR_QUEUE");
     const bool queued = !(qe && atoi(qe) == 0);
-#define KERR_DISPATCH_Q(MB) \
-    do { \
-        int grid = 0; \
-        int rc = lp_grid_for((const void *)lp_kerr_queued_kernel<MB>, KERR_BLOCK, &grid); \
-        if (rc != LP_OK) return rc; \
-        const long long chunks = (a.n + KERR_BLOCK - 1) / KERR_BLOCK; \
-        if (chunks < grid) grid = (int)chunks; \
-        lp_kerr_queued_kernel<MB><<<grid, KERR_BLOCK, 0, stream>>>(a, cam); \
-    } while (0)
+    const void *fn;
     if (queued) {
-        if (minb == 3) { KERR_DISPATCH_Q(3); }
-        else if (minb == 5) { KERR_DISPATCH_Q(5); }
-        else { KERR_DISPATCH_Q(4); }
-        return lp_check_launch();
+        fn = minb == 3 ? (const void *)lp_kerr_queued_kernel<3>
+           : minb == 5 ? (const void *)lp_kerr_queued_kernel<5> : (const void *)lp_kerr_queued_kernel<4>;
+    } else {
+        const void *parked[] = {(const void *)lp_kerr_kernel<2>, (const void *)lp_kerr_kernel<3>,
+                                (const void *)lp_kerr_kernel<4>, (const void *)lp_kerr_kernel<5>,
+                                (const void *)lp_kerr_kernel<6>};
+        fn = parked[minb - 2];
     }
-#undef KERR_DISPATCH_Q
-    if (minb == 2) { KERR_DISPATCH(2); }
-    else if (minb == 3) { KERR_DISPATCH(3); }
-    else if (minb == 4) { KERR_DISPATCH(4); }
-    else if (minb == 5) { KERR_DISPATCH(5); }
-    else { KERR_DISPATCH(6); }
-#undef KERR_DISPATCH
+    int grid = 0;
+    const int rc = lp_grid_for(fn, KERR_BLOCK, a.n, &grid);
+    if (rc != LP_OK) return rc;
+    void *args[] = {&a, (void *)&cam};
+    cudaLaunchKernel(fn, grid, KERR_BLOCK, args, 0, stream);
     return lp_check_launch();
 }
 

@@ -233,10 +233,8 @@ extern "C" int lp_remap(const void *src, int32_t src_dtype, int32_t channels,
     default: return LP_ERR_INVALID_ARG;
     }
     int grid = 0;
-    rc = lp_grid_for(fn, 256, &grid);
+    rc = lp_grid_for(fn, 256, a.n, &grid);
     if (rc != LP_OK) return rc;
-    const long long chunks = (a.n + 255) / 256;
-    if (chunks < grid) grid = (int)chunks;
     switch (src_dtype) {
     case LP_DTYPE_U8: lp_remap_kernel<unsigned char><<<grid, 256, 0, st>>>(a, cam); break;
     case LP_DTYPE_F32: lp_remap_kernel<float><<<grid, 256, 0, st>>>(a, cam); break;

@@ -165,8 +165,12 @@ __device__ __forceinline__ void rk_rhs_kerr(double M, double a, double r_floor, 
 
 // METRIC 0: Schwarzschild (R_S), 1: Kerr (M, a)
 template <int METRIC>
-__device__ __forceinline__ void rk_f(const struct Rk45Args &a, double r_floor, double p_t, double p_phi,
-                                     const double (&y)[RK_NC], ThetaCache &tc, double (&d)[RK_NC]);
+__device__ __forceinline__ void rk_f(const Rk45Args &a, double r_floor, double p_t, double p_phi,
+                                     const double (&y)[RK_NC], ThetaCache &tc, double (&d)[RK_NC])
+{
+    if (METRIC == 0) rk_rhs(a.R_S, r_floor, p_t, p_phi, y, tc, d);
+    else rk_rhs_kerr(a.kerr_M, a.kerr_a, r_floor, p_t, p_phi, y, tc, d);
+}
 
 // Quartic dense output of one component (rk.py:723-737), sequential like the oracle.
 __device__ __forceinline__ double dense_comp(const double (&q)[4], double h, double y_old, double x)
@@ -177,6 +181,19 @@ __device__ __forceinline__ double dense_comp(const double (&q)[4], double h, dou
     s = s + q[2] * p3;
     s = s + q[3] * p4;
     return h * s + y_old;
+}
+
+// Row i of the dense-output coefficients Q = K^T P (rk.py:178-180).
+template <int NC>
+__device__ __forceinline__ void dense_q(const double (&K)[7][NC], int i, double (&q)[4])
+{
+#pragma unroll
+    for (int m = 0; m < 4; ++m) {
+        double acc = K[0][i] * c_P[0][m];
+#pragma unroll
+        for (int j = 2; j < 7; ++j) acc = fma(K[j][i], c_P[j][m], acc);
+        q[m] = acc;
+    }
 }
 
 // scipy/optimize/Zeros/brentq.c on event(t) = r(t) - r_stop, xtol = rtol = 4 EPS, 100 iterations.
@@ -243,313 +260,227 @@ __device__ __forceinline__ void write_point(const Rk45Args &a, long long idx, in
     row[5] = p_t; row[6] = y[4]; row[7] = y[5]; row[8] = p_phi;
 }
 
-template <>
-__device__ __forceinline__ void rk_f<0>(const Rk45Args &a, double r_floor, double p_t, double p_phi,
-                                        const double (&y)[RK_NC], ThetaCache &tc, double (&d)[RK_NC])
+// ---------------------------------------------------------------------------------------------
+// The pieces of scipy's RK45 that every component system runs.  Scalars (rtol, atol, max_step, ...)
+// come by value from the kernel's locals: re-reading them from Rk45Args changes the generated code.
+// ---------------------------------------------------------------------------------------------
+
+// Schwarzschild.initial_conditions, metrics.py:794-809: the six moving components and p_phi (p_t = -1).
+// false where the reference returns None (`p_r_sq < 0`; a NaN would hang solve_ivp).
+__device__ __forceinline__ bool rk_initial_conditions(const Rk45Args &a, long long ray, double (&y)[RK_NC],
+                                                      double &p_phi)
 {
-    rk_rhs(a.R_S, r_floor, p_t, p_phi, y, tc, d);
+    const double alpha = __ldg(a.alphas + ray);
+    const double b = a.r_obs * lp_sin_cr(alpha) / a.sqrt_f0;
+    const double L = b;
+    const double p_r_sq = (1.0 / a.f0 - (L * L) / (a.r_obs * a.r_obs)) / a.f0;
+    if (!(p_r_sq >= 0.0)) return false;
+    y[0] = 0.0; y[1] = a.r_obs; y[2] = LP_PI_D / 2; y[3] = 0.0;
+    y[4] = -__dsqrt_rn(p_r_sq); y[5] = 0.0;
+    p_phi = L;
+    return true;
 }
-template <>
-__device__ __forceinline__ void rk_f<1>(const Rk45Args &a, double r_floor, double p_t, double p_phi,
-                                        const double (&y)[RK_NC], ThetaCache &tc, double (&d)[RK_NC])
+
+// f = rhs(y) (rk.py:95) and select_initial_step (common.py:68-134, direction = +1) on the six-component state.
+template <int METRIC>
+__device__ __forceinline__ double rk_select_initial_step(const Rk45Args &a, double r_floor, double p_t, double p_phi,
+                                                         const double (&y)[RK_NC], ThetaCache &tc, double (&f)[RK_NC],
+                                                         double interval, double rtol, double atol, double max_step)
 {
-    rk_rhs_kerr(a.kerr_M, a.kerr_a, r_floor, p_t, p_phi, y, tc, d);
+    rk_f<METRIC>(a, r_floor, p_t, p_phi, y, tc, f);
+    double sc[RK_NC], d0s = 0.0, d1s = 0.0;
+#pragma unroll
+    for (int i = 0; i < RK_NC; ++i) {
+        sc[i] = atol + fabs(y[i]) * rtol;
+        const double v0 = y[i] / sc[i], v1 = f[i] / sc[i];
+        d0s = fma(v0, v0, d0s); d1s = fma(v1, v1, d1s);
+    }
+    {   // the two constant components contribute to d0 only
+        const double v4 = p_t / (atol + fabs(p_t) * rtol), v7 = p_phi / (atol + fabs(p_phi) * rtol);
+        d0s = fma(v4, v4, d0s); d0s = fma(v7, v7, d0s);
+    }
+    const double d0 = rms8(d0s), d1 = rms8(d1s);
+    double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
+    h0 = fmin(h0, interval);
+    double y1[RK_NC], f1[RK_NC], d2s = 0.0;
+#pragma unroll
+    for (int i = 0; i < RK_NC; ++i) y1[i] = y[i] + h0 * f[i];
+    rk_f<METRIC>(a, r_floor, p_t, p_phi, y1, tc, f1);
+#pragma unroll
+    for (int i = 0; i < RK_NC; ++i) { const double v2 = (f1[i] - f[i]) / sc[i]; d2s = fma(v2, v2, d2s); }
+    const double d2 = rms8(d2s) / h0;
+    double h1;
+    if (d1 <= 1e-15 && d2 <= 1e-15) h1 = fmax(1e-6, h0 * 1e-3);
+    else h1 = pow(0.01 / fmax(d1, d2), 0.2);
+    return fmin(fmin(100 * h0, h1), fmin(interval, max_step));
 }
 
-template <int MINB, int METRIC, bool DENSE = false>
-__global__ void __launch_bounds__(RK_BLOCK, MINB)
-lp_rk45_kernel(const Rk45Args a)
+// The stages of one step attempt (rk_step, rk.py:14-73): K[0] = f on entry; K[1..6] and y_new on exit.
+template <int NC, class Rhs>
+__device__ __forceinline__ void rk_stages(double h, const double (&y)[NC], double (&K)[7][NC], double (&y_new)[NC],
+                                          Rhs rhs)
 {
-    const unsigned full = 0xffffffffu;
-    const int lane = threadIdx.x & 31;
-    const long long warp_id = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
-    const double r_floor = a.r_floor, rtol = a.rtol, atol = a.atol;
-    const double t_bound = a.lambda_max, max_step = a.max_step;
-    const double INF = __longlong_as_double(0x7ff0000000000000LL);
-
-    // per-lane ray state
-    bool active = false, fresh = true, rejected = false;
-    long long idx = -1;
-    double t = 0.0, h_abs = 0.0, p_t = -1.0, p_phi = 0.0, g0 = 0.0, g1 = 0.0, r_out = 0.0;
-    double y[RK_NC], f[RK_NC];
 #pragma unroll
-    for (int i = 0; i < RK_NC; ++i) { y[i] = 0.0; f[i] = 0.0; }
-    int npts = 0, attempts = 0;
-    ThetaCache tc;
-    tc.th = __longlong_as_double(0x7ff8000000000000LL); tc.s = 1.0; tc.c = 0.0;
-
-    // warp queue: virtual position v -> ray ((v / 32) * n_warps + warp_id) * 32 + v % 32
-    long long cursor = 0;
-    bool queue_empty = (warp_id * 32 >= a.n);
-
-    while (true) {
-        // ---------------- lane refill (ballot + rank) ----------------
-        const unsigned idle = __ballot_sync(full, !active);
-        if (idle && !queue_empty && (__popc(idle) >= a.refill_min || idle == full)) {
-            const int rank = __popc(idle & ((1u << lane) - 1u));
-            const long long v = cursor + rank;               // meaningful on idle lanes only
-            const long long ray = ((v >> 5) * n_warps + warp_id) * 32 + (v & 31);
-            cursor += __popc(idle);
-            // ray(v) is increasing in v: the queue is exhausted once the next position is past the batch
-            if (((cursor >> 5) * n_warps + warp_id) * 32 + (cursor & 31) >= a.n) queue_empty = true;
-            if (!active && ray < a.n) {
-                idx = ray;
-                bool valid = true;
-                if (a.state0) {                          // integrate_geodesic(metric, state0, ...)
-                    const double *s0 = a.state0 + ray * 8;
-                    y[0] = __ldg(s0 + 0); y[1] = __ldg(s0 + 1); y[2] = __ldg(s0 + 2); y[3] = __ldg(s0 + 3);
-                    p_t = __ldg(s0 + 4); y[4] = __ldg(s0 + 5); y[5] = __ldg(s0 + 6); p_phi = __ldg(s0 + 7);
-                } else {
-                    // ---- Schwarzschild.initial_conditions, metrics.py:794-809 ----
-                    const double alpha = __ldg(a.alphas + ray);
-                    const double b = a.r_obs * lp_sin_cr(alpha) / a.sqrt_f0;
-                    const double L = b;
-                    const double p_r_sq = (1.0 / a.f0 - (L * L) / (a.r_obs * a.r_obs)) / a.f0;
-                    valid = (p_r_sq >= 0.0);             // `p_r_sq < 0 -> None`; NaN would hang solve_ivp
-                    y[0] = 0.0; y[1] = a.r_obs; y[2] = LP_PI_D / 2; y[3] = 0.0;
-                    y[4] = -__dsqrt_rn(p_r_sq); y[5] = 0.0;
-                    p_t = -1.0; p_phi = L;
-                }
-                if (!valid) {                            // (None, 'invalid'), geodesic_tracer.py:79-81
-                    const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-                    for (int k = 0; k < 8; ++k) a.out_state[idx * 8 + k] = qnan;
-                    a.out_lambda[idx] = qnan;
-                    a.out_outcome[idx] = 0;
-                    if (a.out_nsteps) { a.out_nsteps[2 * idx] = 0; a.out_nsteps[2 * idx + 1] = 0; }
-                    if (a.out_status) a.out_status[idx] = -2;
-                    if (a.n_points) a.n_points[idx] = 0;
-                } else {
-                    t = 0.0;
-                    r_out = a.r_out > 0.0 ? a.r_out : y[1] * 2.0;
-                    rk_f<METRIC>(a, r_floor, p_t, p_phi, y, tc, f);               // rk.py:95
-                    // ---- select_initial_step, common.py:68-134 (direction = +1) ----
-                    const double interval = fabs(t_bound - t);
-                    double sc[RK_NC], d0s = 0.0, d1s = 0.0;
+    for (int s = 1; s < 6; ++s) {
+        double ys[NC];
 #pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) {
-                        sc[i] = atol + fabs(y[i]) * rtol;
-                        const double v0 = y[i] / sc[i], v1 = f[i] / sc[i];
-                        d0s = fma(v0, v0, d0s); d1s = fma(v1, v1, d1s);
-                    }
-                    {   // the two constant components contribute to d0 only
-                        const double v4 = p_t / (atol + fabs(p_t) * rtol), v7 = p_phi / (atol + fabs(p_phi) * rtol);
-                        d0s = fma(v4, v4, d0s); d0s = fma(v7, v7, d0s);
-                    }
-                    const double d0 = rms8(d0s), d1 = rms8(d1s);
-                    double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
-                    h0 = fmin(h0, interval);
-                    double y1[RK_NC], f1[RK_NC], d2s = 0.0;
+        for (int i = 0; i < NC; ++i) {
+            double dy = K[0][i] * c_A[s][0];
 #pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) y1[i] = y[i] + h0 * f[i];
-                    rk_f<METRIC>(a, r_floor, p_t, p_phi, y1, tc, f1);
-#pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) { const double v2 = (f1[i] - f[i]) / sc[i]; d2s = fma(v2, v2, d2s); }
-                    const double d2 = rms8(d2s) / h0;
-                    double h1;
-                    if (d1 <= 1e-15 && d2 <= 1e-15) h1 = fmax(1e-6, h0 * 1e-3);
-                    else h1 = pow(0.01 / fmax(d1, d2), 0.2);
-                    h_abs = fmin(fmin(100 * h0, h1), fmin(interval, max_step));
-                    g0 = y[1] - a.r_in; g1 = y[1] - r_out;                        // ivp.py:650
-                    npts = 1; attempts = 0; fresh = true; rejected = false;
-                    write_point(a, idx, 0, t, y, p_t, p_phi);
-                    active = (interval != 0.0);
-                    if (!active) {     // zero-length interval: solve_ivp returns the initial point, status 0
-                        a.out_state[idx * 8 + 0] = y[0]; a.out_state[idx * 8 + 1] = y[1];
-                        a.out_state[idx * 8 + 2] = y[2]; a.out_state[idx * 8 + 3] = y[3];
-                        a.out_state[idx * 8 + 4] = p_t; a.out_state[idx * 8 + 5] = y[4];
-                        a.out_state[idx * 8 + 6] = y[5]; a.out_state[idx * 8 + 7] = p_phi;
-                        a.out_lambda[idx] = t;
-                        a.out_outcome[idx] = (y[1] <= a.r_in * 1.1) ? -1 : 1;
-                        if (a.out_nsteps) { a.out_nsteps[2 * idx] = 1; a.out_nsteps[2 * idx + 1] = 2; }
-                        if (a.out_status) a.out_status[idx] = 0;
-                        if (a.n_points) a.n_points[idx] = 1;
-                    }
-                }
-            }
+            for (int j = 1; j < s; ++j) dy = fma(K[j][i], c_A[s][j], dy);
+            ys[i] = fma(dy, h, y[i]);
         }
-        if (!__any_sync(full, active)) {
-            if (queue_empty) break;
-            continue;
-        }
-        if (!active) continue;
+        rhs(ys, K[s]);
+    }
+#pragma unroll
+    for (int i = 0; i < NC; ++i) {
+        double acc = K[0][i] * c_B[0];
+        acc = fma(K[2][i], c_B[2], acc);
+        acc = fma(K[3][i], c_B[3], acc);
+        acc = fma(K[4][i], c_B[4], acc);
+        acc = fma(K[5][i], c_B[5], acc);
+        y_new[i] = fma(h, acc, y[i]);
+    }
+    rhs(y_new, K[6]);
+}
 
-        // ---------------- one step attempt (RungeKutta._step_impl, rk.py:111-176) ----------------
-        const double min_step = 10 * fabs((__longlong_as_double(__double_as_longlong(t) + 1LL)) - t);
-        double ha = h_abs;
-        if (fresh) {
-            if (ha > max_step) ha = max_step; else if (ha < min_step) ha = min_step;
-            fresh = false; rejected = false;
-        }
-        int status = 2;                 // 2 = still running
-        double t_fin = t;
-        double yf[RK_NC];
+// Sum of the squared scaled errors, 8 error_norm^2 (rk.py:105-109, :148-149).  The NC quotients use the
+// branch-free division halves (bit-identical to `/` for finite operands, scale >= atol > 0) so their
+// dependent chains interleave; anything non-finite takes the literal IEEE form.
+template <int NC>
+__device__ __forceinline__ double rk_error_sq(const double (&K)[7][NC], const double (&y)[NC], const double (&y_new)[NC],
+                                              double h, double rtol, double atol)
+{
+    double esum = 0.0, en[NC], es[NC];
 #pragma unroll
-        for (int i = 0; i < RK_NC; ++i) yf[i] = y[i];
-
-        if (ha < min_step) {
-            status = -1;                // TOO_SMALL_STEP -> solve_ivp status -1, last accepted point stays
-        } else {
-            double t_new = t + ha;
-            if (t_new - t_bound > 0) t_new = t_bound;
-            const double h = t_new - t;
-            ha = fabs(h);
-            attempts++;
-            // ---- rk_step, rk.py:14-73 ----
-            double K[7][RK_NC];
+    for (int i = 0; i < NC; ++i) {
+        es[i] = atol + max_sel(fabs(y[i]), fabs(y_new[i])) * rtol;
+        double acc = K[0][i] * c_E[0];
+        acc = fma(K[2][i], c_E[2], acc);
+        acc = fma(K[3][i], c_E[3], acc);
+        acc = fma(K[4][i], c_E[4], acc);
+        acc = fma(K[5][i], c_E[5], acc);
+        acc = fma(K[6][i], c_E[6], acc);
+        en[i] = acc * h;
+    }
 #pragma unroll
-            for (int i = 0; i < RK_NC; ++i) K[0][i] = f[i];
+    for (int i = 0; i < NC; ++i) {
+        const double e = en[i] * fast_rcp(es[i]);        // es >= atol > 0; only the controller sees it
+        esum = fma(e, e, esum);
+    }
+    if (!isfinite(esum)) {
+        esum = 0.0;
 #pragma unroll
-            for (int s = 1; s < 6; ++s) {
-                double ys[RK_NC];
-#pragma unroll
-                for (int i = 0; i < RK_NC; ++i) {
-                    double dy = K[0][i] * c_A[s][0];
-#pragma unroll
-                    for (int j = 1; j < s; ++j) dy = fma(K[j][i], c_A[s][j], dy);
-                    ys[i] = fma(dy, h, y[i]);
-                }
-                rk_f<METRIC>(a, r_floor, p_t, p_phi, ys, tc, K[s]);
-            }
-            double y_new[RK_NC];
-#pragma unroll
-            for (int i = 0; i < RK_NC; ++i) {
-                double acc = K[0][i] * c_B[0];
-                acc = fma(K[2][i], c_B[2], acc);
-                acc = fma(K[3][i], c_B[3], acc);
-                acc = fma(K[4][i], c_B[4], acc);
-                acc = fma(K[5][i], c_B[5], acc);
-                y_new[i] = fma(h, acc, y[i]);
-            }
-            rk_f<METRIC>(a, r_floor, p_t, p_phi, y_new, tc, K[6]);
-            // ---- error norm, rk.py:105-109, :148-149 ----
-            // the six quotients use the branch-free division halves (bit-identical to `/` for
-            // finite operands, scale >= atol > 0) so their dependent chains interleave; anything
-            // non-finite takes the literal IEEE form
-            double esum = 0.0, en[RK_NC], es[RK_NC];
-#pragma unroll
-            for (int i = 0; i < RK_NC; ++i) {
-                es[i] = atol + max_sel(fabs(y[i]), fabs(y_new[i])) * rtol;
-                double acc = K[0][i] * c_E[0];
-                acc = fma(K[2][i], c_E[2], acc);
-                acc = fma(K[3][i], c_E[3], acc);
-                acc = fma(K[4][i], c_E[4], acc);
-                acc = fma(K[5][i], c_E[5], acc);
-                acc = fma(K[6][i], c_E[6], acc);
-                en[i] = acc * h;
-            }
-#pragma unroll
-            for (int i = 0; i < RK_NC; ++i) {
-                const double e = en[i] * fast_rcp(es[i]);        // es >= atol > 0; only the controller sees it
-                esum = fma(e, e, esum);
-            }
-            if (!isfinite(esum)) {
-                esum = 0.0;
-#pragma unroll
-                for (int i = 0; i < RK_NC; ++i) {
-                    const double e = en[i] / es[i];
-                    esum = fma(e, e, esum);
-                }
-            }
-            // one power for the accept and the reject controller (rk.py:155-170): divergent branches
-            // would each run their own copy for the whole warp
-            // (fast_pow: the controller on the SQUARED norm, 0.9 err^-0.2 = 0.9 (esum / 8)^-0.1 by
-            // inv_tenth_root — a few ulp, the level at which scipy's own BLAS stage sums already differ
-            // from any restatement; error_norm is then only compared with 0 and 1, which the square
-            // preserves; tests hold the accept/reject sequences identical)
-            double error_norm, pow_term;
-            if (a.fast_pow) { error_norm = esum * 0.125; pow_term = 0.9 * inv_tenth_root(error_norm); }
-            else { error_norm = rms8(esum); pow_term = 0.9 * pow(error_norm, -0.2); }
-            if (error_norm < 1) {
-                double factor = (error_norm == 0) ? 10.0 : min_sel(pow_term, 10.0);
-                if (rejected) factor = min_sel(factor, 1.0);
-                ha *= factor;
-                // ---- accepted: events on the new point (ivp.py:676-699) ----
-                const double gn0 = y_new[1] - a.r_in, gn1 = y_new[1] - r_out;
-                const bool act0 = (g0 >= 0) && (gn0 <= 0);       // direction -1
-                const bool act1 = (g1 <= 0) && (gn1 >= 0);       // direction +1
-                t_fin = t_new;
-#pragma unroll
-                for (int i = 0; i < RK_NC; ++i) yf[i] = y_new[i];
-                if (t_new - t_bound >= 0) status = 0;            // OdeSolver.step: finished
-                if (act0 || act1) {
-                    // dense output Q = K^T P (rk.py:178-180): r first (root), then every component
-                    double q[4];
-#pragma unroll
-                    for (int m = 0; m < 4; ++m) {
-                        double acc = K[0][1] * c_P[0][m];
-#pragma unroll
-                        for (int j = 2; j < 7; ++j) acc = fma(K[j][1], c_P[j][m], acc);
-                        q[m] = acc;
-                    }
-                    double root = 0.0;
-                    if (act0) root = rk_brentq(q, h, y[1], t, a.r_in, t, t_new);
-                    if (act1) {
-                        const double r1 = rk_brentq(q, h, y[1], t, r_out, t, t_new);
-                        root = (act0 && root <= r1) ? root : r1;
-                    }
-                    status = 1;
-                    t_fin = root;
-                    const double x = (root - t) / h;
-#pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) {
-                        double qi[4];
-#pragma unroll
-                        for (int m = 0; m < 4; ++m) {
-                            double acc = K[0][i] * c_P[0][m];
-#pragma unroll
-                            for (int j = 2; j < 7; ++j) acc = fma(K[j][i], c_P[j][m], acc);
-                            qi[m] = acc;
-                        }
-                        yf[i] = dense_comp(qi, h, y[i], x);
-                    }
-                }
-                g0 = gn0; g1 = gn1;
-                if (DENSE && a.dense && npts < a.max_points) {
-                    // the step's interpolant for OdeResult.sol: h and Q = K^T P (rk.py:178-180)
-                    double *row = a.dense + ((size_t)idx * a.max_points + npts) * 25;
-                    row[0] = h;
-#pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) {
-#pragma unroll
-                        for (int m = 0; m < 4; ++m) {
-                            double acc = K[0][i] * c_P[0][m];
-#pragma unroll
-                            for (int j = 2; j < 7; ++j) acc = fma(K[j][i], c_P[j][m], acc);
-                            row[1 + 4 * i + m] = acc;
-                        }
-                    }
-                }
-                write_point(a, idx, npts, t_fin, yf, p_t, p_phi);
-                npts++;
-                t = t_new;
-#pragma unroll
-                for (int i = 0; i < RK_NC; ++i) { y[i] = y_new[i]; f[i] = K[6][i]; }
-                fresh = true;
-            } else {
-                ha *= max_sel(pow_term, 0.2);
-                rejected = true;
-            }
-        }
-        h_abs = ha;
-
-        if (status != 2) {
-            // ---- ray finished: outcome (geodesic_tracer.py:69-70) and outputs ----
-            double *o = a.out_state + idx * 8;
-            o[0] = yf[0]; o[1] = yf[1]; o[2] = yf[2]; o[3] = yf[3];
-            o[4] = p_t; o[5] = yf[4]; o[6] = yf[5]; o[7] = p_phi;
-            a.out_lambda[idx] = t_fin;
-            a.out_outcome[idx] = (yf[1] <= a.r_in * 1.1) ? -1 : 1;
-            if (a.out_nsteps) { a.out_nsteps[2 * idx] = npts; a.out_nsteps[2 * idx + 1] = 2 + 6 * attempts; }
-            if (a.out_status) a.out_status[idx] = (int8_t)status;
-            if (a.n_points) a.n_points[idx] = npts;
-            active = false;
+        for (int i = 0; i < NC; ++i) {
+            const double e = en[i] / es[i];
+            esum = fma(e, e, esum);
         }
     }
+    return esum;
+}
+
+// Terminal events on an accepted step (ivp.py:676-699): r falls to r_in (act0) or rises to r_out (act1).  The
+// earlier root of the two by brentq on r's dense output, every component interpolated there into yf.
+template <int NC>
+__device__ __forceinline__ double rk_event_root(const double (&K)[7][NC], const double (&y)[NC], double t, double h,
+                                                double t_new, double r_in, double r_out, bool act0, bool act1,
+                                                double (&yf)[NC])
+{
+    double q[4];
+    dense_q(K, 1, q);
+    double root = 0.0;
+    if (act0) root = rk_brentq(q, h, y[1], t, r_in, t, t_new);
+    if (act1) {
+        const double r1 = rk_brentq(q, h, y[1], t, r_out, t, t_new);
+        root = (act0 && root <= r1) ? root : r1;
+    }
+    const double x = (root - t) / h;
+#pragma unroll
+    for (int i = 0; i < NC; ++i) {
+        double qi[4];
+        dense_q(K, i, qi);
+        yf[i] = dense_comp(qi, h, y[i], x);
+    }
+    return root;
+}
+
+// (None, 'invalid'), geodesic_tracer.py:79-81
+template <bool PATHS>
+__device__ __forceinline__ void rk_write_invalid(const Rk45Args &a, long long idx)
+{
+    const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+    for (int k = 0; k < 8; ++k) a.out_state[idx * 8 + k] = qnan;
+    a.out_lambda[idx] = qnan;
+    a.out_outcome[idx] = 0;
+    if (a.out_nsteps) { a.out_nsteps[2 * idx] = 0; a.out_nsteps[2 * idx + 1] = 0; }
+    if (a.out_status) a.out_status[idx] = -2;
+    if (PATHS && a.n_points) a.n_points[idx] = 0;
+}
+
+// A finished ray: outcome (geodesic_tracer.py:69-70) and outputs.  y[1] is r in every system.
+template <class Sys>
+__device__ __forceinline__ void rk_write_result(const Rk45Args &a, const Sys &sys, long long idx,
+                                                const double (&y)[Sys::NC], double t, int npts, int nfev, int status)
+{
+    sys.pack(y, a.out_state + idx * 8);
+    a.out_lambda[idx] = t;
+    a.out_outcome[idx] = (y[1] <= a.r_in * 1.1) ? -1 : 1;
+    if (a.out_nsteps) { a.out_nsteps[2 * idx] = npts; a.out_nsteps[2 * idx + 1] = nfev; }
+    if (a.out_status) a.out_status[idx] = (int8_t)status;
+    if (Sys::PATHS && a.n_points) a.n_points[idx] = npts;
 }
 
 // ---------------------------------------------------------------------------------------------
-// Equatorial specialisation of the batch path (the `alphas` entry: every ray starts from
+// Component systems.  A system carries NC moving components in registers and supplies
+//   start():  the initial conditions of a ray, then rk_select_initial_step; false for an invalid ray;
+//   stages(): K[1..6] and y_new of one step attempt;
+//   pack():   the 8-slot output state;
+// and the compile-time flags PATHS (trajectory points, n_points) and DENSE (per-step interpolant rows).
+// ---------------------------------------------------------------------------------------------
+
+// The six moving components (t, r, theta, phi, p_r, p_theta) from alphas or state0, Schwarzschild or Kerr.
+template <int METRIC, bool DENSE_ROWS>
+struct RkSixSystem {
+    static constexpr int NC = RK_NC;
+    static constexpr bool PATHS = true, DENSE = DENSE_ROWS;
+    double p_t, p_phi;
+    ThetaCache tc;                                        // kept across the rays of the lane
+
+    __device__ __forceinline__ RkSixSystem() : p_t(-1.0), p_phi(0.0)
+    {
+        tc.th = __longlong_as_double(0x7ff8000000000000LL); tc.s = 1.0; tc.c = 0.0;
+    }
+    __device__ __forceinline__ bool start(const Rk45Args &a, long long ray, double r_floor, double interval,
+                                          double rtol, double atol, double max_step,
+                                          double (&y)[NC], double (&f)[NC], double &h_abs)
+    {
+        if (a.state0) {                                   // integrate_geodesic(metric, state0, ...)
+            const double *s0 = a.state0 + ray * 8;
+            y[0] = __ldg(s0 + 0); y[1] = __ldg(s0 + 1); y[2] = __ldg(s0 + 2); y[3] = __ldg(s0 + 3);
+            p_t = __ldg(s0 + 4); y[4] = __ldg(s0 + 5); y[5] = __ldg(s0 + 6); p_phi = __ldg(s0 + 7);
+        } else {
+            p_t = -1.0;
+            if (!rk_initial_conditions(a, ray, y, p_phi)) return false;
+        }
+        h_abs = rk_select_initial_step<METRIC>(a, r_floor, p_t, p_phi, y, tc, f, interval, rtol, atol, max_step);
+        return true;
+    }
+    __device__ __forceinline__ void stages(const Rk45Args &a, double r_floor, double h, const double (&y)[NC],
+                                           double (&K)[7][NC], double (&y_new)[NC])
+    {
+        rk_stages(h, y, K, y_new, [&](const double (&ys)[NC], double (&d)[NC]) {
+            rk_f<METRIC>(a, r_floor, p_t, p_phi, ys, tc, d);
+        });
+    }
+    __device__ __forceinline__ void pack(const double (&y)[NC], double *o) const
+    {
+        o[0] = y[0]; o[1] = y[1]; o[2] = y[2]; o[3] = y[3];
+        o[4] = p_t; o[5] = y[4]; o[6] = y[5]; o[7] = p_phi;
+    }
+};
+
+// ---------------------------------------------------------------------------------------------
+// Equatorial system of the batch path (the `alphas` entry: every ray starts from
 // Schwarzschild.initial_conditions, metrics.py:794-809, i.e. theta = pi/2 and p_theta = 0 EXACTLY).
 //
 // In the reference's own integration those two components only carry rounding noise: d theta/d lambda
@@ -558,11 +489,11 @@ lp_rk45_kernel(const Rk45Args a)
 // sin^2(theta) rounds to exactly 1.0 and p_theta^2 + p_phi^2 to p_phi^2, so the right-hand side of the
 // other four components (t, r, phi, p_r) is BIT-IDENTICAL with or without them; their terms of the
 // error norm are ~1e-24 against a sum that is >= 1e-10 whenever the step-size factor is not clamped.
-// This kernel therefore integrates the four live components only (28 stage values instead of 42 in
+// This system therefore integrates the four live components only (28 stage values instead of 42 in
 // registers, ~2/3 of the FP64 work per step attempt) and reports theta = pi/2, p_theta = 0 — within
 // 3e-16 absolute of what the reference's noise integrates to.  The first-step selection is the full
 // six-component arithmetic (it sees theta / scale = 1e8).  tests/test_gpu_rk45.py holds it to the
-// six-component kernel: same accept/reject sequences, (t, r, phi, p_r) within 1e-12.
+// six-component system: same accept/reject sequences, (t, r, phi, p_r) within 1e-12.
 // ---------------------------------------------------------------------------------------------
 #define RK_EQ 4
 
@@ -595,139 +526,93 @@ __device__ __forceinline__ void rk_rhs_eq(double R_S, double r_floor, double p_t
     d[3] = fma(-a, fma(ptf, ptf, p_r * p_r), pp2 * ir3);
 }
 
-// The six stages of one step attempt (rk.py:111-176 / rk_step): K[0] = f on entry; K[1..6] and y_new on exit.
-template <bool SPEC>
-__device__ __forceinline__ void rk_eq_stages(double R_S, double r_floor, double p_t, double p_phi, double pp2, double h,
-                                             const double (&y)[RK_EQ], double (&K)[7][RK_EQ], double (&y_new)[RK_EQ],
-                                             int &r_hi_min)
-{
-#pragma unroll
-    for (int s = 1; s < 6; ++s) {
-        double ys[RK_EQ];
-#pragma unroll
-        for (int i = 0; i < RK_EQ; ++i) {
-            double dy = K[0][i] * c_A[s][0];
-#pragma unroll
-            for (int j = 1; j < s; ++j) dy = fma(K[j][i], c_A[s][j], dy);
-            ys[i] = fma(dy, h, y[i]);
-        }
-        rk_rhs_eq<SPEC>(R_S, r_floor, p_t, p_phi, pp2, ys, K[s], r_hi_min);
-    }
-#pragma unroll
-    for (int i = 0; i < RK_EQ; ++i) {
-        double acc = K[0][i] * c_B[0];
-        acc = fma(K[2][i], c_B[2], acc);
-        acc = fma(K[3][i], c_B[3], acc);
-        acc = fma(K[4][i], c_B[4], acc);
-        acc = fma(K[5][i], c_B[5], acc);
-        y_new[i] = fma(h, acc, y[i]);
-    }
-    rk_rhs_eq<SPEC>(R_S, r_floor, p_t, p_phi, pp2, y_new, K[6], r_hi_min);
-}
+struct RkEquatorialSystem {
+    static constexpr int NC = RK_EQ;                      // (t, r, phi, p_r)
+    static constexpr bool PATHS = false, DENSE = false;
+    double p_t, p_phi, pp2;
 
-template <int MINB>
-__global__ void __launch_bounds__(RK_BLOCK, MINB)
-lp_rk45_eq_kernel(const Rk45Args a)
+    __device__ __forceinline__ RkEquatorialSystem() : p_t(-1.0), p_phi(0.0), pp2(0.0) {}
+    __device__ __forceinline__ bool start(const Rk45Args &a, long long ray, double r_floor, double interval,
+                                          double rtol, double atol, double max_step,
+                                          double (&y)[NC], double (&f)[NC], double &h_abs)
+    {
+        double y6[RK_NC], f6[RK_NC];                      // the six-component state of the reference
+        if (!rk_initial_conditions(a, ray, y6, p_phi)) return false;
+        pp2 = p_phi * p_phi;
+        ThetaCache tc;
+        tc.th = __longlong_as_double(0x7ff8000000000000LL); tc.s = 1.0; tc.c = 0.0;
+        h_abs = rk_select_initial_step<0>(a, r_floor, p_t, p_phi, y6, tc, f6, interval, rtol, atol, max_step);
+        y[0] = y6[0]; y[1] = y6[1]; y[2] = y6[3]; y[3] = y6[4];
+        f[0] = f6[0]; f[1] = f6[1]; f[2] = f6[3]; f[3] = f6[4];
+        return true;
+    }
+    __device__ __forceinline__ void stages(const Rk45Args &a, double r_floor, double h, const double (&y)[NC],
+                                           double (&K)[7][NC], double (&y_new)[NC])
+    {
+        int r_hi_min = 0x7fffffff;
+        rk_stages(h, y, K, y_new, [&](const double (&ys)[NC], double (&d)[NC]) {
+            rk_rhs_eq<true>(a.R_S, r_floor, p_t, p_phi, pp2, ys, d, r_hi_min);
+        });
+        // a stage at or (by less than one high word) above the floor: the tested form decides — cold
+        if (r_hi_min <= __double2hiint(r_floor))
+            rk_stages(h, y, K, y_new, [&](const double (&ys)[NC], double (&d)[NC]) {
+                rk_rhs_eq<false>(a.R_S, r_floor, p_t, p_phi, pp2, ys, d, r_hi_min);
+            });
+    }
+    __device__ __forceinline__ void pack(const double (&y)[NC], double *o) const
+    {
+        o[0] = y[0]; o[1] = y[1]; o[2] = LP_PI_D / 2; o[3] = y[2];
+        o[4] = p_t; o[5] = y[3]; o[6] = 0.0; o[7] = p_phi;
+    }
+};
+
+// ---------------------------------------------------------------------------------------------
+// The step body: warp-queue refill, one step attempt per trip, accept / reject, finish.
+// ---------------------------------------------------------------------------------------------
+template <class Sys>
+__device__ __forceinline__ void rk45_solve(const Rk45Args &a)
 {
+    constexpr int NC = Sys::NC;
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
-    const long long warp_id = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
     const double r_floor = a.r_floor, rtol = a.rtol, atol = a.atol;
     const double t_bound = a.lambda_max, max_step = a.max_step;
-    const double p_t = -1.0;
 
+    // per-lane ray state
+    Sys sys;
     bool active = false, fresh = true, rejected = false;
     long long idx = -1;
-    double t = 0.0, h_abs = 0.0, p_phi = 0.0, pp2 = 0.0, g0 = 0.0, g1 = 0.0, r_out = 0.0;
-    double y[RK_EQ], f[RK_EQ];                           // (t, r, phi, p_r)
+    double t = 0.0, h_abs = 0.0, g0 = 0.0, g1 = 0.0, r_out = 0.0;
+    double y[NC], f[NC];
 #pragma unroll
-    for (int i = 0; i < RK_EQ; ++i) { y[i] = 0.0; f[i] = 0.0; }
+    for (int i = 0; i < NC; ++i) { y[i] = 0.0; f[i] = 0.0; }
     int npts = 0, attempts = 0;
-
-    long long cursor = 0;
-    bool queue_empty = (warp_id * 32 >= a.n);
+    LpWarpQueue queue(a.n);
 
     while (true) {
-        // ---------------- lane refill (ballot + rank), as lp_rk45_kernel ----------------
+        // ---------------- lane refill (ballot + rank) ----------------
         const unsigned idle = __ballot_sync(full, !active);
-        if (idle && !queue_empty && (__popc(idle) >= a.refill_min || idle == full)) {
-            const int rank = __popc(idle & ((1u << lane) - 1u));
-            const long long v = cursor + rank;
-            const long long ray = ((v >> 5) * n_warps + warp_id) * 32 + (v & 31);
-            cursor += __popc(idle);
-            if (((cursor >> 5) * n_warps + warp_id) * 32 + (cursor & 31) >= a.n) queue_empty = true;
+        if (idle && !queue.empty && (__popc(idle) >= a.refill_min || idle == full)) {
+            const long long ray = queue.take(idle, lane);
             if (!active && ray < a.n) {
                 idx = ray;
-                // ---- Schwarzschild.initial_conditions, metrics.py:794-809 ----
-                const double alpha = __ldg(a.alphas + ray);
-                const double b = a.r_obs * lp_sin_cr(alpha) / a.sqrt_f0;
-                const double L = b;
-                const double p_r_sq = (1.0 / a.f0 - (L * L) / (a.r_obs * a.r_obs)) / a.f0;
-                const bool valid = (p_r_sq >= 0.0);
-                if (!valid) {                            // (None, 'invalid'), geodesic_tracer.py:79-81
-                    const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-                    for (int k = 0; k < 8; ++k) a.out_state[idx * 8 + k] = qnan;
-                    a.out_lambda[idx] = qnan;
-                    a.out_outcome[idx] = 0;
-                    if (a.out_nsteps) { a.out_nsteps[2 * idx] = 0; a.out_nsteps[2 * idx + 1] = 0; }
-                    if (a.out_status) a.out_status[idx] = -2;
+                const double interval = fabs(t_bound - 0.0);              // t starts at 0
+                if (!sys.start(a, ray, r_floor, interval, rtol, atol, max_step, y, f, h_abs)) {
+                    rk_write_invalid<Sys::PATHS>(a, idx);
                 } else {
-                    // the six-component state of the reference for the first-step selection
-                    double y6[RK_NC], f6[RK_NC];
-                    y6[0] = 0.0; y6[1] = a.r_obs; y6[2] = LP_PI_D / 2; y6[3] = 0.0;
-                    y6[4] = -__dsqrt_rn(p_r_sq); y6[5] = 0.0;
-                    p_phi = L; pp2 = p_phi * p_phi;
-                    ThetaCache tc;
-                    tc.th = __longlong_as_double(0x7ff8000000000000LL); tc.s = 1.0; tc.c = 0.0;
                     t = 0.0;
-                    r_out = a.r_out > 0.0 ? a.r_out : y6[1] * 2.0;
-                    rk_rhs(a.R_S, r_floor, p_t, p_phi, y6, tc, f6);                  // rk.py:95
-                    // ---- select_initial_step, common.py:68-134 (direction = +1) ----
-                    const double interval = fabs(t_bound - t);
-                    double sc[RK_NC], d0s = 0.0, d1s = 0.0;
-#pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) {
-                        sc[i] = atol + fabs(y6[i]) * rtol;
-                        const double v0 = y6[i] / sc[i], v1 = f6[i] / sc[i];
-                        d0s = fma(v0, v0, d0s); d1s = fma(v1, v1, d1s);
-                    }
-                    {
-                        const double v4 = p_t / (atol + fabs(p_t) * rtol), v7 = p_phi / (atol + fabs(p_phi) * rtol);
-                        d0s = fma(v4, v4, d0s); d0s = fma(v7, v7, d0s);
-                    }
-                    const double d0 = rms8(d0s), d1 = rms8(d1s);
-                    double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
-                    h0 = fmin(h0, interval);
-                    double y1[RK_NC], f1[RK_NC], d2s = 0.0;
-#pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) y1[i] = y6[i] + h0 * f6[i];
-                    rk_rhs(a.R_S, r_floor, p_t, p_phi, y1, tc, f1);
-#pragma unroll
-                    for (int i = 0; i < RK_NC; ++i) { const double v2 = (f1[i] - f6[i]) / sc[i]; d2s = fma(v2, v2, d2s); }
-                    const double d2 = rms8(d2s) / h0;
-                    double h1;
-                    if (d1 <= 1e-15 && d2 <= 1e-15) h1 = fmax(1e-6, h0 * 1e-3);
-                    else h1 = pow(0.01 / fmax(d1, d2), 0.2);
-                    h_abs = fmin(fmin(100 * h0, h1), fmin(interval, max_step));
-                    y[0] = y6[0]; y[1] = y6[1]; y[2] = y6[3]; y[3] = y6[4];
-                    f[0] = f6[0]; f[1] = f6[1]; f[2] = f6[3]; f[3] = f6[4];
+                    r_out = a.r_out > 0.0 ? a.r_out : y[1] * 2.0;
                     g0 = y[1] - a.r_in; g1 = y[1] - r_out;                        // ivp.py:650
                     npts = 1; attempts = 0; fresh = true; rejected = false;
+                    if constexpr (Sys::PATHS) write_point(a, idx, 0, t, y, sys.p_t, sys.p_phi);
                     active = (interval != 0.0);
-                    if (!active) {
-                        double *o = a.out_state + idx * 8;
-                        o[0] = y[0]; o[1] = y[1]; o[2] = LP_PI_D / 2; o[3] = y[2]; o[4] = p_t; o[5] = y[3]; o[6] = 0.0; o[7] = p_phi;
-                        a.out_lambda[idx] = t;
-                        a.out_outcome[idx] = (y[1] <= a.r_in * 1.1) ? -1 : 1;
-                        if (a.out_nsteps) { a.out_nsteps[2 * idx] = 1; a.out_nsteps[2 * idx + 1] = 2; }
-                        if (a.out_status) a.out_status[idx] = 0;
-                    }
+                    // zero-length interval: solve_ivp returns the initial point, status 0
+                    if (!active) rk_write_result(a, sys, idx, y, t, 1, 2, 0);
                 }
             }
         }
         if (!__any_sync(full, active)) {
-            if (queue_empty) break;
+            if (queue.empty) break;
             continue;
         }
         if (!active) continue;
@@ -739,103 +624,70 @@ lp_rk45_eq_kernel(const Rk45Args a)
             if (ha > max_step) ha = max_step; else if (ha < min_step) ha = min_step;
             fresh = false; rejected = false;
         }
-        int status = 2;
+        int status = 2;                 // 2 = still running
         double t_fin = t;
-        double yf[RK_EQ];
+        double yf[NC];
 #pragma unroll
-        for (int i = 0; i < RK_EQ; ++i) yf[i] = y[i];
+        for (int i = 0; i < NC; ++i) yf[i] = y[i];
 
         if (ha < min_step) {
-            status = -1;
+            status = -1;                // TOO_SMALL_STEP -> solve_ivp status -1, last accepted point stays
         } else {
             double t_new = t + ha;
             if (t_new - t_bound > 0) t_new = t_bound;
             const double h = t_new - t;
             ha = fabs(h);
             attempts++;
-            double K[7][RK_EQ];
+            double K[7][NC], y_new[NC];
 #pragma unroll
-            for (int i = 0; i < RK_EQ; ++i) K[0][i] = f[i];
-            double y_new[RK_EQ];
-            int r_hi_min = 0x7fffffff;
-            rk_eq_stages<true>(a.R_S, r_floor, p_t, p_phi, pp2, h, y, K, y_new, r_hi_min);
-            // a stage at or (by less than one high word) above the floor: the tested form decides — cold
-            if (r_hi_min <= __double2hiint(r_floor)) rk_eq_stages<false>(a.R_S, r_floor, p_t, p_phi, pp2, h, y, K, y_new, r_hi_min);
-            double esum = 0.0, en[RK_EQ], es[RK_EQ];
-#pragma unroll
-            for (int i = 0; i < RK_EQ; ++i) {
-                es[i] = atol + max_sel(fabs(y[i]), fabs(y_new[i])) * rtol;
-                double acc = K[0][i] * c_E[0];
-                acc = fma(K[2][i], c_E[2], acc);
-                acc = fma(K[3][i], c_E[3], acc);
-                acc = fma(K[4][i], c_E[4], acc);
-                acc = fma(K[5][i], c_E[5], acc);
-                acc = fma(K[6][i], c_E[6], acc);
-                en[i] = acc * h;
-            }
-#pragma unroll
-            for (int i = 0; i < RK_EQ; ++i) {
-                const double e = en[i] * fast_rcp(es[i]);        // es >= atol > 0; only the controller sees it
-                esum = fma(e, e, esum);
-            }
-            if (!isfinite(esum)) {
-                esum = 0.0;
-#pragma unroll
-                for (int i = 0; i < RK_EQ; ++i) {
-                    const double e = en[i] / es[i];
-                    esum = fma(e, e, esum);
-                }
-            }
-            double error_norm, pow_term;                 // see lp_rk45_kernel
+            for (int i = 0; i < NC; ++i) K[0][i] = f[i];
+            sys.stages(a, r_floor, h, y, K, y_new);
+            const double esum = rk_error_sq(K, y, y_new, h, rtol, atol);
+            // one power for the accept and the reject controller (rk.py:155-170): divergent branches
+            // would each run their own copy for the whole warp
+            // (fast_pow: the controller on the SQUARED norm, 0.9 err^-0.2 = 0.9 (esum / 8)^-0.1 by
+            // inv_tenth_root — a few ulp, the level at which scipy's own BLAS stage sums already differ
+            // from any restatement; error_norm is then only compared with 0 and 1, which the square
+            // preserves; tests hold the accept/reject sequences identical)
+            double error_norm, pow_term;
             if (a.fast_pow) { error_norm = esum * 0.125; pow_term = 0.9 * inv_tenth_root(error_norm); }
             else { error_norm = rms8(esum); pow_term = 0.9 * pow(error_norm, -0.2); }
             if (error_norm < 1) {
                 double factor = (error_norm == 0) ? 10.0 : min_sel(pow_term, 10.0);
                 if (rejected) factor = min_sel(factor, 1.0);
                 ha *= factor;
+                // ---- accepted: events on the new point (ivp.py:676-699) ----
                 const double gn0 = y_new[1] - a.r_in, gn1 = y_new[1] - r_out;
-                const bool act0 = (g0 >= 0) && (gn0 <= 0);
-                const bool act1 = (g1 <= 0) && (gn1 >= 0);
+                const bool act0 = (g0 >= 0) && (gn0 <= 0);       // direction -1
+                const bool act1 = (g1 <= 0) && (gn1 >= 0);       // direction +1
                 t_fin = t_new;
 #pragma unroll
-                for (int i = 0; i < RK_EQ; ++i) yf[i] = y_new[i];
-                if (t_new - t_bound >= 0) status = 0;
+                for (int i = 0; i < NC; ++i) yf[i] = y_new[i];
+                if (t_new - t_bound >= 0) status = 0;            // OdeSolver.step: finished
                 if (act0 || act1) {
-                    double q[4];
-#pragma unroll
-                    for (int m = 0; m < 4; ++m) {
-                        double acc = K[0][1] * c_P[0][m];
-#pragma unroll
-                        for (int j = 2; j < 7; ++j) acc = fma(K[j][1], c_P[j][m], acc);
-                        q[m] = acc;
-                    }
-                    double root = 0.0;
-                    if (act0) root = rk_brentq(q, h, y[1], t, a.r_in, t, t_new);
-                    if (act1) {
-                        const double r1 = rk_brentq(q, h, y[1], t, r_out, t, t_new);
-                        root = (act0 && root <= r1) ? root : r1;
-                    }
+                    t_fin = rk_event_root(K, y, t, h, t_new, a.r_in, r_out, act0, act1, yf);
                     status = 1;
-                    t_fin = root;
-                    const double x = (root - t) / h;
-#pragma unroll
-                    for (int i = 0; i < RK_EQ; ++i) {
-                        double qi[4];
-#pragma unroll
-                        for (int m = 0; m < 4; ++m) {
-                            double acc = K[0][i] * c_P[0][m];
-#pragma unroll
-                            for (int j = 2; j < 7; ++j) acc = fma(K[j][i], c_P[j][m], acc);
-                            qi[m] = acc;
-                        }
-                        yf[i] = dense_comp(qi, h, y[i], x);
-                    }
                 }
                 g0 = gn0; g1 = gn1;
+                if constexpr (Sys::DENSE) {
+                    if (a.dense && npts < a.max_points) {
+                        // the step's interpolant for OdeResult.sol: h and Q = K^T P (rk.py:178-180)
+                        double *row = a.dense + ((size_t)idx * a.max_points + npts) * 25;
+                        row[0] = h;
+#pragma unroll
+                        for (int i = 0; i < NC; ++i) {
+                            double q[4];
+                            dense_q(K, i, q);
+#pragma unroll
+                            for (int m = 0; m < 4; ++m) row[1 + 4 * i + m] = q[m];
+                        }
+                    }
+                }
+                if constexpr (Sys::PATHS) write_point(a, idx, npts, t_fin, yf, sys.p_t, sys.p_phi);
                 npts++;
                 t = t_new;
 #pragma unroll
-                for (int i = 0; i < RK_EQ; ++i) { y[i] = y_new[i]; f[i] = K[6][i]; }
+                for (int i = 0; i < NC; ++i) { y[i] = y_new[i]; f[i] = K[6][i]; }
                 fresh = true;
             } else {
                 ha *= max_sel(pow_term, 0.2);
@@ -845,28 +697,60 @@ lp_rk45_eq_kernel(const Rk45Args a)
         h_abs = ha;
 
         if (status != 2) {
-            double *o = a.out_state + idx * 8;
-            o[0] = yf[0]; o[1] = yf[1]; o[2] = LP_PI_D / 2; o[3] = yf[2];
-            o[4] = p_t; o[5] = yf[3]; o[6] = 0.0; o[7] = p_phi;
-            a.out_lambda[idx] = t_fin;
-            a.out_outcome[idx] = (yf[1] <= a.r_in * 1.1) ? -1 : 1;
-            if (a.out_nsteps) { a.out_nsteps[2 * idx] = npts; a.out_nsteps[2 * idx + 1] = 2 + 6 * attempts; }
-            if (a.out_status) a.out_status[idx] = (int8_t)status;
+            rk_write_result(a, sys, idx, yf, t_fin, npts, 2 + 6 * attempts, status);
             active = false;
         }
     }
 }
 
-template <int MINB>
-static int rk45_launch_eq(const Rk45Args &a, cudaStream_t stream)
+template <int MINB, int METRIC, bool DENSE = false>
+__global__ void __launch_bounds__(RK_BLOCK, MINB)
+lp_rk45_kernel(const Rk45Args a)
 {
-    int grid = 0;
-    int rc = lp_grid_for((const void *)lp_rk45_eq_kernel<MINB>, RK_BLOCK, &grid);
-    if (rc != LP_OK) return rc;
-    const long long chunks = (a.n + RK_BLOCK - 1) / RK_BLOCK;
-    if (chunks < grid) grid = (int)chunks;
-    lp_rk45_eq_kernel<MINB><<<grid, RK_BLOCK, 0, stream>>>(a);
-    return lp_check_launch();
+    rk45_solve<RkSixSystem<METRIC, DENSE>>(a);
+}
+
+template <int MINB>
+__global__ void __launch_bounds__(RK_BLOCK, MINB)
+lp_rk45_eq_kernel(const Rk45Args a)
+{
+    rk45_solve<RkEquatorialSystem>(a);
+}
+
+// The RK45 tuning knobs (DESIGN.md §4), read once per process.
+struct Rk45Knobs {
+    int minb;       // LP_RK45_MINB = 2..4: resident CTAs per SM of the six-component kernel
+    int eq_minb;    // LP_RK45_EQ_MINB = 3..6: the same for the equatorial kernel
+    int refill;     // LP_RK45_REFILL = 1..32: idle lanes before a refill
+    int fast_pow;   // LP_RK45_POW = 0 | 1: pow() or inv_tenth_root() in the step controller; -1 unset
+    int eq;         // LP_RK45_EQ = 0 | 1: the equatorial kernel for the `alphas` batch entry
+};
+
+static int env_int(const char *name, int lo, int hi, int dflt)
+{
+    const char *e = getenv(name);
+    const int v = e ? atoi(e) : 0;
+    return (v >= lo && v <= hi) ? v : dflt;
+}
+
+static const Rk45Knobs &rk45_knobs()
+{
+    static const Rk45Knobs k = [] {
+        Rk45Knobs r;
+        // resident CTAs per SM ptxas must fit: the kernels are bound by the latency of the right-hand side's
+        // dependent chains, so resident warps win until the spills start.  Six-component kernel: 2 -> 240
+        // registers, no spills; 3 -> 168; 4 -> 128 (spills).  Round 1 measured 3 best on the 4K frame, which
+        // that kernel then integrated; the frame now runs the equatorial kernel (4 -> 128 registers).
+        r.minb = env_int("LP_RK45_MINB", 2, 4, RK_DEFAULT_MINB);
+        r.eq_minb = env_int("LP_RK45_EQ_MINB", 3, 6, RK_DEFAULT_EQ_MINB);
+        r.refill = env_int("LP_RK45_REFILL", 1, 32, RK_REFILL_MIN);
+        const char *p = getenv("LP_RK45_POW");
+        r.fast_pow = p ? (atoi(p) != 0) : -1;
+        const char *e = getenv("LP_RK45_EQ");
+        r.eq = e ? (atoi(e) != 0) : RK_DEFAULT_EQ;
+        return r;
+    }();
+    return k;
 }
 
 static int rk45_launch(bool metric_is_kerr, double kerr_a, const double *alphas, const double *state0, int64_t n,
@@ -878,7 +762,6 @@ static int rk45_launch(bool metric_is_kerr, double kerr_a, const double *alphas,
                        double *traj, int32_t max_points, int32_t *n_points, cudaStream_t stream,
                        double *dense = nullptr)
 {
-    (void)M;
     if (n < 0 || max_points < 0) return LP_ERR_INVALID_ARG;
     if (n == 0) return LP_OK;
     if ((!alphas && !state0) || !out_state || !out_lambda || !out_outcome) return LP_ERR_INVALID_ARG;
@@ -898,74 +781,33 @@ static int rk45_launch(bool metric_is_kerr, double kerr_a, const double *alphas,
     a.out_state = out_state; a.out_lambda = out_lambda; a.out_outcome = out_outcome;
     a.out_nsteps = out_nsteps; a.out_status = out_status;
     a.traj = traj; a.max_points = max_points; a.n_points = n_points; a.dense = dense;
-    // resident CTAs per SM ptxas must fit: 2 -> 202 registers, no spills; 3 -> 168; 4 -> 128 (spills).
-    // LP_RK45_MINB selects (tuning knob); the default is the measured best (4K frame: 2 -> 184 ms,
-    // 3 -> 154 ms, 4 -> 164 ms: the kernel is bound by the latency of the right-hand side's dependent
-    // chains, so resident warps win until the spills start).
-    static int minb = 0;
-    if (!minb) {
-        const char *e = getenv("LP_RK45_MINB");
-        const int v = e ? atoi(e) : 0;
-        minb = (v == 2 || v == 3 || v == 4) ? v : RK_DEFAULT_MINB;
-    }
-    static int refill = 0;
-    if (!refill) {
-        const char *e = getenv("LP_RK45_REFILL");
-        const int v = e ? atoi(e) : 0;
-        refill = (v >= 1 && v <= 32) ? v : RK_REFILL_MIN;
-    }
-    a.refill_min = refill;
-    // LP_RK45_POW = 0 | 1: pow() or inv_tenth_root() of the squared norm in the step controller (tuning knob)
-    // default: on in the equatorial batch kernel (4K frame 94 -> 86 ms), off in the six-component kernel of
-    // the single-ray API, whose fixtures were pinned with pow()
-    static int fast_pow = -2;
-    if (fast_pow == -2) {
-        const char *e = getenv("LP_RK45_POW");
-        fast_pow = e ? (atoi(e) != 0) : -1;
-    }
-    a.fast_pow = fast_pow < 0 ? 0 : fast_pow;
+    const Rk45Knobs &k = rk45_knobs();
+    a.refill_min = k.refill;
     const bool kerr = metric_is_kerr;
-    // LP_RK45_EQ = 0 | 1: the equatorial four-component kernel for the `alphas` batch entry (no trajectory)
-    static int eq = -1, eq_minb = 0;
-    if (eq < 0) {
-        const char *e = getenv("LP_RK45_EQ");
-        eq = e ? (atoi(e) != 0) : RK_DEFAULT_EQ;
-        const char *m = getenv("LP_RK45_EQ_MINB");
-        const int v = m ? atoi(m) : 0;
-        eq_minb = (v >= 3 && v <= 6) ? v : RK_DEFAULT_EQ_MINB;
+    // the equatorial four-component kernel serves the `alphas` batch entry (no trajectory, no dense output)
+    const bool eq = k.eq && !kerr && !dense && alphas && !traj && !n_points;
+    // fast_pow default: on in the equatorial batch kernel (4K frame 94 -> 86 ms), off in the six-component
+    // kernel of the single-ray API, whose fixtures were pinned with pow()
+    a.fast_pow = k.fast_pow < 0 ? eq : k.fast_pow;
+    const void *fn;
+    if (eq) {
+        const void *eq_kernels[] = {(const void *)lp_rk45_eq_kernel<3>, (const void *)lp_rk45_eq_kernel<4>,
+                                    (const void *)lp_rk45_eq_kernel<5>, (const void *)lp_rk45_eq_kernel<6>};
+        fn = eq_kernels[k.eq_minb - 3];
+    } else if (dense) {     // single-ray API (OdeResult.sol): the variant that also stores every step's interpolant
+        fn = kerr ? (const void *)lp_rk45_kernel<2, 1, true> : (const void *)lp_rk45_kernel<2, 0, true>;
+    } else if (kerr) {
+        fn = (const void *)lp_rk45_kernel<2, 1>;
+    } else {
+        const void *six_kernels[] = {(const void *)lp_rk45_kernel<2, 0>, (const void *)lp_rk45_kernel<3, 0>,
+                                     (const void *)lp_rk45_kernel<4, 0>};
+        fn = six_kernels[k.minb - 2];
     }
-    if (eq && !kerr && !dense && alphas && !traj && !n_points) {
-        if (fast_pow < 0) a.fast_pow = 1;
-        switch (eq_minb) {
-        case 3: return rk45_launch_eq<3>(a, stream);
-        case 4: return rk45_launch_eq<4>(a, stream);
-        case 5: return rk45_launch_eq<5>(a, stream);
-        default: return rk45_launch_eq<6>(a, stream);
-        }
-    }
-    if (dense) {            // single-ray API (OdeResult.sol): the variant that also stores every step's interpolant
-        const void *fd = kerr ? (const void *)lp_rk45_kernel<2, 1, true> : (const void *)lp_rk45_kernel<2, 0, true>;
-        int gd = 0;
-        int rcd = lp_grid_for(fd, RK_BLOCK, &gd);
-        if (rcd != LP_OK) return rcd;
-        const long long ch = (n + RK_BLOCK - 1) / RK_BLOCK;
-        if (ch < gd) gd = (int)ch;
-        if (kerr) lp_rk45_kernel<2, 1, true><<<gd, RK_BLOCK, 0, stream>>>(a);
-        else lp_rk45_kernel<2, 0, true><<<gd, RK_BLOCK, 0, stream>>>(a);
-        return lp_check_launch();
-    }
-    const void *fn = kerr ? (const void *)lp_rk45_kernel<2, 1>
-                   : minb == 2 ? (const void *)lp_rk45_kernel<2, 0>
-                   : minb == 3 ? (const void *)lp_rk45_kernel<3, 0> : (const void *)lp_rk45_kernel<4, 0>;
     int grid = 0;
-    int rc = lp_grid_for(fn, RK_BLOCK, &grid);
+    const int rc = lp_grid_for(fn, RK_BLOCK, n, &grid);
     if (rc != LP_OK) return rc;
-    const long long chunks = (n + RK_BLOCK - 1) / RK_BLOCK;
-    if (chunks < grid) grid = (int)chunks;
-    if (kerr) lp_rk45_kernel<2, 1><<<grid, RK_BLOCK, 0, stream>>>(a);
-    else if (minb == 2) lp_rk45_kernel<2, 0><<<grid, RK_BLOCK, 0, stream>>>(a);
-    else if (minb == 3) lp_rk45_kernel<3, 0><<<grid, RK_BLOCK, 0, stream>>>(a);
-    else lp_rk45_kernel<4, 0><<<grid, RK_BLOCK, 0, stream>>>(a);
+    void *args[] = {&a};
+    cudaLaunchKernel(fn, grid, RK_BLOCK, args, 0, stream);
     return lp_check_launch();
 }
 

@@ -125,10 +125,8 @@ extern "C" int lp_frame_stats_reduce(const float *fa32, const uint16_t *w16,
     if (n == 0) return LP_OK;
     if (!fa32) return LP_ERR_INVALID_ARG;
     int grid = 0;
-    int rc = lp_grid_for((const void *)lp_stats_reduce_kernel, 256, &grid);
+    int rc = lp_grid_for((const void *)lp_stats_reduce_kernel, 256, n, &grid);
     if (rc != LP_OK) return rc;
-    const long long chunks = (n + 255) / 256;
-    if (chunks < grid) grid = (int)chunks;
     lp_stats_reduce_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(fa32, w16, status, steps, n, stats);
     return lp_check_launch();
 }

@@ -653,10 +653,8 @@ extern "C" int lp_build_alpha_lookup(const lp_camera *h_cam, int32_t row0, int32
     if (n == 0) return LP_OK;
     if (!out_alpha32) return LP_ERR_INVALID_ARG;
     int grid = 0;
-    rc = lp_grid_for((const void *)lp_alpha_lookup_kernel, 256, &grid);
+    rc = lp_grid_for((const void *)lp_alpha_lookup_kernel, 256, n, &grid);
     if (rc != LP_OK) return rc;
-    const long long chunks = (n + 255) / 256;
-    if (chunks < grid) grid = (int)chunks;
     double scale = 1.0;
     for (int i = 0; i < decimals; ++i) scale *= 10.0;
     lp_alpha_lookup_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(cam, row0, n, decimals, scale, out_alpha32);
