@@ -24,8 +24,7 @@ INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(OUT, "liblightpath.so")
 EXT = os.path.join(OUT, "_lp_torch.so")
 
-CU_SOURCES = ["lp_host.cu", "lp_trace.cu", "lp_repack.cu", "lp_peer.cu", "lp_remap.cu", "lp_remap_tma.cu", "lp_shadow.cu", "lp_rk45.cu",
-              "lp_kerr.cu"]
+CU_SOURCES = ["lp_host.cu", "lp_trace.cu", "lp_repack.cu", "lp_peer.cu", "lp_remap.cu", "lp_shadow.cu", "lp_rk45.cu", "lp_kerr.cu"]
 HEADERS = ["lp_internal.cuh", "lp_trace.cuh", "lp_remap.cuh", "lp_sincr.cuh", "lp_sintab.h", os.path.join(INCLUDE, "lightpath.h")]
 
 NVCC_FLAGS = [

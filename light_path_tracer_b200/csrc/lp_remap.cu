@@ -7,7 +7,6 @@
 // neighbouring source texels (L1/L2 resident).  All direction math is fp64 like the
 // reference's; what must match is the INTEGER source index.
 #include "lp_remap.cuh"
-#include <stdlib.h>
 
 template <typename T>
 __global__ void __launch_bounds__(256)
@@ -32,10 +31,6 @@ lp_remap_kernel(const RemapArgs a, const CamConsts cam)
 // the one-pixel-per-thread kernel (the remap is latency-, not bandwidth-limited otherwise).
 // Same per-pixel decisions as remap_pixel(), same integer source index.
 #define LP_REMAP4_BLOCK 128
-#define LP_REMAP4_DEFAULT_QUADS 1
-#define LP_REMAP_DEFAULT_TMA 0
-
-int lp_remap_try_tma(const RemapArgs &a, const CamConsts &cam, int src_dtype, int rows, cudaStream_t stream);
 
 // sin and cos on [0, pi/2] (final_alpha of a sampled pixel is a float32 in that range): one
 // conditional reflection about pi/4 instead of a general quadrant reduction, the fdlibm kernel
@@ -139,37 +134,26 @@ __device__ __forceinline__ void quad_store(float *out, long long i, const float 
     dst[2] = make_float4(o[8], o[9], o[10], o[11]);
 }
 
-// QUADS consecutive quads per thread, software-pipelined: all lookups are loaded up front, the
-// gathers of quad q are issued before the math of quad q+1 starts (so they are in flight under
-// it), all stores come last.
-template <int MINB, int QUADS>
-__global__ void __launch_bounds__(LP_REMAP4_BLOCK, MINB)
+// One quad per thread: both lookup vectors are loaded first, then the index math of the four
+// pixels, their gathers, and the three stores.
+__global__ void __launch_bounds__(LP_REMAP4_BLOCK, 12)
 lp_remap_f32rgb_x4_kernel(const RemapArgs a, const CamConsts cam)
 {
-    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * (4 * QUADS);
+    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (i >= a.n) return;
     int row, col;
     pixel_row_col(i, a.n, cam.width, a.row0, row, col);
-    float4 fa4[QUADS];
-    ushort4 w4[QUADS];
-#pragma unroll
-    for (int q = 0; q < QUADS; ++q) {
-        fa4[q] = __ldg(reinterpret_cast<const float4 *>(a.fa32 + i) + q);
-        w4[q] = a.w16 ? __ldg(reinterpret_cast<const ushort4 *>(a.w16 + i) + q) : make_ushort4(0, 0, 0, 0);
-    }
+    const float4 fa4 = __ldg(reinterpret_cast<const float4 *>(a.fa32 + i));
+    const ushort4 w4 = a.w16 ? __ldg(reinterpret_cast<const ushort4 *>(a.w16 + i)) : make_ushort4(0, 0, 0, 0);
     const float *__restrict__ src = (const float *)a.src;
     // row-constant parts of the two dot products A = v.e_x, B = v.e_y (v = (x_cam, y_cam, 1))
     const double yc = cam_y(cam, row);
     const double Ay = fma(yc, cam.ex1, cam.ex2), By = fma(yc, cam.ey1, cam.ey2);
-    float o[QUADS][12];
-    int off[QUADS][4];
-#pragma unroll
-    for (int q = 0; q < QUADS; ++q) {
-        quad_offsets(a, cam, col + 4 * q, Ay, By, fa4[q], w4[q], o[q], off[q]);
-        quad_gather(src, off[q], o[q]);
-    }
-#pragma unroll
-    for (int q = 0; q < QUADS; ++q) quad_store((float *)a.out, i + 4 * q, o[q]);
+    float o[12];
+    int off[4];
+    quad_offsets(a, cam, col, Ay, By, fa4, w4, o, off);
+    quad_gather(src, off, o);
+    quad_store((float *)a.out, i, o);
 }
 
 extern "C" int lp_remap(const void *src, int32_t src_dtype, int32_t channels,
@@ -195,34 +179,13 @@ extern "C" int lp_remap(const void *src, int32_t src_dtype, int32_t channels,
     if (a.n == 0) return LP_OK;
     if (!src || !out || !fa32) return LP_ERR_INVALID_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    // LP_REMAP_TMA = 1: the TMA-staged kernel (lp_remap_tma.cu) for float32 / uint8 RGB images
-    static int use_tma = -1;
-    if (use_tma < 0) {
-        const char *e = getenv("LP_REMAP_TMA");
-        use_tma = e ? atoi(e) : LP_REMAP_DEFAULT_TMA;
-    }
-    if (use_tma > 0) {
-        const int t = lp_remap_try_tma(a, cam, src_dtype, rows, st);
-        if (t != 0) return t > 0 ? LP_OK : t;
-    }
     if (src_dtype == LP_DTYPE_F32 && channels == 3 && sampling == LP_SAMPLE_NEAREST && cam.width % 4 == 0 &&
         (long long)cam.height * cam.width * 3 < 0x7fffffffLL &&
         ((uintptr_t)out % 16) == 0 && ((uintptr_t)fa32 % 16) == 0 && (!w16 || ((uintptr_t)w16 % 8) == 0)) {
         const long long quads = a.n / 4;                 // width % 4 == 0 -> n % 4 == 0
         const long long blocks = (quads + LP_REMAP4_BLOCK - 1) / LP_REMAP4_BLOCK;
         if (blocks > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
-        // LP_REMAP_QUADS = 1 | 2 quads per thread (tuning knob); 2 needs width % 8 == 0
-        static int quads_per_thread = 0;
-        if (!quads_per_thread) {
-            const char *e = getenv("LP_REMAP_QUADS");
-            const int v = e ? atoi(e) : 0;
-            quads_per_thread = (v == 1 || v == 2) ? v : LP_REMAP4_DEFAULT_QUADS;
-        }
-        const int qpt = (quads_per_thread == 2 && cam.width % 8 == 0) ? 2 : 1;
-        const long long threads = (quads + qpt - 1) / qpt;
-        const long long nblocks = (threads + LP_REMAP4_BLOCK - 1) / LP_REMAP4_BLOCK;
-        if (qpt == 2) lp_remap_f32rgb_x4_kernel<8, 2><<<(unsigned)nblocks, LP_REMAP4_BLOCK, 0, st>>>(a, cam);
-        else lp_remap_f32rgb_x4_kernel<12, 1><<<(unsigned)nblocks, LP_REMAP4_BLOCK, 0, st>>>(a, cam);
+        lp_remap_f32rgb_x4_kernel<<<(unsigned)blocks, LP_REMAP4_BLOCK, 0, st>>>(a, cam);
         return lp_check_launch();
     }
     const void *fn;

@@ -1,8 +1,7 @@
 """GPU parity of the opt-in KERNEL VARIANTS that are selected by environment knobs (the library reads a
 knob once per process, so every variant renders in its own subprocess): 2-step loop trips of the frame
-kernel (LP_RENDER_TRIP, lp_trace.cu), warp-tile shapes (LP_RENDER_TILE_H), CTA sizes (LP_TRACE_BLOCK)
-and the TMA-staged remap (LP_REMAP_TMA, lp_remap_tma.cu).  None of them may change a single output
-byte: they only move work between warps or stage the same source texels differently (reference:
+kernel (LP_RENDER_TRIP, lp_trace.cu), warp-tile shapes (LP_RENDER_TILE_H) and CTA sizes (LP_TRACE_BLOCK).
+None of them may change a single output byte: they only move work between warps (reference:
 metrics.py:49-145, image_lens.py:133-178, :296-397)."""
 import hashlib
 import json
@@ -59,7 +58,7 @@ print("RESULT " + json.dumps(out, sort_keys=True))
 
 def _run(env_extra):
     env = dict(os.environ)
-    for k in ("LP_RENDER_TRIP", "LP_RENDER_TILE_H", "LP_TRACE_BLOCK", "LP_REMAP_TMA"):
+    for k in ("LP_RENDER_TRIP", "LP_RENDER_TILE_H", "LP_TRACE_BLOCK"):
         env.pop(k, None)
     env.update(env_extra)
     r = subprocess.run([sys.executable, "-c", CHILD % {"root": ROOT}], env=env, capture_output=True, text=True,
@@ -79,7 +78,6 @@ def default_outputs(native):
     {"LP_RENDER_TILE_H": "1"},
     {"LP_RENDER_TILE_H": "2", "LP_TRACE_BLOCK": "128"},
     {"LP_TRACE_BLOCK": "32"},
-    {"LP_REMAP_TMA": "1"},
 ], ids=lambda k: ",".join("%s=%s" % kv for kv in sorted(k.items())))
 def test_knob_variants_are_bit_identical(native, default_outputs, knobs):
     got = _run(knobs)

@@ -1,7 +1,7 @@
 """One small, fixed workload per case for ncu captures (gpurun: plain run first, then under ncu).
 
-    python tools/ncu_case.py render_hybrid | render_u8 | render_strict | trace_hybrid | remap | remap_tma | rk45 | rk45_full | kerr | shadow
-(remap_tma and rk45_full set LP_REMAP_TMA=1 / LP_RK45_EQ=0 for their process)
+    python tools/ncu_case.py render_hybrid | render_u8 | render_strict | trace_hybrid | remap | rk45 | rk45_full | kerr | shadow
+(rk45_full sets LP_RK45_EQ=0 for its process)
 """
 import os
 import sys
@@ -14,8 +14,6 @@ from light_path_tracer_b200 import image_lens as il, geodesic_tracer as gt, blac
 from light_path_tracer_b200.metrics import Schwarzschild  # noqa: E402
 
 case = sys.argv[1]
-if case == "remap_tma":
-    os.environ["LP_REMAP_TMA"] = "1"
 if case == "rk45_full":
     os.environ["LP_RK45_EQ"] = "0"
 reps = int(sys.argv[2]) if len(sys.argv) > 2 else 3
@@ -34,7 +32,7 @@ for _ in range(reps):
     elif case == "trace_hybrid":
         a = il.build_alpha_lookup((H, W), fov, device=True)
         m.trace_alpha_table(a, 100.0, flags=4)
-    elif case in ("remap", "remap_tma"):
+    elif case == "remap":
         a = il.build_alpha_lookup((H, W), fov, device=True)
         fa, w = m.trace_alpha_table(a, 100.0)
         il.render_lensed_image(src, a, fa, w, 0.0, fov)

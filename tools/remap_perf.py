@@ -1,6 +1,5 @@
-"""Stand-alone remap (render_lensed_image) timings: the direct-gather kernels vs the TMA-staged
-kernel (LP_REMAP_TMA, read once per process — the caller runs this script once per setting), at
-4K, float32 and uint8 RGB, nearest and bilinear.  CUDA events, L2 flushed between launches."""
+"""Stand-alone remap (render_lensed_image) timings at 4K (r_obs 100 and 15) and 1080p, float32 and
+uint8 RGB, nearest and bilinear.  CUDA events, L2 flushed between launches."""
 import os
 import sys
 
@@ -14,7 +13,6 @@ from light_path_tracer_b200.synthetic import checkerboard  # noqa: E402
 
 metric = Schwarzschild(1.0)
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-print("LP_REMAP_TMA=%s" % os.environ.get("LP_REMAP_TMA", "default"))
 for H, W, r_obs in ((2160, 3840, 100.0), (2160, 3840, 15.0), (1080, 1920, 100.0)):
     vfov = np.radians(40.0)
     fov = (2 * np.arctan(np.tan(vfov / 2) * W / H), vfov)
