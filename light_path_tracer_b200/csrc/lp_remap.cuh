@@ -54,8 +54,9 @@ __device__ __forceinline__ long long pymod(long long a, long long n)
 // (which keep ptxas from interleaving neighbouring pixels' dependency chains) for straight-line
 // code accurate to a few ulp.
 // ---------------------------------------------------------------------------
-// Source direction of an escaped pixel -> pinhole plane coordinates (image_lens.py:310-352).
-// Returns front (src_vz > 1e-12) and the continuous source pixel coordinates.
+// Source direction of an escaped pixel -> pinhole plane coordinates (image_lens.py:310-352), in two parts:
+// source_dir_xy forms the direction (front = src_vz > 1e-12, and (sx, sy) / sz), source_px the continuous
+// source pixel coordinates.  The mirror-image frame kernel forms the direction once for all images of a ray.
 //
 // The reference normalises the pixel ray v, takes theta = arctan2(v.e_x, v.e_y) and then
 // sin(theta), cos(theta).  theta is invariant under scaling of v, and sin/cos of an arctan2
@@ -67,10 +68,14 @@ __device__ __forceinline__ long long pymod(long long a, long long n)
 // fa (RayResult::cf, sf, fa).  The lookup holds fa32 = float32(fa), so the angle the reference takes the
 // sine and cosine of is fa + d with d = fa32 - fa, |d| <= 3e-8 fa: cos(fa32) = c - s d, sin(fa32) = s + c d
 // up to d^2 / 2 < 5e-16 — far inside the 1e-12 the source index needs — instead of a second sincos.
+struct SrcDir {
+    double qx, qy;               // pinhole-plane direction of the source: (sx, sy) / sz
+    bool front;                  // sz > 1e-12
+};
+
 template <bool DIR = false>
-__device__ __forceinline__ bool source_coords_xy(const CamConsts &cam, double xc, double yc, float fa32,
-                                                 double &px, double &py,
-                                                 double fa64 = 0.0, double cfa = 0.0, double sfa = 0.0)
+__device__ __forceinline__ SrcDir source_dir_xy(const CamConsts &cam, double xc, double yc, float fa32,
+                                                double fa64 = 0.0, double cfa = 0.0, double sfa = 0.0)
 {
     const double A = fma(xc, cam.ex0, fma(yc, cam.ex1, cam.ex2));
     const double B = fma(xc, cam.ey0, fma(yc, cam.ey1, cam.ey2));
@@ -92,12 +97,51 @@ __device__ __forceinline__ bool source_coords_xy(const CamConsts &cam, double xc
     const double sx = fma(cf, cam.d0, sf * tx);
     const double sy = fma(cf, cam.d1, sf * ty);
     const double sz = fma(cf, cam.d2, sf * tz);
-    const bool front = sz > 1e-12;
-    const double isz = fast_rcp(front ? sz : 1.0);
+    SrcDir s;
+    s.front = sz > 1e-12;
+    const double isz = fast_rcp(s.front ? sz : 1.0);
+    s.qx = sx * isz;
+    s.qy = sy * isz;
+    return s;
+}
+
+// the per-pixel part: continuous source pixel coordinates of a direction
+__device__ __forceinline__ void source_px(const CamConsts &cam, const SrcDir &s, double &px, double &py)
+{
     // behind the camera: zeros * f + n/2 (image_lens.py:356-361)
-    px = front ? fma(sx * isz, cam.fx, cam.half_w) : cam.half_w;    // image_lens.py:374
-    py = front ? fma(sy * isz, cam.fy, cam.half_h) : cam.half_h;
-    return front;
+    px = s.front ? fma(s.qx, cam.fx, cam.half_w) : cam.half_w;    // image_lens.py:374
+    py = s.front ? fma(s.qy, cam.fy, cam.half_h) : cam.half_h;
+}
+
+template <bool DIR = false>
+__device__ __forceinline__ bool source_coords_xy(const CamConsts &cam, double xc, double yc, float fa32,
+                                                 double &px, double &py,
+                                                 double fa64 = 0.0, double cfa = 0.0, double sfa = 0.0)
+{
+    const SrcDir s = source_dir_xy<DIR>(cam, xc, yc, fa32, fa64, cfa, sfa);
+    source_px(cam, s, px, py);
+    return s.front;
+}
+
+// fast3 layout (see remap_pixel_dir): the element offset o of the source pixel, or false when the pixel
+// is out of frame (magenta).  cvt.rni.s32.f64 rounds half to even like np.rint and saturates, so a far
+// out-of-frame coordinate stays out of frame (same as lp_remap_f32rgb_x4_kernel, pixel-identical).
+__device__ __forceinline__ bool fast3_source(const RemapArgs &a, const CamConsts &cam, const SrcDir &s, int &o)
+{
+    double px, py;
+    source_px(cam, s, px, py);
+    const int H = cam.height, W = cam.width;
+    int ix = __double2int_rn(px), iy = __double2int_rn(py);
+    bool ok;
+    if (a.loop_around) {
+        ix %= W; ix += (ix < 0) ? W : 0;
+        iy %= H; iy += (iy < 0) ? H : 0;
+        ok = true;
+    } else {
+        ok = s.front && (unsigned)ix < (unsigned)W && (unsigned)iy < (unsigned)H;
+    }
+    o = (iy * W + ix) * 3;
+    return ok;
 }
 
 __device__ __forceinline__ bool source_coords(const CamConsts &cam, int row, int col, float fa32,
@@ -106,19 +150,16 @@ __device__ __forceinline__ bool source_coords(const CamConsts &cam, int row, int
     return source_coords_xy(cam, cam_x(cam, col), cam_y(cam, row), fa32, px, py);
 }
 
-// xc, yc: the pixel's camera-plane coordinates cam_x(col), cam_y(row); DIR: see source_coords_xy
-template <typename T, bool DIR = false>
-__device__ __forceinline__ void remap_pixel_xy(const RemapArgs &a, const CamConsts &cam, T *__restrict__ dst,
-                                               double xc, double yc, float fa32, unsigned wnd,
-                                               double fa64 = 0.0, double cfa = 0.0, double sfa = 0.0)
+// dir(): the pixel's SrcDir, formed only for escaped pixels that are not winding-coloured
+template <typename T, typename Dir>
+__device__ __forceinline__ void remap_pixel_dir(const RemapArgs &a, const CamConsts &cam, T *__restrict__ dst,
+                                                float fa32, unsigned wnd, Dir dir)
 {   // dst: where this pixel's `channels` values go (global memory, or a staging slot)
     const int C = a.channels;
     const T *__restrict__ src = (const T *)a.src;
     if (a.fast3) {
         // the common layout — three channels, nearest sampling, an image whose element count fits
-        // 31 bits — with the decisions of the general code below on 32-bit integers:
-        // cvt.rni.s32.f64 rounds half to even like np.rint and saturates, so a far out-of-frame
-        // coordinate stays out of frame (same as lp_remap_f32rgb_x4_kernel, pixel-identical)
+        // 31 bits — with the decisions of the general code below on 32-bit integers (fast3_source)
         if (!isfinite(fa32)) { dst[0] = (T)0; dst[1] = (T)0; dst[2] = (T)0; return; }
         if (fa32 > LP_HALF_PI_F32) {
             const unsigned k = wnd > 4u ? 4u : wnd;
@@ -126,24 +167,13 @@ __device__ __forceinline__ void remap_pixel_xy(const RemapArgs &a, const CamCons
             dst[2] = colour<T>(c_wind_rgb[k][2], a.u8_scale);
             return;
         }
-        double px, py;
-        const bool front = source_coords_xy<DIR>(cam, xc, yc, fa32, px, py, fa64, cfa, sfa);
-        const int H = cam.height, W = cam.width;
-        int ix = __double2int_rn(px), iy = __double2int_rn(py);
-        bool ok;
-        if (a.loop_around) {
-            ix %= W; ix += (ix < 0) ? W : 0;
-            iy %= H; iy += (iy < 0) ? H : 0;
-            ok = true;
-        } else {
-            ok = front && (unsigned)ix < (unsigned)W && (unsigned)iy < (unsigned)H;
-        }
-        if (!ok) {
+        int o;
+        if (!fast3_source(a, cam, dir(), o)) {
             const T one = colour<T>(1.0f, a.u8_scale);
             dst[0] = one; dst[1] = (T)0; dst[2] = one;
             return;
         }
-        const T *s = src + (iy * W + ix) * 3;
+        const T *s = src + o;
         dst[0] = __ldg(s); dst[1] = __ldg(s + 1); dst[2] = __ldg(s + 2);
         return;
     }
@@ -160,8 +190,10 @@ __device__ __forceinline__ void remap_pixel_xy(const RemapArgs &a, const CamCons
         }
         return;
     }
+    const SrcDir sd = dir();
+    const bool front = sd.front;
     double px, py;
-    const bool front = source_coords_xy<DIR>(cam, xc, yc, fa32, px, py, fa64, cfa, sfa);
+    source_px(cam, sd, px, py);
     const long long H = cam.height, W = cam.width;
     long long ix = (long long)rint(px), iy = (long long)rint(py);   // np.rint -> intp
     bool ok;
@@ -203,6 +235,16 @@ __device__ __forceinline__ void remap_pixel_xy(const RemapArgs &a, const CamCons
         if (sizeof(T) == 1) dst[ch] = (T)(int)rint(v);
         else dst[ch] = (T)v;
     }
+}
+
+// xc, yc: the pixel's camera-plane coordinates cam_x(col), cam_y(row); DIR: see source_coords_xy
+template <typename T, bool DIR = false>
+__device__ __forceinline__ void remap_pixel_xy(const RemapArgs &a, const CamConsts &cam, T *__restrict__ dst,
+                                               double xc, double yc, float fa32, unsigned wnd,
+                                               double fa64 = 0.0, double cfa = 0.0, double sfa = 0.0)
+{
+    remap_pixel_dir<T>(a, cam, dst, fa32, wnd,
+                       [&] { return source_dir_xy<DIR>(cam, xc, yc, fa32, fa64, cfa, sfa); });
 }
 
 template <typename T>

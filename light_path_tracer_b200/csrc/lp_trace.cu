@@ -325,21 +325,96 @@ lp_render_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts c, con
 // xc * d0 = +-0, and a signed zero added to the nonzero d2 (or to yc * d1) disappears.  Pairs are col <-> W - col
 // and row <-> H - row; column 0 / row 0 have no partner and W / 2, H / 2 (even sizes) are their own.
 // So a lane traces a pixel of the traced quarter (or half) once and then remaps and stores each of its
-// images with that image's own camera coordinates: the frame, the lookups and the statistics are the ones
-// of the one-ray-per-pixel kernel.  8x4 warp tiles over the traced domain (see TraceArgs::mx_main).
-// Staged stores (RGB, float32 / 8-bit): each run of an image (a tile row: up to 8 pixels, contiguous in the
-// output, in reverse order for an x mirror) is staged at the same address modulo 16 as its destination; the
-// run's lanes then store the 16-byte (float32) / 8-byte (8-bit) windows that lie inside it as vectors and the
-// run's ends element by element.  A mirror image starts one pixel off the vector grid (column 0 is unpaired).
+// images: the frame, the lookups and the statistics are the ones of the one-ray-per-pixel kernel.  8x4 warp
+// tiles over the traced domain (see TraceArgs::mx_main).
+//
+// The remap's source direction (source_dir_xy) is formed once per ray.  With ex1 == ex2 == ey0 == 0 and d0 == 0
+// (mir_share & 1) the x image's direction is (-qx, qy, front) exactly: A = RN(xc ex0) is odd in xc, B is even, so
+// n2, inv, ct, tz and sz are unchanged while st, tx, sx and qx = sx * isz change sign exactly (round-to-nearest
+// is odd); every signed zero on the way is added to a nonzero term, or to half_w / half_h in source_px.  The
+// same holds for y with ex1 == ey0 == ey2 == 0 and d1 == 0 (mir_share & 2): (qx, -qy).  The cos / sin
+// correction (DIR) depends on the ray only.  A camera whose basis is rotated about d keeps a32 symmetric but
+// not the direction: its images form their own, one image at a time (the bits are warp-uniform, not a
+// template parameter, so that the kernel does not grow by another instantiation).
+//
+// fast3 (the common layout, see remap_pixel_dir) with every image's direction shared: each image's outcome —
+// zeros, winding colour, magenta or a source offset — is decided first, then all images' gathers are issued
+// back to back, then staged / stored.  Every other case remaps one image at a time (remap_pixel_dir).
+// Staged stores (RGB, float32 / 8-bit): the run of tile row q in image k (up to 8 pixels, contiguous in the
+// output, in reverse order for an x mirror) follows from the warp tile's geometry and the mirror flags: it
+// loses a pixel where a lane has no partner (column 0, column W / 2, row 0, row H / 2).  Every image's runs
+// are staged at the same address modulo the vector width as their destinations, then one __syncwarp, then one
+// pass in which lane j of row q stores the run's 16-byte (float32) / 8-byte (8-bit) window j: as a vector,
+// or at the run's two ends as at most three naturally aligned pieces (8 / 4 bytes, 4 / 2 / 1 bytes).
 // ---------------------------------------------------------------------------
-#define LP_MIRROR_RUN_SLOT 112      /* bytes of one staged run: 96 + up to 15 of alignment offset, rounded */
+/* bytes of one staged run: 8 pixels + the alignment offset inside a vector, rounded up to whole vectors:
+   112 for float32 (96 + 12), 32 for 8-bit (24 + 7).  stage[8][4][4][slot] = 14 336 / 4 096 bytes per CTA */
+#define LP_MIRROR_RUN_SLOT(T) (sizeof(T) == 4 ? 112 : 32)
+
+// one naturally aligned piece of N bytes of a staged run to global memory
+template <unsigned N> struct MirrorPiece;
+template <> struct MirrorPiece<1> { typedef unsigned char t; };
+template <> struct MirrorPiece<2> { typedef unsigned short t; };
+template <> struct MirrorPiece<4> { typedef unsigned t; };
+template <> struct MirrorPiece<8> { typedef uint2 t; };
+template <> struct MirrorPiece<16> { typedef uint4 t; };
+template <unsigned N>
+__device__ __forceinline__ void mirror_piece(unsigned char *g, const unsigned char *s, unsigned p)
+{
+    typedef typename MirrorPiece<N>::t P;
+    P *const d = reinterpret_cast<P *>(__builtin_assume_aligned(g + p, N));
+    const P v = *reinterpret_cast<const P *>(s + p);
+    // a global-space store (the destination is the output frame; a generic one would be ST.E)
+    if constexpr (N == 1) asm volatile("st.global.u8 [%0], %1;" :: "l"(d), "h"((unsigned short)v) : "memory");
+    else if constexpr (N == 2) asm volatile("st.global.u16 [%0], %1;" :: "l"(d), "h"(v) : "memory");
+    else if constexpr (N == 4) asm volatile("st.global.u32 [%0], %1;" :: "l"(d), "r"(v) : "memory");
+    else if constexpr (N == 8) asm volatile("st.global.v2.u32 [%0], {%1, %2};" :: "l"(d), "r"(v.x), "r"(v.y) : "memory");
+    else asm volatile("st.global.v4.u32 [%0], {%1, %2, %3, %4};" :: "l"(d), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
+
+// bytes [s, e) of a staged window of VB bytes (0 <= s < e <= VB): climb from s to the window's alignment, then
+// descend to e — a window that holds a run's start (e == VB) or end (s == 0) takes at most three pieces
+template <unsigned VB>
+__device__ __forceinline__ void mirror_window_part(unsigned char *g, const unsigned char *sm, unsigned s, unsigned e)
+{
+    unsigned p = s;
+    if constexpr (VB == 8) {                                     // 8-bit RGB: 1, 2, 4 up, then 4, 2, 1 down
+        if ((p & 1u) && p + 1u <= e) { mirror_piece<1>(g, sm, p); p += 1u; }
+        if ((p & 2u) && p + 2u <= e) { mirror_piece<2>(g, sm, p); p += 2u; }
+        if ((p & 4u) && p + 4u <= e) { mirror_piece<4>(g, sm, p); p += 4u; }
+        if (p + 4u <= e) { mirror_piece<4>(g, sm, p); p += 4u; }
+        if (p + 2u <= e) { mirror_piece<2>(g, sm, p); p += 2u; }
+        if (p + 1u <= e) mirror_piece<1>(g, sm, p);
+    } else {                                                     // float32 RGB: 4, 8 up, then 8, 4 down
+        if ((p & 4u) && p + 4u <= e) { mirror_piece<4>(g, sm, p); p += 4u; }
+        if ((p & 8u) && p + 8u <= e) { mirror_piece<8>(g, sm, p); p += 8u; }
+        if (p + 8u <= e) { mirror_piece<8>(g, sm, p); p += 8u; }
+        if (p + 4u <= e) mirror_piece<4>(g, sm, p);
+    }
+}
+
+// The run of tile row q in image (fx, fy): image row ir, image columns [cs, cs + n); n == 0: no run.  c0, ncol:
+// the warp tile's traced columns c0 .. c0 + ncol - 1; r: the row's traced (tile-local) row, row_ok: it exists.
+__device__ __forceinline__ int mirror_run(const CamConsts &cam, bool fx, bool fy, bool main_x, int c0, int ncol,
+                                          int r, bool row_ok, int &ir, int &cs)
+{
+    const int W = cam.width, H = cam.height;
+    ir = fy ? H - r : r;
+    if (!row_ok || (fy && (r == 0 || 2 * r == H))) return 0;
+    if (!fx) { cs = c0; return ncol; }
+    if (!main_x) return 0;                                       // column 0 alone
+    const int first = c0 + (2 * c0 == W ? 1 : 0), last = c0 + ncol - 1;      // without column W / 2
+    cs = W - last;
+    return last - first + 1;
+}
 
 template <bool FUSED, bool FAST, typename T, int MINB, int TRIP>
 __global__ void __launch_bounds__(LP_TRACE_BLOCK, MINB)
 lp_render_mirror_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts c, const CamConsts cam)
 {
     const LoopRegs L = load_loop_regs<FUSED>(c);
-    __shared__ __align__(16) unsigned char stage[LP_TRACE_BLOCK / 32][4][LP_MIRROR_RUN_SLOT];
+    constexpr unsigned SLOT = LP_MIRROR_RUN_SLOT(T);
+    __shared__ __align__(16) unsigned char stage[LP_TRACE_BLOCK / 32][4][4][SLOT];
     const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5, j = lane & 7, q = lane >> 3;
     const unsigned wt = blockIdx.x * (blockDim.x >> 5) + wrp;
     const unsigned ty = wt / a.mtiles_x, tx = wt - ty * a.mtiles_x;
@@ -363,60 +438,128 @@ lp_render_mirror_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts
     const float fa32 = (float)((res.status == 1) ? res.fa : __longlong_as_double(0x7ff8000000000000LL));
     const unsigned nh = (unsigned)(res.nh < 0 ? 0 : (res.nh > 65535 ? 65535 : res.nh));
     const int W = cam.width, H = cam.height;
-    const bool xm = live && !(a.mir_skip & 1) && col != 0 && 2 * col != W;     // has an x mirror image
-    const bool ym = live && !(a.mir_skip & 2) && r != 0 && 2 * r != H;         // (y mirror: row0 == 0, rows == H)
-    const bool vec = (sizeof(T) == 4 || sizeof(T) == 1) && ra.vec_ok;
-    const int px = 3 * (int)sizeof(T);               // bytes of a staged (RGB) pixel
+    const int skip = a.mir_skip, share = a.mir_share;
+    const bool xm = live && !(skip & 1) && col != 0 && 2 * col != W;        // has an x mirror image
+    const bool ym = live && !(skip & 2) && r != 0 && 2 * r != H;            // (y mirror: row0 == 0, rows == H)
+    if (a.out_fa || a.out_w) {
 #pragma unroll 1
-    for (int k = 0; k < 4; ++k) {
-        if (k & a.mir_skip) continue;                                   // warp-uniform
-        const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
-        const bool has = live && (!fx || xm) && (!fy || ym);
-        const int ic = fx ? W - col : col, ir = fy ? H - r : r;
-        const long long pi = (long long)ir * W + ic;                    // compact tile index of this image
-        if (has) {
+        for (int k = 0; k < 4; ++k) {
+            const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
+            if ((k & skip) || !live || (fx && !xm) || (fy && !ym)) continue;
+            const long long pi = (long long)(fy ? H - r : r) * W + (fx ? W - col : col);   // compact tile index
             if (a.out_fa) ((float *)a.out_fa)[pi] = fa32;
             if (a.out_w) ((unsigned short *)a.out_w)[pi] = (unsigned short)nh;
         }
-        // cam_x(W - col) == -cam_x(col), cam_y(H - r) == -cam_y(r) bit for bit (see above)
-        const double xi = fx ? -xc : xc, yi = fy ? -yc : yc;
-        if (vec) {
-            // the run of tile row q in this image: columns [cmin, cmax] of tile-local row rr
-            int cmin = has ? ic : 0x7fffffff, cmax = has ? ic : -1, rr = has ? ir : -1;
+    }
+    // image k's source direction: the direction of the image k & ~share, with qx / qy negated where k mirrors
+    // an axis in share (see above)
+    auto image_dir = [&](int k) -> SrcDir {
+        const int own = k & ~share;
+        SrcDir dk = source_dir_xy<true>(cam, (own & 1) ? -xc : xc, (own & 2) ? -yc : yc, fa32, res.fa, res.cf, res.sf);
+        if (k & share & 1) dk.qx = -dk.qx;
+        if (k & share & 2) dk.qy = -dk.qy;
+        return dk;
+    };
+    // warp tile geometry of the write-out (the runs of every image follow from it: mirror_run)
+    // (from col and r rather than tx, ty: fewer registers live across the trace.  With a mirror on, column 0 /
+    // row 0 is traced only by the extra tile column / row, whose lanes all hold it)
+    const bool main_x = (skip & 1) || col != 0, main_y = (skip & 2) || r != 0;
+    const int c0 = main_x ? col - j : 0;
+    const int ncol = main_x ? min(8, a.mx_base + a.mx_main - c0) : 1;
+    const bool row_ok = (main_y ? r - a.my_base < a.my_main : q == 0) && wt < a.m_warps;
+    const bool vec = (sizeof(T) == 4 || sizeof(T) == 1) && ra.vec_ok;
+    constexpr int PX = 3 * (int)sizeof(T);                                  // bytes of a staged (RGB) pixel
+    constexpr unsigned VB = (sizeof(T) == 4) ? 16u : 8u;                    // store vector width
+    // image k's pixel in the output, and (vec) its place in the run's staging slot
+    auto image_out = [&](int k) -> T * {
+        const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
+        return (T *)ra.out + ((long long)(fy ? H - r : r) * W + (fx ? W - col : col)) * ra.channels;
+    };
+    auto image_slot = [&](int k) -> T * {
+        const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
+        const int ic = fx ? W - col : col;
+        int ir, cs = 0;
+        mirror_run(cam, fx, fy, main_x, c0, ncol, r, row_ok, ir, cs);
+        const unsigned off = ((unsigned)(uintptr_t)ra.out + ((unsigned)ir * (unsigned)W + (unsigned)cs) * (unsigned)PX) & (VB - 1u);
+        return (T *)(stage[wrp][k][q] + off + (ic - cs) * PX);
+    };
+    if (sizeof(T) <= 4 && ra.fast3 && ((skip | share) & 3) == 3) {     // warp-uniform
+        // 1. outcomes: a colour for the whole ray (zeros: captured / invalid, or the winding colour), else per
+        //    image magenta (src_off < 0) or a source offset
+        const bool ray_colour = !isfinite(fa32) || fa32 > LP_HALF_PI_F32;
+        const SrcDir d0 = image_dir(0);                                     // the ray's, shared by every image
+        int src_off[4];
 #pragma unroll
-            for (int off = 1; off < 8; off <<= 1) {
-                cmin = min(cmin, __shfl_xor_sync(0xffffffffu, cmin, off));
-                cmax = max(cmax, __shfl_xor_sync(0xffffffffu, cmax, off));
-                rr = max(rr, __shfl_xor_sync(0xffffffffu, rr, off));
-            }
-            uintptr_t lo = 0, hi = 0;
-            unsigned char *sb = stage[wrp][q];
-            if (cmax >= 0) {
-                lo = (uintptr_t)ra.out + (uintptr_t)(((long long)rr * W + cmin) * px);
-                hi = lo + (uintptr_t)((cmax - cmin + 1) * px);
-                sb += lo & 15u;                                         // same address modulo 16 as the run
-            }
-            if (has) remap_pixel_xy<T, true>(ra, cam, (T *)(sb + (ic - cmin) * px), xi, yi, fa32, nh, res.fa, res.cf, res.sf);
-            __syncwarp();
-            if (cmax >= 0) {
-                const unsigned vb = (sizeof(T) == 4) ? 16u : 8u;
-                const uintptr_t g = (lo & ~(uintptr_t)(vb - 1u)) + j * vb;      // lane j: the run's window j
-                const unsigned char *s = sb - (lo & (vb - 1u)) + j * vb;
-                if (g < hi) {
-                    if (g >= lo && g + vb <= hi) {
-                        if (vb == 16u) *reinterpret_cast<uint4 *>(g) = *reinterpret_cast<const uint4 *>(s);
-                        else *reinterpret_cast<uint2 *>(g) = *reinterpret_cast<const uint2 *>(s);
-                    } else {
-#pragma unroll
-                        for (unsigned e = 0; e < vb; e += (unsigned)sizeof(T))
-                            if (g + e >= lo && g + e < hi) *reinterpret_cast<T *>(g + e) = *reinterpret_cast<const T *>(s + e);
-                    }
-                }
-            }
-            __syncwarp();      // the staging slots are reused by the next image
-        } else if (has) {
-            remap_pixel_xy<T, true>(ra, cam, (T *)ra.out + pi * ra.channels, xi, yi, fa32, nh, res.fa, res.cf, res.sf);
+        for (int k = 0; k < 4; ++k) {
+            src_off[k] = -1;
+            if (k & skip) continue;                                          // warp-uniform
+            SrcDir dk = d0;                                                  // (every image shares it here)
+            if (k & 1) dk.qx = -dk.qx;
+            if (k & 2) dk.qy = -dk.qy;
+            int o;
+            if (!ray_colour && fast3_source(ra, cam, dk, o)) src_off[k] = o;
         }
+        // 2. every image's gather in flight at once
+        const T *__restrict__ src = (const T *)ra.src;
+        T v[4][3];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
+            if (!(k & skip) && live && (!fx || xm) && (!fy || ym) && src_off[k] >= 0) {
+                const T *s = src + src_off[k];
+                v[k][0] = __ldg(s); v[k][1] = __ldg(s + 1); v[k][2] = __ldg(s + 2);
+            }
+        }
+        // 3. stage (or store)
+        const T one = colour<T>(1.0f, ra.u8_scale);
+        T k0 = one, k1 = (T)0, k2 = one;                                     // magenta
+        if (ray_colour) {
+            k0 = k1 = k2 = (T)0;
+            if (isfinite(fa32)) {
+                const unsigned kw = nh > 4u ? 4u : nh;
+                k0 = colour<T>(c_wind_rgb[kw][0], ra.u8_scale); k1 = colour<T>(c_wind_rgb[kw][1], ra.u8_scale);
+                k2 = colour<T>(c_wind_rgb[kw][2], ra.u8_scale);
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
+            if (!(k & skip) && live && (!fx || xm) && (!fy || ym)) {
+                const bool g = src_off[k] >= 0;
+                T *dst = vec ? image_slot(k) : image_out(k);
+                dst[0] = g ? v[k][0] : k0; dst[1] = g ? v[k][1] : k1; dst[2] = g ? v[k][2] : k2;
+            }
+        }
+    } else {
+        // other channel counts, bilinear sampling, large or float64 images, unshared directions: one image at a time
+#pragma unroll 1
+        for (int k = 0; k < 4; ++k) {
+            const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
+            if ((k & skip) || !live || (fx && !xm) || (fy && !ym)) continue;
+            if (vec) remap_pixel_dir<T>(ra, cam, image_slot(k), fa32, nh, [&] { return image_dir(k); });
+            else remap_pixel_dir<T>(ra, cam, image_out(k), fa32, nh, [&] { return image_dir(k); });
+        }
+    }
+    if (vec) {
+        // one write-out pass: lane j of tile row q stores window j of the row's run in every image
+        __syncwarp();
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            if (k & skip) continue;                                          // warp-uniform
+            int ir, cs = 0;
+            const int n = mirror_run(cam, (k & 1) != 0, (k & 2) != 0, main_x, c0, ncol, r, row_ok, ir, cs);
+            if (n <= 0) continue;
+            unsigned char *const base = (unsigned char *)ra.out + ((long long)ir * W + cs) * PX;     // the run's start
+            const unsigned off = (unsigned)(uintptr_t)base & (VB - 1u), end = off + (unsigned)(n * PX);
+            const unsigned w0 = (unsigned)j * VB;                            // window j: bytes [w0, w0 + VB) of the slot
+            if (w0 >= end) continue;
+            unsigned char *const g = base - off + w0;
+            const unsigned char *const sm = stage[wrp][k][q] + w0;
+            const unsigned s = off > w0 ? off - w0 : 0u, e = min(end - w0, VB);
+            if (s == 0u && e == VB) mirror_piece<VB>(g, sm, 0u);
+            else mirror_window_part<VB>(g, sm, s, e);
+        }
+        __syncwarp();      // reconverge the warp after the lane-divergent stores
     }
     if (a.stats) {
         const unsigned m = (xm ? 2u : 1u) * (ym ? 2u : 1u);
@@ -473,7 +616,10 @@ static int launch_render_mirror(const TraceArgs &a_in, const RemapArgs &ra, cons
     const bool icmp = (fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) != 0;
     TraceArgs a = a_in;
     const int W = cam.width;
-    a.mir_skip = (mir_x ? 0 : 1) | (mir_y ? 0 : 2);
+    a.mir_skip = (int16_t)((mir_x ? 0 : 1) | (mir_y ? 0 : 2));
+    // exact zeros of the basis that carry a mirror over to the remap's source direction (lp_render_mirror_kernel)
+    a.mir_share = (int16_t)((cam.ex1 == 0.0 && cam.ex2 == 0.0 && cam.ey0 == 0.0 && cam.d0 == 0.0 ? 1 : 0) |
+                            (cam.ex1 == 0.0 && cam.ey0 == 0.0 && cam.ey2 == 0.0 && cam.d1 == 0.0 ? 2 : 0));
     a.mx_main = mir_x ? W / 2 : W;           a.mx_base = mir_x ? W - W / 2 : 0;
     a.my_main = mir_y ? rows / 2 : rows;     a.my_base = mir_y ? rows - rows / 2 : 0;
     a.mtx_main = (a.mx_main + 7) / 8;        a.mty_main = (a.my_main + 3) / 4;

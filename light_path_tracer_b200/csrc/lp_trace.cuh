@@ -45,8 +45,9 @@ struct TraceArgs {
     // mirror-image frame kernel (lp_render_mirror_kernel): the traced columns are mx_base .. mx_base + mx_main - 1
     // in mtx_main warp-tile columns of 8, then (x mirror) one more tile column whose first lane traces column 0;
     // the same for tile-local rows in tiles of 4 (my_*).  Image k = 0..3 of a ray is mirrored in x when k & 1 and
-    // in y when k & 2; the images with k & mir_skip do not exist in this launch.
-    int32_t mir_skip;
+    // in y when k & 2; the images with k & mir_skip do not exist in this launch.  Bit 1 (x) / 2 (y) of mir_share:
+    // the camera basis carries that mirror over to the remap's source direction exactly (lp_render_mirror_kernel).
+    int16_t mir_skip, mir_share;
     int32_t mx_main, mx_base, mtx_main, my_main, my_base, mty_main;
     uint32_t mtiles_x;      // warp tiles per tile row
 };
