@@ -1,6 +1,7 @@
 // lp_host.cu — host-side pieces of liblightpath: per-configuration constants,
 // camera frame, error strings, launch helpers.  No device code here.
 #include "lp_internal.cuh"
+#include <stdlib.h>
 #include <string.h>
 
 extern "C" int lp_abi_version(void) { return LP_ABI_VERSION; }
@@ -56,6 +57,22 @@ int lp_grid_for(const void *kernel, int block, long long n, int *grid_out)
     const long long chunks = (n + block - 1) / block;
     if (chunks < *grid_out) *grid_out = (int)chunks;
     return LP_OK;
+}
+
+int lp_launch_ctas(const void *kernel, long long n, long long per_cta, int block, size_t smem, void **args,
+                   cudaStream_t stream)
+{
+    const long long ctas = (n + per_cta - 1) / per_cta;
+    if (ctas > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
+    cudaLaunchKernel(kernel, dim3((unsigned)ctas), dim3((unsigned)block), args, smem, stream);
+    return lp_check_launch();
+}
+
+int lp_env_int(const char *name, int lo, int hi, int dflt)
+{
+    const char *e = getenv(name);
+    const int v = e ? atoi(e) : 0;
+    return (v >= lo && v <= hi) ? v : dflt;
 }
 
 // metrics.py:51-78 evaluated once per configuration instead of once per ray.  Every

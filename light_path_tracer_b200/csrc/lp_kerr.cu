@@ -651,27 +651,29 @@ lp_kerr_queued_kernel(const KerrArgs a, const CamConsts cam)
     }
 }
 
+// The Kerr tuning knobs (DESIGN.md §4), read once per process.  LP_KERR_QUEUE is read at every launch.
+struct KerrKnobs {
+    int refill;     // LP_KERR_REFILL = 1..32: idle lanes before a refill
+    // LP_KERR_MINB = 2..6: resident CTAs per SM ptxas must fit (register cap): the kernel is latency-bound, so
+    // more resident warps win until the spills cost more (the queued kernel is built for 3..5 and runs 4 for
+    // the others)
+    int minb;
+};
+
+static const KerrKnobs &kerr_knobs()
+{
+    static const KerrKnobs k = {lp_env_int("LP_KERR_REFILL", 1, 32, KERR_REFILL_MIN),
+                                lp_env_int("LP_KERR_MINB", 2, 6, KERR_DEFAULT_MINB)};
+    return k;
+}
+
 static int kerr_launch(KerrArgs &a, const CamConsts &cam, cudaStream_t stream)
 {
     if (a.n == 0) return LP_OK;
     a.sin_th_obs = sin(a.theta_obs);
     a.cos_th_obs = cos(a.theta_obs);
-    static int refill = 0;
-    if (!refill) {
-        const char *e = getenv("LP_KERR_REFILL");
-        const int v = e ? atoi(e) : 0;
-        refill = (v >= 1 && v <= 32) ? v : KERR_REFILL_MIN;
-    }
-    a.refill_min = refill;
-    // resident CTAs per SM ptxas must fit (register cap): the kernel is latency-bound, so more
-    // resident warps win until the spills cost more (LP_KERR_MINB = 2..6, tuning knob; the queued
-    // kernel is built for 3..5 and runs 4 for the others)
-    static int minb = 0;
-    if (!minb) {
-        const char *e = getenv("LP_KERR_MINB");
-        const int v = e ? atoi(e) : 0;
-        minb = (v >= 2 && v <= 6) ? v : KERR_DEFAULT_MINB;
-    }
+    a.refill_min = kerr_knobs().refill;
+    const int minb = kerr_knobs().minb;
     const char *qe = getenv("LP_KERR_QUEUE");
     const bool queued = !(qe && atoi(qe) == 0);
     const void *fn;

@@ -34,7 +34,13 @@ struct RemapArgs {
     int32_t channels;
     int32_t loop_around;
     int32_t sampling;
-    int32_t vec_ok;              // fused kernel: float32 RGB into a 16-byte aligned tile
+    // vector (staged) stores of the frame kernels; each kernel's launcher decides it:
+    //   lp_render_kernel: LP_RENDER_STAGED_STORES, RGB float32 / 8-bit, every run of a warp tile contiguous in the
+    //     output and the output 16-byte aligned;
+    //   lp_render_mirror_kernel: LP_RENDER_STAGED_STORES, RGB float32 / 8-bit, the output aligned to its elements;
+    //   lp_render_repack_kernel: a chunk's 32-pixel batches contiguous in the output, the output 16-byte aligned.
+    // The stand-alone remap kernel does not read it (0).
+    int32_t vec_ok;
     float u8_scale;              // 255 for LP_DTYPE_U8_UNIT images, else 1
     int32_t fast3;               // RGB, nearest sampling, H*W*3 < 2^31: 32-bit index arithmetic
 };

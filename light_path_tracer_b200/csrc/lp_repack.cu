@@ -27,13 +27,11 @@
 // (blockIdx), CTAs are small (64 threads = 2 chunks) and back-filled by the hardware work
 // distributor exactly like lp_render_kernel's.
 #include "lp_trace.cuh"
-#include <stdlib.h>
 
 #define LP_RP_CHUNK 256
 #define LP_RP_BLOCK 64
 #define LP_RP_WARPS (LP_RP_BLOCK / 32)
 #define LP_RP_OUTQ 64
-#define LP_RP_DEFAULT_REFILL 4
 
 enum { RP_INVALID = 0, RP_ESCAPE = 1, RP_CAPTURE = 2, RP_RANOUT = 3 };
 
@@ -357,46 +355,30 @@ lp_render_repack_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts
     }
 }
 
-template <typename T>
-static int launch_repack_t(const TraceArgs &a, const RemapArgs &ra, const BinetConsts &c, const CamConsts &cam,
-                           bool fused, cudaStream_t stream)
+// The lane re-packing frame kernel.  vec_ok: every full 32-pixel batch of a chunk is contiguous in the output
+// (contiguous rows, or frame rows a multiple of 32 wide) and 16-byte aligned (the chunks are staged by construction).
+int lp_launch_render_repack(TraceArgs a, RemapArgs ra, const BinetConsts &c, const CamConsts &cam, int elem,
+                            bool fused, cudaStream_t stream)
 {
-    const size_t stage_bytes = ((size_t)LP_RP_CHUNK * ra.channels * sizeof(T) + 15) & ~(size_t)15;
-    const size_t smem = LP_RP_WARPS * (sizeof(RpQueues) + stage_bytes);
-    const long long per_cta = (long long)LP_RP_WARPS * LP_RP_CHUNK;
-    const long long ctas = (a.n + per_cta - 1) / per_cta;
-    if (ctas > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
+    ra.vec_ok = ((!a.out_frame_rows || cam.width % 32 == 0) && ((uintptr_t)ra.out % 16) == 0) ? 1 : 0;
     // 16 CTAs of 64 threads per SM at 64 registers; let the whole shared memory be used for it
-    auto kf = lp_render_repack_kernel<true, T, 16>;
-    auto ks = lp_render_repack_kernel<false, T, 16>;
-    const void *fn = fused ? (const void *)kf : (const void *)ks;
+    const void *const kernels[3][2] = {
+        {(const void *)lp_render_repack_kernel<false, unsigned char, 16>, (const void *)lp_render_repack_kernel<true, unsigned char, 16>},
+        {(const void *)lp_render_repack_kernel<false, float, 16>, (const void *)lp_render_repack_kernel<true, float, 16>},
+        {(const void *)lp_render_repack_kernel<false, double, 16>, (const void *)lp_render_repack_kernel<true, double, 16>}};
+    const void *fn = kernels[elem][fused];
+    const size_t esz = elem == ELEM_F64 ? 8 : elem == ELEM_F32 ? 4 : 1;
+    const size_t stage_bytes = ((size_t)LP_RP_CHUNK * ra.channels * esz + 15) & ~(size_t)15;
+    const size_t smem = LP_RP_WARPS * (sizeof(RpQueues) + stage_bytes);
     if (cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, 100) != cudaSuccess) cudaGetLastError();
     if (smem > 48 * 1024 &&
         cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
         cudaGetLastError();
         return LP_ERR_UNSUPPORTED;
     }
-    // idle lanes that trigger a refill (LP_REPACK_REFILL = 1..32, tuning knob: 1 = refill after every trip
-    // that saw an exit; larger values trade idle lanes for less bookkeeping)
-    static int refill = 0;
-    if (!refill) {
-        const char *e = getenv("LP_REPACK_REFILL");
-        const int v = e ? atoi(e) : 0;
-        refill = (v >= 1 && v <= 32) ? v : LP_RP_DEFAULT_REFILL;
-    }
-    if (fused) kf<<<(unsigned)ctas, LP_RP_BLOCK, smem, stream>>>(a, ra, c, cam, refill);
-    else       ks<<<(unsigned)ctas, LP_RP_BLOCK, smem, stream>>>(a, ra, c, cam, refill);
-    return lp_check_launch();
-}
-
-int lp_launch_render_repack(const TraceArgs &a, const RemapArgs &ra, const BinetConsts &c, const CamConsts &cam,
-                            int src_dtype, uint32_t flags, cudaStream_t stream)
-{
-    const bool fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
-    switch (src_dtype) {
-    case LP_DTYPE_U8: return launch_repack_t<unsigned char>(a, ra, c, cam, fused, stream);
-    case LP_DTYPE_F32: return launch_repack_t<float>(a, ra, c, cam, fused, stream);
-    case LP_DTYPE_F64: return launch_repack_t<double>(a, ra, c, cam, fused, stream);
-    default: return LP_ERR_INVALID_ARG;
-    }
+    // refill: idle lanes that trigger a refill (1 = after every trip that saw an exit; larger values trade idle
+    // lanes for less bookkeeping)
+    int refill = lp_trace_knobs().repack_refill;
+    void *args[] = {&a, &ra, (void *)&c, (void *)&cam, &refill};
+    return lp_launch_ctas(fn, a.n, (long long)LP_RP_WARPS * LP_RP_CHUNK, LP_RP_BLOCK, smem, args, stream);
 }

@@ -726,13 +726,6 @@ struct Rk45Knobs {
     int eq;         // LP_RK45_EQ = 0 | 1: the equatorial kernel for the `alphas` batch entry
 };
 
-static int env_int(const char *name, int lo, int hi, int dflt)
-{
-    const char *e = getenv(name);
-    const int v = e ? atoi(e) : 0;
-    return (v >= lo && v <= hi) ? v : dflt;
-}
-
 static const Rk45Knobs &rk45_knobs()
 {
     static const Rk45Knobs k = [] {
@@ -741,9 +734,9 @@ static const Rk45Knobs &rk45_knobs()
         // dependent chains, so resident warps win until the spills start.  Six-component kernel: 2 -> 240
         // registers, no spills; 3 -> 168; 4 -> 128 (spills).  Round 1 measured 3 best on the 4K frame, which
         // that kernel then integrated; the frame now runs the equatorial kernel (4 -> 128 registers).
-        r.minb = env_int("LP_RK45_MINB", 2, 4, RK_DEFAULT_MINB);
-        r.eq_minb = env_int("LP_RK45_EQ_MINB", 3, 6, RK_DEFAULT_EQ_MINB);
-        r.refill = env_int("LP_RK45_REFILL", 1, 32, RK_REFILL_MIN);
+        r.minb = lp_env_int("LP_RK45_MINB", 2, 4, RK_DEFAULT_MINB);
+        r.eq_minb = lp_env_int("LP_RK45_EQ_MINB", 3, 6, RK_DEFAULT_EQ_MINB);
+        r.refill = lp_env_int("LP_RK45_REFILL", 1, 32, RK_REFILL_MIN);
         const char *p = getenv("LP_RK45_POW");
         r.fast_pow = p ? (atoi(p) != 0) : -1;
         const char *e = getenv("LP_RK45_EQ");

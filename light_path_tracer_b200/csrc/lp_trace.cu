@@ -8,8 +8,6 @@
 // strided phi table arrive through the kernel parameter (constant) bank.
 #include "lp_trace.cuh"
 
-#include <stdlib.h>
-
 #define LP_RENDER_DEFAULT_TRIP 4
 #define LP_RENDER_DEFAULT_TILE_H 4
 #define LP_TRACE_DEFAULT_BLOCK 256  /* rays per CTA; LP_TRACE_BLOCK=32|64|128|256 overrides (tuning).  Measured on the
@@ -23,6 +21,7 @@
    mirrored 4K frame (2.08M traces; within 2 % either way) and 1080p (12 % faster), 4 for 8K (3 % faster):
    profiles/r3a_trip_sweep.log */
 #define LP_RENDER_TRIP4_MIN_RAYS 4000000LL
+#define LP_REPACK_DEFAULT_REFILL 4  /* idle lanes that trigger a refill of the lane re-packing kernel (lp_repack.cu) */
 
 // LP_TRACE_HYBRID rule.  The FMA loop (scaled second-order form, lp_internal.cuh) differs from the strict one
 // by ~1e-16 per operation.  A perturbation d of the orbit obeys d'' = (-1 + 6 M u) d: it can only grow where
@@ -150,38 +149,35 @@ lp_trace_kernel(const TraceArgs a, const BinetConsts c, const CamConsts cam)
     }
 }
 
-static int trace_block_size()
+const TraceKnobs &lp_trace_knobs()
 {
-    static int cached = 0;
-    if (!cached) {
-        int v = LP_TRACE_DEFAULT_BLOCK;
-        const char *e = getenv("LP_TRACE_BLOCK");
-        if (e) { const int t = atoi(e); if (t == 32 || t == 64 || t == 128 || t == 256) v = t; }
-        cached = v;
-    }
-    return cached;
+    // a knob whose accepted values are the powers of two in [lo, hi]
+    auto pow2 = [](const char *name, int lo, int hi, int dflt) {
+        const int v = lp_env_int(name, lo, hi, dflt);
+        return (v & (v - 1)) == 0 ? v : dflt;
+    };
+    static const TraceKnobs k = {pow2("LP_TRACE_BLOCK", 32, 256, LP_TRACE_DEFAULT_BLOCK),
+                                 pow2("LP_RENDER_TRIP", 2, 4, 0),
+                                 pow2("LP_RENDER_TILE_H", 1, 4, 0),
+                                 lp_env_int("LP_REPACK_REFILL", 1, 32, LP_REPACK_DEFAULT_REFILL)};
+    return k;
 }
 
-template <int SRC, bool WIDE>
-static int launch_trace(const TraceArgs &a, const BinetConsts &c, const CamConsts &cam,
-                        uint32_t flags, cudaStream_t stream)
+// The stand-alone tracer: its loop trip is fixed by the kernel's template arguments.
+static int launch_trace(const TraceArgs &a, const BinetConsts &c, const CamConsts &cam, int src, uint32_t flags,
+                        cudaStream_t stream)
 {
     if (a.n == 0) return LP_OK;
-    // the FMA loop integrates 3M u: without a usable scale (c.scaled_ok) the request runs strictly
-    const bool fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
-    const bool icmp = (fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) != 0;
-    const int block = trace_block_size();
-    const long long chunks = (a.n + block - 1) / block;
-    if (chunks > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
-    const unsigned grid = (unsigned)chunks;
-    if (fused) {
-        if (icmp) lp_trace_kernel<true, true, SRC, WIDE><<<grid, block, 0, stream>>>(a, c, cam);
-        else      lp_trace_kernel<true, false, SRC, WIDE><<<grid, block, 0, stream>>>(a, c, cam);
-    } else {
-        if (icmp) lp_trace_kernel<false, true, SRC, WIDE><<<grid, block, 0, stream>>>(a, c, cam);
-        else      lp_trace_kernel<false, false, SRC, WIDE><<<grid, block, 0, stream>>>(a, c, cam);
-    }
-    return lp_check_launch();
+    const BinetVariant v = lp_binet_variant(flags, c);
+#define LP_TRACE_KERNELS(SRC, WIDE) \
+    {{(const void *)lp_trace_kernel<false, false, SRC, WIDE>, (const void *)lp_trace_kernel<false, true, SRC, WIDE>}, \
+     {(const void *)lp_trace_kernel<true, false, SRC, WIDE>, (const void *)lp_trace_kernel<true, true, SRC, WIDE>}}
+    const void *const kernels[3][2][2] = {LP_TRACE_KERNELS(SRC_F64, true), LP_TRACE_KERNELS(SRC_F32, false),
+                                          LP_TRACE_KERNELS(SRC_CAM, false)};
+#undef LP_TRACE_KERNELS
+    const int block = lp_trace_knobs().block;
+    void *args[] = {(void *)&a, (void *)&c, (void *)&cam};
+    return lp_launch_ctas(kernels[src][v.fused][v.icmp], a.n, block, block, 0, args, stream);
 }
 
 extern "C" int lp_schw_trace_batch_f64(const double *alphas, int64_t n,
@@ -201,7 +197,7 @@ extern "C" int lp_schw_trace_batch_f64(const double *alphas, int64_t n,
     lp_hybrid_rule(flags, M, r_obs, h_max, &a);
     a.alphas = alphas; a.n = n; a.out_fa = out_fa; a.out_w = out_w;
     a.out_status = out_status; a.out_steps = out_steps; a.stats = stats;
-    return launch_trace<SRC_F64, true>(a, c, cam, flags, (cudaStream_t)stream);
+    return launch_trace(a, c, cam, SRC_F64, flags, (cudaStream_t)stream);
 }
 
 extern "C" int lp_schw_trace_alpha32(const float *alpha32, int64_t n,
@@ -221,7 +217,7 @@ extern "C" int lp_schw_trace_alpha32(const float *alpha32, int64_t n,
     lp_hybrid_rule(flags, M, r_obs, h_max, &a);
     a.alphas = alpha32; a.n = n; a.out_fa = out_fa32; a.out_w = out_w16;
     a.out_status = out_status; a.out_steps = out_steps; a.stats = stats;
-    return launch_trace<SRC_F32, false>(a, c, cam, flags, (cudaStream_t)stream);
+    return launch_trace(a, c, cam, SRC_F32, flags, (cudaStream_t)stream);
 }
 
 extern "C" int lp_schw_trace_frame(const lp_camera *h_cam, int32_t row0, int32_t rows,
@@ -244,7 +240,7 @@ extern "C" int lp_schw_trace_frame(const lp_camera *h_cam, int32_t row0, int32_t
     lp_hybrid_rule(flags, M, r_obs, h_max, &a);
     a.n = n; a.out_fa = out_fa32; a.out_w = out_w16; a.out_alpha32 = out_alpha32;
     a.out_status = out_status; a.out_steps = out_steps; a.stats = stats; a.row0 = row0;
-    return launch_trace<SRC_CAM, false>(a, c, cam, flags, (cudaStream_t)stream);
+    return launch_trace(a, c, cam, SRC_CAM, flags, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------
@@ -570,51 +566,68 @@ lp_render_mirror_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts
     }
 }
 
-// RK4 steps per loop trip of the fast path: LP_RENDER_TRIP=2|4 (tuning knob).
-static int render_trip(long long n_rays)
+// The frame kernels' builds of one element type: [FUSED][0: FAST = false; 1, 2: FAST with 2, 4 RK4 steps per trip]
+#define LP_FRAME_KERNELS(K, T) \
+    {{(const void *)K<false, false, T, 4, 2>, (const void *)K<false, true, T, 4, 2>, (const void *)K<false, true, T, 4, 4>}, \
+     {(const void *)K<true, false, T, 4, 2>, (const void *)K<true, true, T, 4, 2>, (const void *)K<true, true, T, 4, 4>}}
+
+// Column of that table: the fast path runs LP_RENDER_TRIP steps per trip, else 4 from LP_RENDER_TRIP4_MIN_RAYS
+// traced rays on.
+static int frame_variant(BinetVariant v, long long traced)
 {
-    static int cached = -1;
-    if (cached < 0) {
-        const char *e = getenv("LP_RENDER_TRIP");
-        cached = (e && atoi(e) == 2) ? 2 : (e && atoi(e) == 4) ? 4 : 0;      // 0: by frame size
-    }
-    if (cached) return cached;
-    return n_rays >= LP_RENDER_TRIP4_MIN_RAYS ? 4 : 2;
+    if (!v.icmp) return 0;
+    const int trip = lp_trace_knobs().trip;
+    return (trip ? trip : traced >= LP_RENDER_TRIP4_MIN_RAYS ? 4 : 2) / 2;
 }
 
+// The one-ray-per-pixel frame kernel (lp_render_kernel) for a tile of `rows` rows.
 // MINB = 4 CTAs of LP_TRACE_BLOCK threads per SM -> ptxas keeps the kernel at 64 registers
 // (32 warps/SM); a 48-register build (40 warps/SM, spills outside the loop) measured 1 % slower.
-template <typename T>
-static int launch_render(const TraceArgs &a, const RemapArgs &ra, const BinetConsts &c,
-                         const CamConsts &cam, uint32_t flags, cudaStream_t stream)
+static int launch_render(TraceArgs a, RemapArgs ra, const BinetConsts &c, const CamConsts &cam, int32_t rows,
+                         int elem, BinetVariant v, uint32_t flags, cudaStream_t stream)
 {
-    const bool fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
-    const bool icmp = (fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) != 0;
-    const int block = trace_block_size();
-    const long long chunks = (a.n + block - 1) / block;
-    if (chunks > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
-    const unsigned grid = (unsigned)chunks;
-    if (fused) {
-        if (icmp && render_trip(a.n) == 4) lp_render_kernel<true, true, T, 4, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else if (icmp) lp_render_kernel<true, true, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else      lp_render_kernel<true, false, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-    } else {
-        if (icmp && render_trip(a.n) == 4) lp_render_kernel<false, true, T, 4, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else if (icmp) lp_render_kernel<false, true, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else      lp_render_kernel<false, false, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
+    // warp tile: LP_RENDER_TILE_H = 1 | 2 | 4 rows per warp (tuning knob; default 4 = 8x4 pixels).
+    // LP_RENDER_ROW_RUNS: 8-bit row bands of a frame that MANY peers store into one GPU's memory over NVLink
+    // (dist.PeerFrame at more than four ranks).  An 8 x 4 tile's runs are 24 bytes — 8-byte stores into partial
+    // 32-byte sectors, ~200 GB/s into the root at 8 GPUs (measured: config 4 at 0.447 ms against 0.31 of compute)
+    // — where a 32 x 1 tile's run is 96 bytes = three whole sectors in 16-byte stores, like the float32 tiles'.
+    int th = lp_trace_knobs().tile_h;
+    if (!th) th = ((flags & LP_RENDER_ROW_RUNS) && elem == ELEM_U8) ? 1 : LP_RENDER_DEFAULT_TILE_H;
+    while (th > 1 && (cam.width % (32 / th) != 0 || rows % th != 0)) th >>= 1;
+    a.tile_h = th; a.tiles_x = cam.width / (32 / th);
+    a.tile_shift = (th == 4) ? 2u : (th == 2) ? 1u : 0u;
+    a.tiles_x_magic = 0u;
+    if ((th > 1 || cam.width % 32 == 0) && a.tiles_x > 1) {
+        // w / tiles_x == (w * ceil(2^32 / tiles_x)) >> 32 for all w <= w_max iff w_max * e < 2^32,
+        // e = tiles_x * ceil(2^32 / tiles_x) - 2^32
+        const unsigned long long d = (unsigned long long)a.tiles_x, two32 = 1ull << 32;
+        const unsigned long long m = (two32 + d - 1) / d, e = m * d - two32;
+        const unsigned long long w_max = (unsigned long long)((a.n + 31) / 32) + 64;
+        if (m < two32 && w_max * e < two32) a.tiles_x_magic = (uint32_t)m;
     }
-    return lp_check_launch();
+    // write-out geometry of a warp tile (see TraceArgs)
+    const int esz = (elem == ELEM_F32) ? 4 : (elem == ELEM_F64) ? 8 : 1;
+    a.st_run_bytes = (32 / th) * 3 * esz;
+    a.st_vb = (a.st_run_bytes % 16 == 0) ? 16 : 8;
+    a.st_per_run = a.st_run_bytes / a.st_vb;
+    a.st_lanes = th * a.st_per_run;
+    a.st_magic = (65536u + (uint32_t)a.st_per_run - 1u) / (uint32_t)a.st_per_run;
+    // every run of a warp tile contiguous and vector-aligned
+    const bool runs_ok = th > 1 || !a.out_frame_rows || cam.width % 32 == 0;
+    ra.vec_ok = ((flags & LP_RENDER_STAGED_STORES) && ra.channels == 3 && runs_ok && elem != ELEM_F64 &&
+                 ((uintptr_t)ra.out % 16) == 0 && a.st_run_bytes % 8 == 0 && a.st_lanes <= 32) ? 1 : 0;
+    const void *const kernels[3][2][3] = {LP_FRAME_KERNELS(lp_render_kernel, unsigned char),
+                                          LP_FRAME_KERNELS(lp_render_kernel, float),
+                                          LP_FRAME_KERNELS(lp_render_kernel, double)};
+    const int block = lp_trace_knobs().block;
+    void *args[] = {&a, &ra, (void *)&c, (void *)&cam};
+    return lp_launch_ctas(kernels[elem][v.fused][frame_variant(v, a.n)], a.n, block, block, 0, args, stream);
 }
 
 // The mirror-image kernel for a contiguous row tile: x mirror when mir_x, y mirror when mir_y (whole frame).
-template <typename T>
-static int launch_render_mirror(const TraceArgs &a_in, const RemapArgs &ra, const BinetConsts &c,
-                                const CamConsts &cam, int32_t rows, bool mir_x, bool mir_y, uint32_t flags,
-                                cudaStream_t stream)
+static int launch_render_mirror(TraceArgs a, RemapArgs ra, const BinetConsts &c, const CamConsts &cam, int32_t rows,
+                                bool mir_x, bool mir_y, int elem, BinetVariant v, uint32_t flags, cudaStream_t stream)
 {
-    const bool fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
-    const bool icmp = (fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) != 0;
-    TraceArgs a = a_in;
     const int W = cam.width;
     a.mir_skip = (int16_t)((mir_x ? 0 : 1) | (mir_y ? 0 : 2));
     // exact zeros of the basis that carry a mirror over to the remap's source direction (lp_render_mirror_kernel)
@@ -625,23 +638,21 @@ static int launch_render_mirror(const TraceArgs &a_in, const RemapArgs &ra, cons
     a.mtx_main = (a.mx_main + 7) / 8;        a.mty_main = (a.my_main + 3) / 4;
     const long long tiles_x = a.mtx_main + (mir_x ? 1 : 0), tiles_y = a.mty_main + (mir_y ? 1 : 0);
     const long long warps = tiles_x * tiles_y;
-    const int block = trace_block_size();
     if (warps * 32 > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
     a.mtiles_x = (uint32_t)tiles_x; a.m_warps = (uint32_t)warps;
-    const unsigned grid = (unsigned)((warps * 32 + block - 1) / block);
     const long long traced = (long long)(a.mx_main + (mir_x ? 1 : 0)) * (a.my_main + (mir_y ? 1 : 0));
-    const int trip = render_trip(traced);
-    if (fused) {
-        if (icmp && trip == 4) lp_render_mirror_kernel<true, true, T, 4, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else if (icmp) lp_render_mirror_kernel<true, true, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else      lp_render_mirror_kernel<true, false, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-    } else {
-        if (icmp && trip == 4) lp_render_mirror_kernel<false, true, T, 4, 4><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else if (icmp) lp_render_mirror_kernel<false, true, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-        else      lp_render_mirror_kernel<false, false, T, 4, 2><<<grid, block, 0, stream>>>(a, ra, c, cam);
-    }
-    return lp_check_launch();
+    // staged runs: RGB, float32 / 8-bit, an output aligned to its elements
+    const int esz = (elem == ELEM_F32) ? 4 : 1;
+    ra.vec_ok = ((flags & LP_RENDER_STAGED_STORES) && ra.channels == 3 && elem != ELEM_F64 &&
+                 ((uintptr_t)ra.out % esz) == 0) ? 1 : 0;
+    const void *const kernels[3][2][3] = {LP_FRAME_KERNELS(lp_render_mirror_kernel, unsigned char),
+                                          LP_FRAME_KERNELS(lp_render_mirror_kernel, float),
+                                          LP_FRAME_KERNELS(lp_render_mirror_kernel, double)};
+    const int block = lp_trace_knobs().block;
+    void *args[] = {&a, &ra, (void *)&c, (void *)&cam};
+    return lp_launch_ctas(kernels[elem][v.fused][frame_variant(v, traced)], warps * 32, block, block, 0, args, stream);
 }
+#undef LP_FRAME_KERNELS
 
 // Frame rows of a (possibly interleaved) tile: last frame row + 1, or -1 for a bad request.
 static long long tile_row_end(int32_t row0, int32_t rows, int32_t band_rows, int32_t band_stride)
@@ -674,89 +685,38 @@ extern "C" int lp_render_frame_bands(const void *src, int32_t src_dtype, int32_t
     BinetConsts c;
     rc = lp_make_binet_consts(M, R_S, r_obs, phi_max, h_max, &c);
     if (rc != LP_OK) return rc;
+    int elem;
+    switch (src_dtype) {
+    case LP_DTYPE_U8: case LP_DTYPE_U8_UNIT: elem = ELEM_U8; break;
+    case LP_DTYPE_F32: elem = ELEM_F32; break;
+    case LP_DTYPE_F64: elem = ELEM_F64; break;
+    default: return LP_ERR_INVALID_ARG;
+    }
     const bool frame_rows = (flags & LP_RENDER_OUT_FRAME_ROWS) != 0;
     TraceArgs a = {};
     lp_hybrid_rule(flags, M, r_obs, h_max, &a);
     a.n = n; a.out_fa = out_fa32; a.out_w = out_w16; a.stats = stats; a.row0 = row0;
     a.band_rows = band_rows; a.band_stride = band_stride;
     a.out_frame_rows = (frame_rows && band_rows > 0) ? 1 : 0;     // contiguous rows: frame-addressed == compact
-    RemapArgs ra;
+    RemapArgs ra = {};                                             // (vec_ok: each kernel's launcher)
     ra.src = src; ra.out = out; ra.fa32 = nullptr; ra.w16 = nullptr; ra.n = n;
     ra.row0 = row0; ra.channels = channels; ra.loop_around = render_loop_around; ra.sampling = sampling;
-    // warp tile: LP_RENDER_TILE_H = 1 | 2 | 4 rows per warp (tuning knob; default 4 = 8x4 pixels)
-    static int tile_h_pref = 0, tile_h_env = 0;
-    if (!tile_h_pref) {
-        const char *e = getenv("LP_RENDER_TILE_H");
-        const int v = e ? atoi(e) : 0;
-        tile_h_env = (v == 1 || v == 2 || v == 4);
-        tile_h_pref = tile_h_env ? v : LP_RENDER_DEFAULT_TILE_H;
-    }
-    int th = tile_h_pref;
-    // LP_RENDER_ROW_RUNS: 8-bit row bands of a frame that MANY peers store into one GPU's memory over NVLink
-    // (dist.PeerFrame at more than four ranks).  An 8 x 4 tile's runs are 24 bytes — 8-byte stores into partial
-    // 32-byte sectors, ~200 GB/s into the root at 8 GPUs (measured: config 4 at 0.447 ms against 0.31 of compute)
-    // — where a 32 x 1 tile's run is 96 bytes = three whole sectors in 16-byte stores, like the float32 tiles'.
-    if (!tile_h_env && (flags & LP_RENDER_ROW_RUNS) && (src_dtype == LP_DTYPE_U8 || src_dtype == LP_DTYPE_U8_UNIT)) th = 1;
-    while (th > 1 && (cam.width % (32 / th) != 0 || rows % th != 0)) th >>= 1;
-    a.tile_h = th; a.tiles_x = cam.width / (32 / th);
-    a.tile_shift = (th == 4) ? 2u : (th == 2) ? 1u : 0u;
-    a.tiles_x_magic = 0u;
-    if ((th > 1 || cam.width % 32 == 0) && a.tiles_x > 1) {
-        // w / tiles_x == (w * ceil(2^32 / tiles_x)) >> 32 for all w <= w_max iff w_max * e < 2^32,
-        // e = tiles_x * ceil(2^32 / tiles_x) - 2^32
-        const unsigned long long d = (unsigned long long)a.tiles_x, two32 = 1ull << 32;
-        const unsigned long long m = (two32 + d - 1) / d, e = m * d - two32;
-        const unsigned long long w_max = (unsigned long long)((n + 31) / 32) + 64;
-        if (m < two32 && w_max * e < two32) a.tiles_x_magic = (uint32_t)m;
-    }
-    const bool contiguous32 = !a.out_frame_rows || cam.width % 32 == 0;
-    const bool runs_ok = th > 1 || contiguous32;        // every run of a warp tile contiguous and vector-aligned
-    ra.vec_ok = ((flags & LP_RENDER_STAGED_STORES) && channels == 3 && runs_ok &&
-                 (src_dtype == LP_DTYPE_F32 || src_dtype == LP_DTYPE_U8 || src_dtype == LP_DTYPE_U8_UNIT) &&
-                 ((uintptr_t)out % 16) == 0) ? 1 : 0;
-    {   // write-out geometry of a warp tile (see TraceArgs)
-        const int esz = (src_dtype == LP_DTYPE_F32) ? 4 : (src_dtype == LP_DTYPE_F64) ? 8 : 1;
-        a.st_run_bytes = (32 / th) * 3 * esz;
-        a.st_vb = (a.st_run_bytes % 16 == 0) ? 16 : 8;
-        a.st_per_run = a.st_run_bytes / a.st_vb;
-        a.st_lanes = th * a.st_per_run;
-        a.st_magic = (65536u + (uint32_t)a.st_per_run - 1u) / (uint32_t)a.st_per_run;
-        if (a.st_run_bytes % 8 != 0 || a.st_lanes > 32) ra.vec_ok = 0;
-    }
     ra.u8_scale = (src_dtype == LP_DTYPE_U8_UNIT) ? 255.0f : 1.0f;
     ra.fast3 = (channels == 3 && sampling == LP_SAMPLE_NEAREST &&
                 (long long)cam.height * cam.width * 3 < 0x7fffffffLL) ? 1 : 0;
-    if (src_dtype == LP_DTYPE_U8_UNIT) src_dtype = LP_DTYPE_U8;
     cudaStream_t st = (cudaStream_t)stream;
+    const BinetVariant v = lp_binet_variant(flags, c);
     // opt-in lane re-packing schedule; it needs the fast-path precondition (observer strictly inside
     // the integration band), otherwise the request falls through to the default kernel
-    const bool rp_fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
-    if ((flags & LP_TRACE_REPACK) && (rp_fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) && c.valid && n <= 0x7fffffffLL) {
-        ra.vec_ok = (contiguous32 && ((uintptr_t)out % 16) == 0) ? 1 : 0;   // chunks are staged by construction
-        return lp_launch_render_repack(a, ra, c, cam, src_dtype, flags, st);
-    }
+    if ((flags & LP_TRACE_REPACK) && v.icmp && c.valid && n <= 0x7fffffffLL)
+        return lp_launch_render_repack(a, ra, c, cam, elem, v.fused, st);
     // mirror images (lp_render_mirror_kernel): contiguous rows stored compactly, default schedule; x needs
     // d0 == 0 (either sign), y needs d1 == 0 and the whole frame, both need d2 != 0
     const bool mir_ok = band_rows == 0 && !(flags & (LP_RENDER_OUT_FRAME_ROWS | LP_RENDER_ROW_RUNS)) && cam.d2 != 0.0;
     const bool mir_x = mir_ok && cam.d0 == 0.0;
     const bool mir_y = mir_ok && cam.d1 == 0.0 && row0 == 0 && rows == cam.height;
-    if (mir_x || mir_y) {
-        const int esz = (src_dtype == LP_DTYPE_F32) ? 4 : 1;
-        ra.vec_ok = ((flags & LP_RENDER_STAGED_STORES) && channels == 3 &&
-                     (src_dtype == LP_DTYPE_F32 || src_dtype == LP_DTYPE_U8) && ((uintptr_t)out % esz) == 0) ? 1 : 0;
-        switch (src_dtype) {
-        case LP_DTYPE_U8: return launch_render_mirror<unsigned char>(a, ra, c, cam, rows, mir_x, mir_y, flags, st);
-        case LP_DTYPE_F32: return launch_render_mirror<float>(a, ra, c, cam, rows, mir_x, mir_y, flags, st);
-        case LP_DTYPE_F64: return launch_render_mirror<double>(a, ra, c, cam, rows, mir_x, mir_y, flags, st);
-        default: return LP_ERR_INVALID_ARG;
-        }
-    }
-    switch (src_dtype) {
-    case LP_DTYPE_U8: return launch_render<unsigned char>(a, ra, c, cam, flags, st);
-    case LP_DTYPE_F32: return launch_render<float>(a, ra, c, cam, flags, st);
-    case LP_DTYPE_F64: return launch_render<double>(a, ra, c, cam, flags, st);
-    default: return LP_ERR_INVALID_ARG;
-    }
+    if (mir_x || mir_y) return launch_render_mirror(a, ra, c, cam, rows, mir_x, mir_y, elem, v, flags, st);
+    return launch_render(a, ra, c, cam, rows, elem, v, flags, st);
 }
 
 extern "C" int lp_render_frame(const void *src, int32_t src_dtype, int32_t channels,

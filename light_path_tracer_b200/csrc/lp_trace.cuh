@@ -100,5 +100,28 @@ __device__ __forceinline__ bool hybrid_needs_retrace(const RayResult &r, int ret
     if (r.status != 1) return false;
     return fmaxf((float)r.fa, 1.0e-3f) < __expf((float)r.steps * h - off);
 }
-int lp_launch_render_repack(const TraceArgs &a, const RemapArgs &ra, const BinetConsts &c, const CamConsts &cam,
-                            int src_dtype, uint32_t flags, cudaStream_t stream);
+
+// The build of the Binet loop a request runs: the FMA loop (FUSED) for LP_TRACE_FUSED / LP_TRACE_HYBRID, and the
+// fast path (FAST, "icmp") where its precondition holds for the loops that kernel runs.
+struct BinetVariant { bool fused, icmp; };
+static inline BinetVariant lp_binet_variant(uint32_t flags, const BinetConsts &c)
+{
+    // the FMA loop integrates 3M u: without a usable scale (c.scaled_ok) the request runs strictly
+    const bool fused = (flags & (LP_TRACE_FUSED | LP_TRACE_HYBRID)) != 0 && c.scaled_ok;
+    return {fused, (fused ? lp_binet_fast_ok_fused(&c) : lp_binet_fast_ok(&c)) != 0};
+}
+
+// The Binet kernels' tuning knobs (DESIGN.md §4), read once per process (lp_trace.cu).
+struct TraceKnobs {
+    int block;          // LP_TRACE_BLOCK = 32 | 64 | 128 | 256: threads per CTA of the tracer and frame kernels
+    int trip;           // LP_RENDER_TRIP = 2 | 4: RK4 steps per loop trip of the frame kernels; 0: by frame size
+    int tile_h;         // LP_RENDER_TILE_H = 1 | 2 | 4: rows of lp_render_kernel's warp tile; 0: not set
+    int repack_refill;  // LP_REPACK_REFILL = 1..32: idle lanes that trigger a refill of the re-packing kernel
+};
+const TraceKnobs &lp_trace_knobs();
+
+// element type of a frame's source and output image: the index of the frame kernel tables
+enum { ELEM_U8 = 0, ELEM_F32 = 1, ELEM_F64 = 2 };
+
+int lp_launch_render_repack(TraceArgs a, RemapArgs ra, const BinetConsts &c, const CamConsts &cam, int elem,
+                            bool fused, cudaStream_t stream);
