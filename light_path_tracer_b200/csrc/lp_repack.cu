@@ -49,7 +49,7 @@ struct RpQueues {
     int pad_[3];
 };
 
-// The per-ray tail for one queue entry: what binet_trace_fast4 does after its loop.
+// The per-ray tail for one queue entry: what binet_trace_fast does after its loop.
 template <bool FUSED>
 __device__ __forceinline__ void rp_finish_ray(const BinetConsts &c, const LoopRegs &L, int code, int k,
                                               double up, double wp, double u, double w, double alpha,
@@ -63,7 +63,7 @@ __device__ __forceinline__ void rp_finish_ray(const BinetConsts &c, const LoopRe
     double phi;
     if (code == RP_RANOUT) {
         // cold path (a ray that reaches phi_max): the remaining full steps one at a time, then the
-        // shortened last steps — metrics.py:72-115 as in binet_trace_fast4
+        // shortened last steps — metrics.py:72-115 as in binet_trace_fast
         const double M3 = L.M3, h = L.h, hh = L.hh, h6 = L.h6;
         bool crossed = false;
         double u1, w1;
@@ -259,7 +259,7 @@ lp_render_repack_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts
             if (__ballot_sync(full, code == -2) != 0u && (in_count > 0 || next_batch < n_batches)) continue;
         }
 
-        // ---- integrate: trips of four RK4 steps (binet_trace_fast4's loop body) until enough lanes have left
+        // ---- integrate: trips of four RK4 steps (a trip of binet_trace_fast<FUSED, 4>) until enough lanes have left
         // the band to make a refill worth its bookkeeping (refill_min; everything, once no ray is left to pop) ----
         // A lane that leaves the band claims a slot of the out-queue (shared-memory atomic) and stores its raw
         // exit state there at once — nothing but (u, w, k) stays live across trips.

@@ -2,7 +2,7 @@
 //   (1) dependent-DFMA issue latency (one warp, one chain, clock64),
 //   (2) FP64-pipe utilisation of the FMA-contracted RK4 loop of lp_internal.cuh as a function of
 //       resident warps per SM sub-partition and of independent rays per thread (ILP), with the
-//       4-steps-per-trip band test of binet_trace_fast4.
+//       4-steps-per-trip band test of binet_trace_fast<FUSED, 4>.
 // Utilisation = FP64 warp instructions x 2 cycles / (elapsed cycles x 592 sub-partitions), SM clock
 // taken as 1.965 GHz (the bench's NVML samples sit there under this load).
 //   nvcc -gencode arch=compute_100a,code=sm_100a -I include -I light_path_tracer_b200/csrc \
