@@ -58,6 +58,8 @@ def lib():
         L.lp_oracle_trace_rays_batch.argtypes = [d, d, d, vp, i64, d, d, vp, vp, vp, vp]
         L.lp_oracle_trace_rays_batch_shift.restype = None
         L.lp_oracle_trace_rays_batch_shift.argtypes = [d, d, d, vp, i64, ctypes.c_int, d, d, vp, vp, vp]
+        L.lp_oracle_trace_rays_batch_sin.restype = None
+        L.lp_oracle_trace_rays_batch_sin.argtypes = [d, d, d, vp, vp, i64, d, d, vp, vp, vp, vp]
         L.lp_oracle_trace_frame_f32.restype = None
         L.lp_oracle_trace_frame_f32.argtypes = [d, d, d, vp, i64, d, d, vp, vp, vp, vp]
         L.lp_oracle_shadow.restype = None
@@ -141,6 +143,23 @@ def trace_rays_batch_sin_shift(M, r_obs, alphas, sin_shift, phi_max=PHI_MAX, h_m
     lib().lp_oracle_trace_rays_batch_shift(M, 2 * M, r_obs, _p(alphas), n, int(sin_shift),
                                            phi_max, h_max, _p(fa), _p(w), _p(st))
     return fa, w, st
+
+
+def trace_rays_batch_sin(M, R_S, r_obs, alphas, sins, phi_max=PHI_MAX, h_max=H_MAX):
+    """Sensitivity entry, not a reference path: trace_rays_batch with the caller's sin(alpha)
+    (``sins``, e.g. the correctly rounded sine the GPU kernels use) in place of the host libm's
+    np.sin(alpha) at metrics.py:55.  -> (out_fa f64[n], out_w i64[n], status i8[n], steps i32[n])."""
+    alphas = np.ascontiguousarray(alphas, dtype=np.float64)
+    sins = np.ascontiguousarray(sins, dtype=np.float64)
+    assert sins.shape == alphas.shape
+    n = alphas.size
+    fa = np.empty(n, np.float64)
+    w = np.empty(n, np.int64)
+    st = np.empty(n, np.int8)
+    steps = np.empty(n, np.int32)
+    lib().lp_oracle_trace_rays_batch_sin(M, R_S, r_obs, _p(alphas), _p(sins), n, phi_max, h_max,
+                                         _p(fa), _p(w), _p(st), _p(steps))
+    return fa, w, st, steps
 
 
 # --------------------------------------------------------------------------
