@@ -336,16 +336,20 @@ lp_render_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts c, con
 // fast3 (the common layout, see remap_pixel_dir) with every image's direction shared: each image's outcome —
 // zeros, winding colour, magenta or a source offset — is decided first, then all images' gathers are issued
 // back to back, then staged / stored.  Every other case remaps one image at a time (remap_pixel_dir).
-// Staged stores (RGB, float32 / 8-bit): the run of tile row q in image k (up to 8 pixels, contiguous in the
-// output, in reverse order for an x mirror) follows from the warp tile's geometry and the mirror flags: it
-// loses a pixel where a lane has no partner (column 0, column W / 2, row 0, row H / 2).  Every image's runs
-// are staged at the same address modulo the vector width as their destinations, then one __syncwarp, then one
-// pass in which lane j of row q stores the run's 16-byte (float32) / 8-byte (8-bit) window j: as a vector,
-// or at the run's two ends as at most three naturally aligned pieces (8 / 4 bytes, 4 / 2 / 1 bytes).
+// A CTA owns a strip of its warps' tiles side by side in one tile row (64 x 4 pixels for 8 warps), strips in
+// row-major order from the centre outwards; the tiles of column 0 and row 0, which have no partner in one axis,
+// come in CTAs of their own after all strips and store their pixels directly.
+// Staged stores (RGB, float32 / 8-bit): the run of strip row q in image k (up to 64 pixels, contiguous in the
+// output, in reverse order for an x mirror) follows from the strip's geometry and the mirror flags: it loses
+// a pixel where a lane has no partner (column W / 2, row H / 2).  Every image's runs are staged at the same
+// address modulo 16 as their destinations, then one __syncthreads, then one pass across the CTA in which
+// thread t stores 16-byte window t of the staged runs: as a vector, or at a run's two ends as at most four
+// naturally aligned pieces (8 / 4 bytes for float32, 8 / 4 / 2 / 1 bytes for 8-bit).
 // ---------------------------------------------------------------------------
-/* bytes of one staged run: 8 pixels + the alignment offset inside a vector, rounded up to whole vectors:
-   112 for float32 (96 + 12), 32 for 8-bit (24 + 7).  stage[8][4][4][slot] = 14 336 / 4 096 bytes per CTA */
-#define LP_MIRROR_RUN_SLOT(T) (sizeof(T) == 4 ? 112 : 32)
+#define LP_MIRROR_STRIP_W (LP_TRACE_BLOCK / 32 * 8)     /* pixels in a strip row of a full CTA */
+/* bytes of one staged run: a strip row + the alignment offset inside a vector, rounded up to whole vectors:
+   784 for float32 (768 + 15), 208 for 8-bit (192 + 15).  stage[4][4][slot] = 12 544 / 3 328 bytes per CTA */
+#define LP_MIRROR_RUN_SLOT(T) ((LP_MIRROR_STRIP_W * 3 * (unsigned)sizeof(T) + 30u) / 16u * 16u)
 
 // one naturally aligned piece of N bytes of a staged run to global memory
 template <unsigned N> struct MirrorPiece;
@@ -368,40 +372,24 @@ __device__ __forceinline__ void mirror_piece(unsigned char *g, const unsigned ch
     else asm volatile("st.global.v4.u32 [%0], {%1, %2, %3, %4};" :: "l"(d), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
 
-// bytes [s, e) of a staged window of VB bytes (0 <= s < e <= VB): climb from s to the window's alignment, then
-// descend to e — a window that holds a run's start (e == VB) or end (s == 0) takes at most three pieces
-template <unsigned VB>
+// bytes [s, e) of a staged 16-byte window (0 <= s < e <= 16) whose bytes come in granules of G (a pixel's
+// element size): climb from s to the window's alignment, then descend to e
+template <unsigned G>
 __device__ __forceinline__ void mirror_window_part(unsigned char *g, const unsigned char *sm, unsigned s, unsigned e)
 {
     unsigned p = s;
-    if constexpr (VB == 8) {                                     // 8-bit RGB: 1, 2, 4 up, then 4, 2, 1 down
+    if constexpr (G == 1) {                                      // 8-bit RGB: 1, 2, 4, 8 up, then 8, 4, 2, 1 down
         if ((p & 1u) && p + 1u <= e) { mirror_piece<1>(g, sm, p); p += 1u; }
         if ((p & 2u) && p + 2u <= e) { mirror_piece<2>(g, sm, p); p += 2u; }
-        if ((p & 4u) && p + 4u <= e) { mirror_piece<4>(g, sm, p); p += 4u; }
-        if (p + 4u <= e) { mirror_piece<4>(g, sm, p); p += 4u; }
+    }                                                            // float32 RGB: 4, 8 up, then 8, 4 down
+    if ((p & 4u) && p + 4u <= e) { mirror_piece<4>(g, sm, p); p += 4u; }
+    if ((p & 8u) && p + 8u <= e) { mirror_piece<8>(g, sm, p); p += 8u; }
+    if (p + 8u <= e) { mirror_piece<8>(g, sm, p); p += 8u; }
+    if (p + 4u <= e) { mirror_piece<4>(g, sm, p); p += 4u; }
+    if constexpr (G == 1) {
         if (p + 2u <= e) { mirror_piece<2>(g, sm, p); p += 2u; }
         if (p + 1u <= e) mirror_piece<1>(g, sm, p);
-    } else {                                                     // float32 RGB: 4, 8 up, then 8, 4 down
-        if ((p & 4u) && p + 4u <= e) { mirror_piece<4>(g, sm, p); p += 4u; }
-        if ((p & 8u) && p + 8u <= e) { mirror_piece<8>(g, sm, p); p += 8u; }
-        if (p + 8u <= e) { mirror_piece<8>(g, sm, p); p += 8u; }
-        if (p + 4u <= e) mirror_piece<4>(g, sm, p);
     }
-}
-
-// The run of tile row q in image (fx, fy): image row ir, image columns [cs, cs + n); n == 0: no run.  c0, ncol:
-// the warp tile's traced columns c0 .. c0 + ncol - 1; r: the row's traced (tile-local) row, row_ok: it exists.
-__device__ __forceinline__ int mirror_run(const CamConsts &cam, bool fx, bool fy, bool main_x, int c0, int ncol,
-                                          int r, bool row_ok, int &ir, int &cs)
-{
-    const int W = cam.width, H = cam.height;
-    ir = fy ? H - r : r;
-    if (!row_ok || (fy && (r == 0 || 2 * r == H))) return 0;
-    if (!fx) { cs = c0; return ncol; }
-    if (!main_x) return 0;                                       // column 0 alone
-    const int first = c0 + (2 * c0 == W ? 1 : 0), last = c0 + ncol - 1;      // without column W / 2
-    cs = W - last;
-    return last - first + 1;
 }
 
 template <bool FUSED, bool FAST, typename T, int MINB, int TRIP>
@@ -410,17 +398,29 @@ lp_render_mirror_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts
 {
     const LoopRegs L = load_loop_regs<FUSED>(c);
     constexpr unsigned SLOT = LP_MIRROR_RUN_SLOT(T);
-    __shared__ __align__(16) unsigned char stage[LP_TRACE_BLOCK / 32][4][4][SLOT];
+    __shared__ __align__(16) unsigned char stage[4][4][SLOT];
     const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5, j = lane & 7, q = lane >> 3;
-    const unsigned wt = blockIdx.x * (blockDim.x >> 5) + wrp;
-    const unsigned ty = wt / a.mtiles_x, tx = wt - ty * a.mtiles_x;
+    const unsigned nw = blockDim.x >> 5;
+    // this warp's tile: in a strip (CTA-uniform), or column 0 / row 0 (the x mirror's column-0 tiles first)
+    const bool strip = blockIdx.x < a.m_ctas;
+    unsigned ty, tx;
+    bool tile_ok;
+    if (strip) {
+        ty = blockIdx.x / a.m_strips;
+        tx = (blockIdx.x - ty * a.m_strips) * nw + wrp;
+        tile_ok = (int)tx < a.mtx_main;
+    } else {
+        const unsigned e = (blockIdx.x - a.m_ctas) * nw + wrp, ecol = (a.mir_skip & 1) ? 0u : (unsigned)a.mty_main;
+        if (e < ecol) { tx = a.mtx_main; ty = e; } else { tx = e - ecol; ty = a.mty_main; }
+        tile_ok = e < a.m_edge;
+    }
     int col, r;                  // frame column, tile-local row of the traced pixel
     bool live;
     if ((int)tx < a.mtx_main) { col = (int)(tx * 8u) + j; live = col < a.mx_main; col += a.mx_base; }
     else { col = 0; live = j == 0; }
     if ((int)ty < a.mty_main) { r = (int)(ty * 4u) + q; live = live && r < a.my_main; r += a.my_base; }
     else { r = 0; live = live && q == 0; }
-    live = live && wt < a.m_warps;
+    live = live && tile_ok;
     RayResult res;
     res.status = 0; res.steps = 0; res.nh = 0; res.fa = 0.0;
     if (live) {
@@ -456,28 +456,24 @@ lp_render_mirror_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts
         if (k & share & 2) dk.qy = -dk.qy;
         return dk;
     };
-    // warp tile geometry of the write-out (the runs of every image follow from it: mirror_run)
-    // (from col and r rather than tx, ty: fewer registers live across the trace.  With a mirror on, column 0 /
-    // row 0 is traced only by the extra tile column / row, whose lanes all hold it)
-    const bool main_x = (skip & 1) || col != 0, main_y = (skip & 2) || r != 0;
-    const int c0 = main_x ? col - j : 0;
-    const int ncol = main_x ? min(8, a.mx_base + a.mx_main - c0) : 1;
-    const bool row_ok = (main_y ? r - a.my_base < a.my_main : q == 0) && wt < a.m_warps;
-    const bool vec = (sizeof(T) == 4 || sizeof(T) == 1) && ra.vec_ok;
+    // strip geometry of the write-out: tile row sy, traced columns cs0 .. last (from blockIdx rather than kept
+    // across the trace).  Edge CTAs store directly.
+    const bool vec = (sizeof(T) == 4 || sizeof(T) == 1) && ra.vec_ok && strip;       // CTA-uniform
+    const unsigned sy = strip ? blockIdx.x / a.m_strips : 0u;
+    const int cs0 = a.mx_base + (int)((blockIdx.x - sy * a.m_strips) * nw * 8u);
+    const int last = min(cs0 + (int)(nw * 8u), a.mx_base + a.mx_main) - 1;
     constexpr int PX = 3 * (int)sizeof(T);                                  // bytes of a staged (RGB) pixel
-    constexpr unsigned VB = (sizeof(T) == 4) ? 16u : 8u;                    // store vector width
-    // image k's pixel in the output, and (vec) its place in the run's staging slot
+    // image k's pixel in the output, and (vec) its place in the staging slot of its run: the run of strip row q
+    // starts at image column cs0 (W - last for an x mirror) and sits at its destination's address modulo 16
     auto image_out = [&](int k) -> T * {
         const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
         return (T *)ra.out + ((long long)(fy ? H - r : r) * W + (fx ? W - col : col)) * ra.channels;
     };
     auto image_slot = [&](int k) -> T * {
         const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
-        const int ic = fx ? W - col : col;
-        int ir, cs = 0;
-        mirror_run(cam, fx, fy, main_x, c0, ncol, r, row_ok, ir, cs);
-        const unsigned off = ((unsigned)(uintptr_t)ra.out + ((unsigned)ir * (unsigned)W + (unsigned)cs) * (unsigned)PX) & (VB - 1u);
-        return (T *)(stage[wrp][k][q] + off + (ic - cs) * PX);
+        const unsigned run = (unsigned)(fy ? H - r : r) * (unsigned)W + (unsigned)(fx ? W - last : cs0);
+        const unsigned off = ((unsigned)(uintptr_t)ra.out + run * (unsigned)PX) & 15u;
+        return (T *)(stage[k][q] + off + (fx ? last - col : col - cs0) * PX);
     };
     if (sizeof(T) <= 4 && ra.fast3 && ((skip | share) & 3) == 3) {     // warp-uniform
         // 1. outcomes: a colour for the whole ray (zeros: captured / invalid, or the winding colour), else per
@@ -537,25 +533,26 @@ lp_render_mirror_kernel(const TraceArgs a, const RemapArgs ra, const BinetConsts
         }
     }
     if (vec) {
-        // one write-out pass: lane j of tile row q stores window j of the row's run in every image
-        __syncwarp();
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            if (k & skip) continue;                                          // warp-uniform
-            int ir, cs = 0;
-            const int n = mirror_run(cam, (k & 1) != 0, (k & 2) != 0, main_x, c0, ncol, r, row_ok, ir, cs);
+        // one store pass across the CTA: thread t stores window t % NWIN of the run t / NWIN = (image k, row q)
+        constexpr unsigned NWIN = SLOT / 16u;
+        __syncthreads();
+        for (unsigned t = threadIdx.x; t < 16u * NWIN; t += blockDim.x) {
+            const unsigned kq = t / NWIN, w0 = (t - kq * NWIN) * 16u;        // window: bytes [w0, w0 + 16) of the slot
+            const int k = (int)(kq >> 2), rr = (int)(sy * 4u + (kq & 3u));   // rr: the row's index in the traced rows
+            const bool fx = (k & 1) != 0, fy = (k & 2) != 0;
+            const int rw = a.my_base + rr;
+            if ((k & skip) || rr >= a.my_main || (fy && 2 * rw == H)) continue;
+            const int n = last - ((fx && 2 * cs0 == W) ? cs0 + 1 : cs0) + 1;   // (x images: without column W / 2)
             if (n <= 0) continue;
-            unsigned char *const base = (unsigned char *)ra.out + ((long long)ir * W + cs) * PX;     // the run's start
-            const unsigned off = (unsigned)(uintptr_t)base & (VB - 1u), end = off + (unsigned)(n * PX);
-            const unsigned w0 = (unsigned)j * VB;                            // window j: bytes [w0, w0 + VB) of the slot
+            unsigned char *const base = (unsigned char *)ra.out + ((long long)(fy ? H - rw : rw) * W + (fx ? W - last : cs0)) * PX;
+            const unsigned off = (unsigned)(uintptr_t)base & 15u, end = off + (unsigned)(n * PX);
             if (w0 >= end) continue;
             unsigned char *const g = base - off + w0;
-            const unsigned char *const sm = stage[wrp][k][q] + w0;
-            const unsigned s = off > w0 ? off - w0 : 0u, e = min(end - w0, VB);
-            if (s == 0u && e == VB) mirror_piece<VB>(g, sm, 0u);
-            else mirror_window_part<VB>(g, sm, s, e);
+            const unsigned char *const sm = stage[k][kq & 3u] + w0;
+            const unsigned s = off > w0 ? off - w0 : 0u, e = min(end - w0, 16u);
+            if (s == 0u && e == 16u) mirror_piece<16>(g, sm, 0u);
+            else mirror_window_part<(unsigned)sizeof(T)>(g, sm, s, e);
         }
-        __syncwarp();      // reconverge the warp after the lane-divergent stores
     }
     if (a.stats) {
         const unsigned m = (xm ? 2u : 1u) * (ym ? 2u : 1u);
@@ -636,10 +633,15 @@ static int launch_render_mirror(TraceArgs a, RemapArgs ra, const BinetConsts &c,
     a.mx_main = mir_x ? W / 2 : W;           a.mx_base = mir_x ? W - W / 2 : 0;
     a.my_main = mir_y ? rows / 2 : rows;     a.my_base = mir_y ? rows - rows / 2 : 0;
     a.mtx_main = (a.mx_main + 7) / 8;        a.mty_main = (a.my_main + 3) / 4;
-    const long long tiles_x = a.mtx_main + (mir_x ? 1 : 0), tiles_y = a.mty_main + (mir_y ? 1 : 0);
-    const long long warps = tiles_x * tiles_y;
-    if (warps * 32 > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
-    a.mtiles_x = (uint32_t)tiles_x; a.m_warps = (uint32_t)warps;
+    // strips of a CTA's warp tiles side by side, row-major from the centre outwards (the photon ring's CTAs
+    // start first), then the tiles of column 0 (one per tile row) and of row 0 (one per tile column and the
+    // corner), one per warp
+    const int block = lp_trace_knobs().block, nw = block / 32;
+    const long long strips = (a.mtx_main + nw - 1) / nw, ctas = strips * a.mty_main;
+    const long long edge = (mir_x ? a.mty_main : 0) + (mir_y ? a.mtx_main + (mir_x ? 1 : 0) : 0);
+    const long long all_ctas = ctas + (edge + nw - 1) / nw;
+    if (all_ctas * block > 0x7fffffffLL) return LP_ERR_UNSUPPORTED;
+    a.m_strips = (uint32_t)strips; a.m_ctas = (uint32_t)ctas; a.m_edge = (uint32_t)edge;
     const long long traced = (long long)(a.mx_main + (mir_x ? 1 : 0)) * (a.my_main + (mir_y ? 1 : 0));
     // staged runs: RGB, float32 / 8-bit, an output aligned to its elements
     const int esz = (elem == ELEM_F32) ? 4 : 1;
@@ -648,9 +650,9 @@ static int launch_render_mirror(TraceArgs a, RemapArgs ra, const BinetConsts &c,
     const void *const kernels[3][2][3] = {LP_FRAME_KERNELS(lp_render_mirror_kernel, unsigned char),
                                           LP_FRAME_KERNELS(lp_render_mirror_kernel, float),
                                           LP_FRAME_KERNELS(lp_render_mirror_kernel, double)};
-    const int block = lp_trace_knobs().block;
     void *args[] = {&a, &ra, (void *)&c, (void *)&cam};
-    return lp_launch_ctas(kernels[elem][v.fused][frame_variant(v, traced)], warps * 32, block, block, 0, args, stream);
+    return lp_launch_ctas(kernels[elem][v.fused][frame_variant(v, traced)], all_ctas * block, block, block, 0, args,
+                          stream);
 }
 #undef LP_FRAME_KERNELS
 

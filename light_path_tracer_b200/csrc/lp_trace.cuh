@@ -35,8 +35,8 @@ struct TraceArgs {
     // tile_shift = log2(tile_h); tiles_x_magic = ceil(2^32 / tiles_x) when the host has verified that
     // __umulhi(w, magic) == w / tiles_x for every warp tile index w of this launch, else 0 (plain division)
     uint32_t tile_shift, tiles_x_magic;
-    uint32_t m_warps;       // mirror-image frame kernel: warp tiles in the launch (placed here so that the
-                            // 4-byte fields below share 8-byte words in pairs as the kernels load them)
+    uint32_t m_edge;        // mirror-image frame kernel: warp tiles of column 0 / row 0 (placed here so that
+                            // the 4-byte fields below share 8-byte words in pairs as the kernels load them)
     // staged stores of the frame kernel (host-side arithmetic of the warp's write-out, so that the kernel
     // has no integer division): bytes of one run of the warp tile, vector width (16 / 8), vectors per run,
     // lanes that store (tile_h * per_run), and ceil(2^16 / per_run) for lane / per_run by multiply-shift
@@ -49,7 +49,9 @@ struct TraceArgs {
     // the camera basis carries that mirror over to the remap's source direction exactly (lp_render_mirror_kernel).
     int16_t mir_skip, mir_share;
     int32_t mx_main, mx_base, mtx_main, my_main, my_base, mty_main;
-    uint32_t mtiles_x;      // warp tiles per tile row
+    // CTA b < m_ctas owns strip b % m_strips of tile row b / m_strips: its warps' tiles side by side (m_strips
+    // strips per tile row); the CTAs after them hold the m_edge tiles of column 0 and row 0, one per warp
+    uint32_t m_strips, m_ctas;
 };
 
 // frame row of tile-local row r (interleaved bands, see above)
