@@ -25,7 +25,7 @@ LIB = os.path.join(OUT, "liblightpath.so")
 EXT = os.path.join(OUT, "_lp_torch.so")
 
 CU_SOURCES = ["lp_host.cu", "lp_trace.cu", "lp_repack.cu", "lp_peer.cu", "lp_remap.cu", "lp_shadow.cu", "lp_rk45.cu", "lp_kerr.cu"]
-HEADERS = ["lp_internal.cuh", "lp_trace.cuh", "lp_remap.cuh", "lp_sincr.cuh", "lp_sintab.h", os.path.join(INCLUDE, "lightpath.h")]
+HEADERS = ["lp_internal.cuh", "lp_rk45_rhs.cuh", "lp_trace.cuh", "lp_remap.cuh", "lp_sincr.cuh", "lp_sintab.h", os.path.join(INCLUDE, "lightpath.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

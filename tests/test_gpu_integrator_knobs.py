@@ -3,8 +3,9 @@ process, so every setting runs in its own subprocess): resident CTAs per SM of t
 equatorial RK45 kernels (LP_RK45_MINB, LP_RK45_EQ_MINB), the RK45 refill threshold (LP_RK45_REFILL) and the
 Kerr schedule knobs (LP_KERR_MINB, LP_KERR_REFILL, LP_KERR_QUEUE=0 = the parked schedule).  They change
 register limits or which lane runs a ray, never the operations of a ray, so no output byte may change.
-LP_RK45_POW and LP_RK45_EQ=0 do change results within the parity bar and are not covered here; the
-LP_RK45_EQ pair is held together by test_gpu_rk45.py."""
+LP_RK45_POW and LP_RK45_EQ=0 do change results within the parity bar: test_gpu_rk45_offplane.py holds the
+six-component and Kerr kernels to the oracle under LP_RK45_POW=1, and test_gpu_rk45.py holds the LP_RK45_EQ
+pair together."""
 import json
 import os
 import subprocess
@@ -45,6 +46,14 @@ for r_obs in (100.0, 15.0):
                                         for sol, outcome in paths]
 sol, outcome = gt.integrate_geodesic(m, [0.0, 30.0, 1.1, 0.3, -1.0, -0.93, 2.5, 6.0])
 out["integrate_geodesic"] = digest(sol.t, sol.y, [sol.nfev, sol.status]) + outcome
+# the Kerr RK45 kernel on rays with angular momentum (every screen angle, off the equator)
+k = Kerr(1.0, 0.9)
+rng = np.random.default_rng(9)
+s0 = np.array([k.initial_conditions(30.0, al, sc, 1.1) for al, sc in zip(rng.uniform(0.0, 0.45, 400),
+                                                                         rng.uniform(-np.pi, np.pi, 400))])
+traj, npts, state, lam, oc, ns, status, _, _ = gt._paths(k, state0=s0)
+out["kerr_rk45_paths"] = digest(np.concatenate([traj[i, :npts[i]] for i in range(npts.size)]), npts, state, lam, oc,
+                                ns, status)
 H, W = 135, 243
 vfov = np.radians(40.0)
 fov = (2 * np.arctan(np.tan(vfov / 2) * W / H), vfov)

@@ -251,12 +251,21 @@ def test_dense_output_sol_vs_scipy(native):
     scipy_integrate = pytest.importorskip("scipy.integrate")
     gt = _gt()
     from light_path_tracer_b200.metrics import Schwarzschild, Kerr
-    cases = [(Schwarzschild(1.0), 50.0, np.radians(8.0)), (Schwarzschild(1.0), 50.0, np.radians(3.0)),
-             (Schwarzschild(2.0), 120.0, np.radians(7.0)), (Schwarzschild(1.0), 30.0, np.radians(120.0)),
-             (Kerr(1.0, 0.6), 40.0, np.radians(10.0))]
+    # (metric, r_obs, alpha, screen angle, theta_obs); the last two Kerr rays have angular momentum and
+    # leave the equator
+    cases = [(Schwarzschild(1.0), 50.0, np.radians(8.0), 0.0, np.pi / 2),
+             (Schwarzschild(1.0), 50.0, np.radians(3.0), 0.0, np.pi / 2),
+             (Schwarzschild(2.0), 120.0, np.radians(7.0), 0.0, np.pi / 2),
+             (Schwarzschild(1.0), 30.0, np.radians(120.0), 0.0, np.pi / 2),
+             (Kerr(1.0, 0.6), 40.0, np.radians(10.0), 0.0, np.pi / 2),
+             (Kerr(1.0, 0.9), 40.0, np.radians(10.0), 1.0, 1.2),
+             (Kerr(1.0, -0.998), 40.0, np.radians(8.0), 2.0, 0.3)]
+    states = [(metric, metric.initial_conditions(r_obs, alpha, screen, theta_obs))
+              for metric, r_obs, alpha, screen, theta_obs in cases]
+    # an off-plane Schwarzschild state (Schwarzschild.initial_conditions only makes equatorial ones)
+    states.append((Schwarzschild(1.0), [0.0, 30.0, 1.1, 0.3, -1.0, -0.93, 2.5, 6.0]))
     worst = 0.0
-    for metric, r_obs, alpha in cases:
-        state0 = metric.initial_conditions(r_obs, alpha)
+    for metric, state0 in states:
         sol, outcome = gt.integrate_geodesic(metric, state0)
         assert callable(sol.sol) and sol.sol.n_segments == sol.t.size - 1
         r_in, r_out = metric.capture_radius(), 2.0 * state0[1]
@@ -277,7 +286,7 @@ def test_dense_output_sol_vs_scipy(native):
         got, want = sol.sol(tt), ref.sol(tt)
         assert got.shape == want.shape == (8, tt.size)
         err = np.abs(got - want) / np.maximum(np.abs(want), FLOOR[:, None])
-        assert err.max() <= 1e-10, (type(metric).__name__, r_obs, alpha, err.max(axis=1))
+        assert err.max() <= 1e-10, (type(metric).__name__, state0, err.max(axis=1))
         worst = max(worst, float(err.max()))
         one = sol.sol(float(mids[3]))
         assert one.shape == (8,) and np.allclose(one, got[:, ref.t.size + 3], rtol=1e-14, atol=0.0)
